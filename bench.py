@@ -63,7 +63,12 @@ def parse_args():
     ap.add_argument("--profile-region", default="steps", choices=("steps", "png"),
                     help="what sits between cudaProfilerStart/Stop for `ncu --profile-from-start off`: the timed steps or the PNG stage")
     ap.add_argument("--profile-host", default=None, help="write a cProfile of the timed step loop to this path")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
 
 
 # ----------------------------------------------------------------------------------------
@@ -639,6 +644,30 @@ def api_e2e_leg(args, cubes, files, orbits, state, with_reference, dist=None, ra
             shutil.rmtree(work, ignore_errors=True)
 
 
+DUMP_RGBA_PIXELS = 2_000_000  # 32 MB as float32 RGBA: with the other arrays well inside 64 MB
+
+
+def dump_outputs(out_dir, state, batch):
+    """What one step hands its caller, as float arrays under ``out_dir``, so that two builds can be compared
+    output for output on the same seeded workload:
+
+    ``extrema.npy``          float64, the ``*_y_min / _y_max / _z_min / _z_max`` entries of the global extrema
+                             in sorted key order (None -> NaN)
+    ``panel_vmin_vmax.npy``  float64 (panels, 2), every panel's resolved norm bounds, by panel id
+    ``rgba_sample.npy``      float32 (pixels, 4), the RGBA rasters at a fixed, seeded sample of
+                             ``DUMP_RGBA_PIXELS`` pixel positions (all of them when there are fewer)"""
+    os.makedirs(out_dir, exist_ok=True)
+    keys = sorted(k for k in state if k.endswith(("_y_min", "_y_max", "_z_min", "_z_max")))
+    extrema = np.array([np.nan if state[k] is None else float(state[k]) for k in keys], dtype=np.float64)
+    norms = batch.norms()
+    bounds = np.stack([norms["vmin"], norms["vmax"]], axis=1).astype(np.float64)
+    rgba = batch.all_rgba().reshape(-1, 4)
+    if len(rgba) > DUMP_RGBA_PIXELS:
+        rgba = rgba[np.sort(np.random.default_rng(0).choice(len(rgba), DUMP_RGBA_PIXELS, replace=False))]
+    for name, arr in (("extrema", extrema), ("panel_vmin_vmax", bounds), ("rgba_sample", rgba.astype(np.float32))):
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+
 def bind_near_gpu(torch, local):
     """Multi-rank runs: keep this process (and so the first-touch placement of its pinned staging
     buffers) on the CPUs of the GPU's NUMA node, so every rank's H2D traffic stays on its own socket."""
@@ -767,6 +796,8 @@ def main():
     host_enqueue_ms = (time.perf_counter() - host_t0) * 1e3 / args.steps
     step.finish()
     barrier()
+    if args.dump_outputs and rank == 0:  # before the per-stage passes below rewrite the rasters
+        dump_outputs(args.dump_outputs, state, shard.batch)
 
     def exchange_of(sh):
         sel = getattr(sh, "_pool_selector_side", None) or getattr(sh, "_pool_selector", None)
