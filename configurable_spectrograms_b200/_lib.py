@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 # CSG_LIBRARY: another build of the same ABI (A/B experiments: a kernel variant compiled with a different -D)
 LIB_PATH = os.environ.get("CSG_LIBRARY") or os.path.join(HERE, "libcsgpu.so")
 
-ABI_VERSION = 24
+ABI_VERSION = 25
 F32, F64 = 0, 1
 LAYOUT_TPE, LAYOUT_TEP = 0, 1
 K1_GENERIC, K1_STREAM = 0, 1
@@ -191,7 +191,6 @@ SIGNATURES = {
     "csg_collapse_blocks": (C.c_int32, [C.c_int32, C.c_int32, C.c_int32, _i, _i, _i]),
     "csg_sums_elems": (_i64, [C.c_int32, C.c_int32, _i]),
     "csg_collapse": (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp]),
-    "csg_collapse_range": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp]),
     "csg_window_any": (_i, [_vp, _vp, _vp, _i, _vp, _vp]),
     "csg_collapse_host": (_i, [_vp, _vp, C.c_int32, C.c_int32, C.c_int32, _i, _i, _vp, _i, _vp, _vp]),
     "csg_region_stats_run": (_i, [_vp, _vp, _i, _vp, _i, _vp, _vp]),
@@ -480,14 +479,6 @@ class Context:
             side = self._side = Context(self.device, side=True)
         return side
 
-    def worker_context(self) -> "Context":
-        """A second companion context (own high-priority stream): the per-piece K2a / K3 work that runs
-        next to the main stream's K1 (``fast.pipeline.BatchStep``)."""
-        worker = self.__dict__.get("_worker")
-        if worker is None:
-            worker = self._worker = Context(self.device, side=True)
-        return worker
-
     def background_context(self) -> "Context":
         """A companion context on the LEAST urgent stream: long kernels that should yield to everything else
         (the K4 encoder beside the next chunk's K2a / K3)."""
@@ -565,10 +556,9 @@ class Context:
     def launch_count(self) -> int:
         """Kernels launched by this context and by its side context (if it has one)."""
         n = int(self.lib.csg_launch_count(self.handle))
-        for name in ("_side", "_worker"):
-            other = self.__dict__.get(name)
-            if other is not None:
-                n += other.launch_count()
+        side = self.__dict__.get("_side")
+        if side is not None:
+            n += side.launch_count()
         return n
 
     def d2h_side(self, host_ptr: int, dev_ptr: int, nbytes: int):

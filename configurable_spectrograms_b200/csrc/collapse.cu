@@ -19,10 +19,12 @@
 // Kernels
 //   collapse_stream_kernel (TPE, the FAST shapes) block = 16 time rows x all energy chunks; the pitch
 //       axis is walked in host-built runs of constant group membership with a loop body
-//       specialised per membership mask.  PIPE: every thread keeps a two-stage cp.async pipeline
+//       specialised per membership mask.  Blocks of up to 384 threads (E = 96 float32 / 48 float64,
+//       the FAST tables) take the PIPE body: every thread keeps a two-stage cp.async pipeline
 //       of its own 16-byte chunks (8 pitch bins per stage) in shared memory, so loads stay in
-//       flight while the previous bins are summed (6.7 TB/s; the register-staged variant with
-//       eight 128-bit streaming loads per batch reaches 5.7 TB/s).  The transposed 16-row tile
+//       flight while the previous bins are summed (6.7 TB/s).  Larger blocks, whose load slots
+//       would not leave room for two blocks per SM, take the register-staged body with eight
+//       128-bit streaming loads per batch (5.7 TB/s on the same shapes).  The transposed 16-row tile
 //       leaves through shared memory as 64-byte row segments.  The tile loads are per-thread
 //       cp.async (LDGSTS), not TMA: every thread consumes exactly the bytes it requested, so there
 //       is no block-wide tile to hand around and no mbarrier to wait on; the kernel sits at the
@@ -32,7 +34,6 @@
 //   collapse_tep_rows_kernel (stored (T,E,P) view, no groups, 8 <= P <= 128, P % 8 == 0) two lanes
 //       per (t,e) row own numpy's eight pairwise accumulators; P/8 vector loads in flight.
 //   collapse_tep_kernel      (stored (T,E,P) view, general) rows staged in shared memory.
-#include <stdlib.h>
 #include <string.h>
 
 #include <vector>
@@ -219,7 +220,7 @@ template <typename T, int NG, int TPB, bool PIPE>
 __global__ void __launch_bounds__(TPB, (TPB <= 512 ? 2 : 1))
     collapse_stream_kernel(const csg_file_desc* __restrict__ files, int n_files, const int32_t* __restrict__ runs,
                            const uint8_t* __restrict__ pa_bits, int n_groups, T* __restrict__ sums,
-                           uint8_t* __restrict__ row_flags, int block_offset) {
+                           uint8_t* __restrict__ row_flags) {
   constexpr int V = VecOf<T>::N;
   constexpr int EV = TPB / kTileRows;  // energy chunks per row
   constexpr int E = EV * V;
@@ -227,10 +228,9 @@ __global__ void __launch_bounds__(TPB, (TPB <= 512 ? 2 : 1))
   T* s_out = reinterpret_cast<T*>(smem_raw);  // [(NG+1)][E][kOutPitch]; PIPE: first the threads' load slots [16][TPB] x 16 B
   __shared__ unsigned s_flags[kTileRows];
 
-  const int blk = (int)blockIdx.x + block_offset;  // a launch may cover a sub-range of the table's blocks
-  const int fi = find_file(files, n_files, blk);
+  const int fi = find_file(files, n_files, blockIdx.x);
   const csg_file_desc f = files[fi];
-  const int t0 = (blk - f.first_block) * kTileRows;
+  const int t0 = (blockIdx.x - f.first_block) * kTileRows;
   const int rows_here = min(kTileRows, f.T - t0);
   const int r = threadIdx.x / EV, c = threadIdx.x - r * EV;
   if (threadIdx.x < kTileRows) s_flags[threadIdx.x] = 0;
@@ -690,32 +690,21 @@ int launch_tpe(csg_ctx* ctx, const csg_file_desc* d_files, int n_files, int tota
 }
 
 // The cp.async pipeline needs 256 bytes of shared memory per thread; two blocks per SM must still
-// fit, so it is used for blocks of up to 384 threads (E = 96 float32 / 48 float64 -- the FAST
-// tables).  CSG_K1_PIPE=0 selects the register-staged variant (A/B measurements).
-inline bool stream_pipe_enabled(int tpb) {
-  static int env = -1;
-  if (env < 0) {
-    const char* e = getenv("CSG_K1_PIPE");
-    env = (e && e[0] == '0') ? 0 : 1;
-  }
-  return env == 1 && (size_t)tpb * 256 <= 100 * 1024;
-}
-
+// fit, so blocks of up to 384 threads (E = 96 float32 / 48 float64 -- the FAST tables) take it and
+// larger blocks (e.g. E = 96 float64) the register-staged body.  The block size fixes the body, so
+// only that one is instantiated.
 template <typename T, int NG, int TPB>
 int launch_stream_one(csg_ctx* ctx, size_t smem, const csg_file_desc* d_files, int n_files, int total_blocks,
-                      const int32_t* d_runs, const uint8_t* d_pa_bits, int n_groups, T* d_sums, uint8_t* d_row_flags,
-                      int block_offset) {
-  if (stream_pipe_enabled(TPB)) {
+                      const int32_t* d_runs, const uint8_t* d_pa_bits, int n_groups, T* d_sums, uint8_t* d_row_flags) {
+  if constexpr (TPB * 256 <= 100 * 1024) {
     auto kern = collapse_stream_kernel<T, NG, TPB, true>;
     const size_t need = smem > (size_t)TPB * 256 ? smem : (size_t)TPB * 256;
     CSG_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need));
-    kern<<<total_blocks, TPB, need, ctx->stream>>>(d_files, n_files, d_runs, d_pa_bits, n_groups, d_sums, d_row_flags,
-                                                   block_offset);
+    kern<<<total_blocks, TPB, need, ctx->stream>>>(d_files, n_files, d_runs, d_pa_bits, n_groups, d_sums, d_row_flags);
   } else {
     auto kern = collapse_stream_kernel<T, NG, TPB, false>;
     CSG_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<total_blocks, TPB, smem, ctx->stream>>>(d_files, n_files, d_runs, d_pa_bits, n_groups, d_sums, d_row_flags,
-                                                   block_offset);
+    kern<<<total_blocks, TPB, smem, ctx->stream>>>(d_files, n_files, d_runs, d_pa_bits, n_groups, d_sums, d_row_flags);
   }
   CSG_LAUNCH_CHECK(ctx, "collapse_stream_kernel");
   return CSG_OK;
@@ -723,12 +712,11 @@ int launch_stream_one(csg_ctx* ctx, size_t smem, const csg_file_desc* d_files, i
 
 template <typename T, int NG>
 int launch_stream_ng(csg_ctx* ctx, int tpb, size_t smem, const csg_file_desc* d_files, int n_files, int total_blocks,
-                     const int32_t* d_runs, const uint8_t* d_pa_bits, int n_groups, T* d_sums, uint8_t* d_row_flags,
-                     int block_offset) {
+                     const int32_t* d_runs, const uint8_t* d_pa_bits, int n_groups, T* d_sums, uint8_t* d_row_flags) {
 #define CSG_GO(TPB)                                                                                                   \
   case TPB:                                                                                                           \
     return launch_stream_one<T, NG, TPB>(ctx, smem, d_files, n_files, total_blocks, d_runs, d_pa_bits, n_groups, d_sums, \
-                                         d_row_flags, block_offset);
+                                         d_row_flags);
   switch (tpb) {
     CSG_GO(256)
     CSG_GO(384)
@@ -742,20 +730,19 @@ int launch_stream_ng(csg_ctx* ctx, int tpb, size_t smem, const csg_file_desc* d_
 
 template <typename T>
 int launch_stream(csg_ctx* ctx, int E, int dtype, const csg_file_desc* d_files, int n_files, int total_blocks,
-                  const int32_t* d_runs, const uint8_t* d_pa_bits, int n_groups, T* d_sums, uint8_t* d_row_flags,
-                  int block_offset) {
+                  const int32_t* d_runs, const uint8_t* d_pa_bits, int n_groups, T* d_sums, uint8_t* d_row_flags) {
   const int tpb = stream_tpb(E, dtype);
   const size_t smem = stream_smem(E, n_groups, dtype);
   if (tpb == 0 || smem > 200 * 1024)
     return csg_fail(ctx, CSG_ERR_ARG, "stream kernel cannot handle E=%d: use CSG_K1_GENERIC for this table", E);
   if (n_groups == 0)
     return launch_stream_ng<T, 0>(ctx, tpb, smem, d_files, n_files, total_blocks, d_runs, d_pa_bits, n_groups, d_sums,
-                                  d_row_flags, block_offset);
+                                  d_row_flags);
   if (n_groups <= 4)
     return launch_stream_ng<T, 4>(ctx, tpb, smem, d_files, n_files, total_blocks, d_runs, d_pa_bits, n_groups, d_sums,
-                                  d_row_flags, block_offset);
+                                  d_row_flags);
   return launch_stream_ng<T, CSG_MAX_GROUPS>(ctx, tpb, smem, d_files, n_files, total_blocks, d_runs, d_pa_bits, n_groups,
-                                             d_sums, d_row_flags, block_offset);
+                                             d_sums, d_row_flags);
 }
 
 template <typename T>
@@ -830,13 +817,6 @@ int64_t csg_sums_elems(int32_t T, int32_t E, int n_groups) {
 int csg_collapse(csg_ctx* ctx, const csg_file_desc* d_files, int n_files, int total_blocks,
                  const uint8_t* d_pa_bits, const int32_t* d_runs, int n_groups, int max_P, int max_E, int dtype,
                  int layout, int kernel, void* d_sums, uint8_t* d_row_flags) {
-  return csg_collapse_range(ctx, d_files, n_files, 0, total_blocks, d_pa_bits, d_runs, n_groups, max_P, max_E, dtype, layout,
-                            kernel, d_sums, d_row_flags);
-}
-
-int csg_collapse_range(csg_ctx* ctx, const csg_file_desc* d_files, int n_files, int block_offset, int total_blocks,
-                       const uint8_t* d_pa_bits, const int32_t* d_runs, int n_groups, int max_P, int max_E, int dtype,
-                       int layout, int kernel, void* d_sums, uint8_t* d_row_flags) {
   if (!ctx) return CSG_ERR_ARG;
   if (n_groups < 0 || n_groups > CSG_MAX_GROUPS) return csg_fail(ctx, CSG_ERR_ARG, "n_groups %d out of range", n_groups);
   if (n_groups > 0 && !d_pa_bits) return csg_fail(ctx, CSG_ERR_ARG, "d_pa_bits is NULL with n_groups > 0");
@@ -850,16 +830,14 @@ int csg_collapse_range(csg_ctx* ctx, const csg_file_desc* d_files, int n_files, 
       if (!d_runs) return csg_fail(ctx, CSG_ERR_ARG, "d_runs is NULL for the stream kernel");
       if (dtype == CSG_F32)
         return launch_stream<float>(ctx, max_E, dtype, d_files, n_files, total_blocks, d_runs, d_pa_bits, n_groups,
-                                    (float*)d_sums, d_row_flags, block_offset);
+                                    (float*)d_sums, d_row_flags);
       return launch_stream<double>(ctx, max_E, dtype, d_files, n_files, total_blocks, d_runs, d_pa_bits, n_groups,
-                                   (double*)d_sums, d_row_flags, block_offset);
+                                   (double*)d_sums, d_row_flags);
     }
-    if (block_offset != 0) return csg_fail(ctx, CSG_ERR_ARG, "block sub-ranges are only supported by the stream kernel");
     if (dtype == CSG_F32)
       return launch_tpe<float>(ctx, d_files, n_files, total_blocks, d_pa_bits, n_groups, max_P, (float*)d_sums, d_row_flags);
     return launch_tpe<double>(ctx, d_files, n_files, total_blocks, d_pa_bits, n_groups, max_P, (double*)d_sums, d_row_flags);
   }
-  if (block_offset != 0) return csg_fail(ctx, CSG_ERR_ARG, "block sub-ranges are only supported by the stream kernel");
   if (kernel == CSG_K1_STREAM) {  // the row kernel: total only, 8 <= P <= 128, P % 8 == 0 (csg_collapse_kernel_for)
     if (n_groups != 0 || max_P > 128 || max_P % 8 != 0)
       return csg_fail(ctx, CSG_ERR_ARG, "the TEP row kernel needs n_groups = 0 and P a multiple of 8 up to 128");

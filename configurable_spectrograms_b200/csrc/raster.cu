@@ -245,10 +245,6 @@ constexpr int kPixPerThread = 16;
 constexpr int kPixPerBlock = kRasterThreads * kPixPerThread;
 constexpr int kRows = kThr + 2;       // thr[-1] = -inf, thr[0..256], thr[257] = +inf
 constexpr int kLutRows = 260;
-#ifndef CSG_K3_PIPE
-#define CSG_K3_PIPE 0
-#endif
-constexpr bool kPipe = CSG_K3_PIPE != 0;  // software-pipeline the pixel loop by one group
 
 __device__ __forceinline__ float fast_log2(float x) {
   float r;
@@ -288,7 +284,7 @@ template <typename T>
 __global__ void __launch_bounds__(kRasterThreads, sizeof(T) == 4 ? 3 : 2)
     rasterise_kernel(const T* __restrict__ mats, const csg_region* __restrict__ regions,
                      const int32_t* __restrict__ pool, const csg_panel* __restrict__ panels,
-                     const csg_panel_norm* __restrict__ norms, int n_panels, int chunk_offset, int n_chunks,
+                     const csg_panel_norm* __restrict__ norms, int chunk_offset, int n_chunks,
                      const int32_t* __restrict__ block_panel, const T* __restrict__ thresholds,
                      const uint32_t* __restrict__ lut, uint32_t* __restrict__ rgba, uint16_t* __restrict__ index) {
   extern __shared__ __align__(16) unsigned char s_raw[];
@@ -340,20 +336,7 @@ __global__ void __launch_bounds__(kRasterThreads, sizeof(T) == 4 ? 3 : 2)
 
   for (int chunk = c_begin; chunk < c_end; ++chunk) {
     const int blk = chunk + chunk_offset;
-    int pi;
-    if (block_panel != nullptr) {
-      pi = __ldg(block_panel + blk);
-    } else {
-      int lo = 0, hi = n_panels - 1;
-      while (lo < hi) {
-        const int mid = (lo + hi + 1) >> 1;
-        if (__ldg(&panels[mid].first_block) <= blk)
-          lo = mid;
-        else
-          hi = mid - 1;
-      }
-      pi = lo;
-    }
+    const int pi = __ldg(block_panel + blk);
     if (pi != cur_panel) {
       cur_panel = pi;
       const csg_panel* pn = panels + pi;
@@ -500,8 +483,6 @@ __global__ void __launch_bounds__(kRasterThreads, sizeof(T) == 4 ? 3 : 2)
         i += STEP, j += dq, tt += dr;
         if (tt >= nt) tt -= nt, ++j;
       };
-      // full groups; with kPipe the loop is software-pipelined by one (the next group's cells are requested
-      // before the current group is classified)
       auto classify_store = [&](unsigned at, T* v) {
         int x[G];
         bool ok = true;
@@ -516,40 +497,24 @@ __global__ void __launch_bounds__(kRasterThreads, sizeof(T) == 4 ? 3 : 2)
         }
         store4(at, x);
       };
-      if constexpr (kPipe) {
+      // full groups, two per trip: both loads are in flight before either group is classified (the kernel is
+      // bound by the latency of these loads, not by issue slots: ncu long-scoreboard stall 10-12 per issue)
+      while (i + STEP + (G - 1) < last) {
+        T a[G], b[G];
+        const unsigned ia = i;
+        load4(j, tt, a);
+        advance();
+        const unsigned ib = i;
+        load4(j, tt, b);
+        advance();
+        classify_store(ia, a);
+        classify_store(ib, b);
+      }
+      while (i + (G - 1) < last) {
         T cur[G];
-        bool have = i + (G - 1) < last;
-        if (have) load4(j, tt, cur);
-        while (have) {
-          const unsigned at = i;
-          advance();
-          T nxt[G];
-          have = i + (G - 1) < last;
-          if (have) load4(j, tt, nxt);
-          classify_store(at, cur);
-#pragma unroll
-          for (unsigned u = 0; u < G; ++u) cur[u] = nxt[u];
-        }
-      } else {
-        // two groups per trip: both loads are in flight before either group is classified (the kernel is
-        // bound by the latency of these loads, not by issue slots: ncu long-scoreboard stall 10-12 per issue)
-        while (i + STEP + (G - 1) < last) {
-          T a[G], b[G];
-          const unsigned ia = i;
-          load4(j, tt, a);
-          advance();
-          const unsigned ib = i;
-          load4(j, tt, b);
-          advance();
-          classify_store(ia, a);
-          classify_store(ib, b);
-        }
-        while (i + (G - 1) < last) {
-          T cur[G];
-          load4(j, tt, cur);
-          classify_store(i, cur);
-          advance();
-        }
+        load4(j, tt, cur);
+        classify_store(i, cur);
+        advance();
       }
       if (i < last) {  // the last, partial group of the panel (i was advanced past every full group)
         unsigned jj = j, t = tt;
@@ -631,7 +596,7 @@ int csg_rasterise(csg_ctx* ctx, const void* d_mats, int dtype, const csg_region*
                   const int32_t* d_block_panel, const uint8_t* d_lut, uint8_t* d_rgba, uint16_t* d_index) {
   if (!ctx) return CSG_ERR_ARG;
   if (n_panels <= 0 || total_blocks <= 0) return CSG_OK;
-  if (!d_mats || !d_regions || !d_index_pool || !d_panels || !d_norms || !d_thresholds)
+  if (!d_mats || !d_regions || !d_index_pool || !d_panels || !d_norms || !d_thresholds || !d_block_panel)
     return csg_fail(ctx, CSG_ERR_ARG, "NULL argument");
   if (d_rgba && !d_lut) return csg_fail(ctx, CSG_ERR_ARG, "d_rgba requested without d_lut");
   // persistent blocks: as many as fit the SMs at once (shared memory allows 2-3 per SM), each a contiguous chunk range
@@ -650,11 +615,11 @@ int csg_rasterise(csg_ctx* ctx, const void* d_mats, int dtype, const csg_region*
   if (grid > total_blocks) grid = total_blocks;
   if (dtype == CSG_F32)
     rasterise_kernel<float><<<grid, kRasterThreads, raster_smem_bytes<float>(), ctx->stream>>>(
-        (const float*)d_mats, d_regions, d_index_pool, d_panels, d_norms, n_panels, block_offset, total_blocks, d_block_panel,
+        (const float*)d_mats, d_regions, d_index_pool, d_panels, d_norms, block_offset, total_blocks, d_block_panel,
         (const float*)d_thresholds, (const uint32_t*)d_lut, (uint32_t*)d_rgba, d_index);
   else if (dtype == CSG_F64)
     rasterise_kernel<double><<<grid, kRasterThreads, raster_smem_bytes<double>(), ctx->stream>>>(
-        (const double*)d_mats, d_regions, d_index_pool, d_panels, d_norms, n_panels, block_offset, total_blocks, d_block_panel,
+        (const double*)d_mats, d_regions, d_index_pool, d_panels, d_norms, block_offset, total_blocks, d_block_panel,
         (const double*)d_thresholds, (const uint32_t*)d_lut, (uint32_t*)d_rgba, d_index);
   else
     return csg_fail(ctx, CSG_ERR_ARG, "bad dtype %d", dtype);

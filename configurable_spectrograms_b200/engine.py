@@ -345,36 +345,6 @@ class Batch:
         self._tables_dirty = True
         return len(todo)
 
-    def piece_blocks(self, file_bounds):
-        """Block ranges of K1 for pieces of the file list: ``file_bounds`` = ascending file indices
-        f_0 = 0 < f_1 < ... < f_k = n_files.  Returns ``[(block_offset, n_blocks)]`` or None when the
-        shard is not one stream-kernel table in file order (then it is collapsed in one launch)."""
-        if self._tables_dirty:
-            self._build_file_tables()
-        if len(self.d_files) != 1:
-            return None
-        (layout, kern, _e), (_tab, n, blocks, _mp, _me) = next(iter(self.d_files.items()))
-        if kern != _lib.K1_STREAM or layout != _lib.LAYOUT_TPE or n != len(self.files):
-            return None
-        per_file = [self.ctx.lib.csg_collapse_blocks(f["T"], f["P"], f["E"], self.code, layout, kern) for f in self.files]
-        first = np.concatenate([[0], np.cumsum(per_file)])
-        return [(int(first[a]), int(first[b] - first[a])) for a, b in zip(file_bounds[:-1], file_bounds[1:])]
-
-    def collapse_piece(self, block_offset: int, n_blocks: int, first: bool):
-        """K1 over a block sub-range of the (single, stream-kernel) file table."""
-        if first:
-            self.d_flags.zero()
-        if n_blocks <= 0:
-            return
-        (layout, kern, _e), (tab, n, _blocks, max_p, max_e) = next(iter(self.d_files.items()))
-        self.ctx._check(
-            self.ctx.lib.csg_collapse_range(
-                self.ctx.handle, tab.ptr, n, block_offset, n_blocks, self.d_bits.ptr,
-                self.d_runs.ptr if self.d_runs is not None else None, self.G, max_p, max_e, self.code, layout, kern,
-                self.d_sums.ptr, self.d_flags.ptr,
-            )
-        )
-
     def mat_off(self, file: int, group: int) -> int:
         """Element offset of the file's energy-major [E][Tp] matrix of one group in the sums buffer."""
         f = self.files[file]
@@ -551,9 +521,6 @@ class Batch:
                            for p in dev], dtype=np.int64)
         first = np.concatenate([[0], np.cumsum(blocks)[:-1]])
         dev["first_block"] = first
-        self._dev_first = np.concatenate([first, [int(blocks.sum())]])  # block range of device panel k: [k], [k+1]
-        # device position of the free (slot-less) panels, in logical order: pieces of the shard address them by range
-        self._free_logical = np.flatnonzero(free)
         # region-stat references stay valid (they index regions, not panels)
         self._dev_order = order
         self._n_free = int(free.sum())
@@ -574,18 +541,14 @@ class Batch:
         self._panels[panel] = tuple(p)
 
     # ------------------------------------------------------------------ stages
-    def run_stats(self, ctx=None, lo: int = 0, hi: int | None = None):
-        """K2a over the regions [lo, hi) (default: all), on ``ctx``'s stream (default: the batch's)."""
+    def run_stats(self):
+        """K2a over every region."""
         if not self._regions:
             return
-        ctx = ctx or self.ctx
-        hi = len(self._regions) if hi is None else hi
-        if hi <= lo:
-            return
-        ctx._check(
-            ctx.lib.csg_region_stats_run(
-                ctx.handle, self.d_sums.ptr, self.code, self.d_regions.ptr + lo * REGION.itemsize, hi - lo,
-                self.d_pool.ptr, self.d_stats.ptr + lo * REGION_STATS.itemsize,
+        self.ctx._check(
+            self.ctx.lib.csg_region_stats_run(
+                self.ctx.handle, self.d_sums.ptr, self.code, self.d_regions.ptr, len(self._regions), self.d_pool.ptr,
+                self.d_stats.ptr,
             )
         )
 
@@ -636,42 +599,6 @@ class Batch:
                 self.d_norms.ptr + p0 * PANEL_NORM.itemsize, self.d_thr.ptr + p0 * thr_one,
             )
         )
-
-    def free_panels_before(self, logical_panel: int) -> int:
-        """How many slot-free panels have a logical id below ``logical_panel`` = where such panels start
-        in the device order (they come first, in logical order)."""
-        return int(np.searchsorted(self._free_logical, logical_panel))
-
-    def ensure_outputs(self, want_rgba: bool, want_index: bool):
-        if want_rgba and self.d_lut is None:
-            raise CsgError("set_lut() before rasterise(want_rgba=True)")
-        if want_rgba and (self.d_rgba is None or self.d_rgba.nbytes < self._pixels * 4):
-            self.d_rgba = self.ctx.alloc(max(self._pixels, 1) * 4)
-        if want_index and (self.d_index is None or self.d_index.nbytes < self._pixels * 2):
-            self.d_index = self.ctx.alloc(max(self._pixels, 1) * 2)
-
-    def run_free_panels(self, ctx, lo: int, hi: int, want_rgba: bool, want_index: bool):
-        """Prepare + K3 for the device-order panels [lo, hi) (all slot-free: hi <= number of free
-        panels) on ``ctx``'s stream.  Output buffers must exist (:meth:`ensure_outputs`)."""
-        if hi <= lo:
-            return
-        thr_one = ctx.lib.csg_threshold_bytes(1, self.code)
-        ctx._check(
-            ctx.lib.csg_panel_prepare(
-                ctx.handle, self.d_panels.ptr + lo * PANEL.itemsize, hi - lo, self.d_regions.ptr, self.d_stats.ptr,
-                self.code, None, self.d_norms.ptr + lo * PANEL_NORM.itemsize, self.d_thr.ptr + lo * thr_one,
-            )
-        )
-        b0, b1 = int(self._dev_first[lo]), int(self._dev_first[hi])
-        if b1 > b0:
-            ctx._check(
-                ctx.lib.csg_rasterise(
-                    ctx.handle, self.d_sums.ptr, self.code, self.d_regions.ptr, self.d_pool.ptr, self.d_panels.ptr,
-                    self.d_norms.ptr, self.d_thr.ptr, len(self._panels), b1 - b0, b0, self.d_block_panel.ptr,
-                    self.d_lut.ptr if self.d_lut is not None else None,
-                    self.d_rgba.ptr if want_rgba else None, self.d_index.ptr if want_index else None,
-                )
-            )
 
     def norms(self) -> np.ndarray:
         """Resolved normalisation of every panel, indexed by panel id."""

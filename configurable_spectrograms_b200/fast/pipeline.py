@@ -486,9 +486,7 @@ class BatchStep:
                 if v is not None:
                     slotted[key] = self._slots[(inst, name)] = b.zslot(v)
         self.figure_ranges = {}  # (orbit, with_extrema) -> [first, last) in shard.figures
-        self._marks = []  # per orbit of the shard: (first file, first region, first panel) it owns
         for ob in sh.orbits:
-            self._marks.append((min(ob["files"].values(), default=len(b.files)), len(b._regions), len(b._panels)))
             if self.plot_orbits is not None and ob["orbit"] not in self.plot_orbits:
                 continue
             for with_extrema in self.submissions:  # batch_directory.py:237-243
@@ -504,7 +502,6 @@ class BatchStep:
                 sh.plan_instrument_grid(ob, "given", global_extrema=slotted if with_extrema else None)
                 sh.plan_instrument_grid(ob, "raw", global_extrema=None)
                 self.figure_ranges[(ob["orbit"], with_extrema)] = (first, len(sh.figures))
-        self._marks.append((len(b.files), len(b._regions), len(b._panels)))
         sh.upload_tables()
         if self.lut is not None:
             b.set_lut(self.lut)
@@ -519,35 +516,6 @@ class BatchStep:
                 if slot is not None:
                     b.set_zslot(slot.slot, v)
 
-    def _pieces(self):
-        """Split the shard into a few runs of consecutive orbits: ``[(K1 block offset, K1 blocks, region
-        lo, region hi, free-panel lo, free-panel hi)]``, or None when the shard cannot be collapsed in
-        pieces (mixed layouts / kernels, files out of order, a single orbit).  ``CSG_PIECES`` sets the
-        count.  Default 1 = off: measured on B200 (125 orbits) the overlap LOSES -- 3.29 ms per step in
-        one piece, 3.47 / 3.60 / 3.71 ms in 2 / 4 / 8 pieces: K1 already keeps HBM at 90 % of the read
-        ceiling, so K2a / K3 blocks sharing its SMs only take occupancy and bandwidth away from it."""
-        import os
-
-        want = int(os.environ.get("CSG_PIECES", "1"))
-        marks = getattr(self, "_marks", None)
-        b = self.shard.batch
-        if want <= 1 or not marks or len(marks) < 3:
-            return None
-        files = [m[0] for m in marks]
-        if any(a > c for a, c in zip(files[:-1], files[1:])) or files[0] != 0:
-            return None
-        n_orbits = len(marks) - 1
-        k = min(want, n_orbits)
-        cuts = sorted({round(i * n_orbits / k) for i in range(k + 1)})
-        blocks = b.piece_blocks([marks[c][0] for c in cuts])
-        if blocks is None:
-            return None
-        out = []
-        for (off, n), c0, c1 in zip(blocks, cuts[:-1], cuts[1:]):
-            out.append((off, n, marks[c0][1], marks[c1][1], b.free_panels_before(marks[c0][2]),
-                        b.free_panels_before(marks[c1][2])))
-        return out
-
     def run(self, cache_state: dict | None = None, state: dict | None = None, collapse: bool = True) -> dict:
         """Enqueue one whole step; returns the extrema state (rasters stay on the device).
 
@@ -559,21 +527,7 @@ class BatchStep:
         planned = self._sig is not None
         want_rgba = b.d_lut is not None
         early = False
-        pieces = self._pieces() if (planned and collapse) else None
-        worker = None
-        if pieces:
-            # K1 runs piece by piece on the main stream; as soon as a piece is collapsed the worker
-            # stream takes its K2a and the K3 of its slot-free panels -- issue-bound work that shares
-            # the SMs with the next piece's HBM-bound collapse instead of queueing behind it
-            worker = b.ctx.worker_context()
-            b.ensure_outputs(want_rgba, self.want_index)
-            for i, (off, n, r_lo, r_hi, p_lo, p_hi) in enumerate(pieces):
-                b.collapse_piece(off, n, first=i == 0)
-                worker.wait_for(b.ctx)
-                b.run_stats(worker, r_lo, r_hi)
-                b.run_free_panels(worker, p_lo, p_hi, want_rgba, self.want_index)
-            early = True
-        elif collapse:
+        if collapse:
             sh.collapse()
 
         def independent_stages():
@@ -581,8 +535,6 @@ class BatchStep:
             # panels that read no z slot (the raw variants) -- the GPU stays busy while the host
             # turns the pooled results into bounds
             b.run_windows()
-            if pieces:
-                return
             b.run_stats()
             b.prepare(part=0)
             # with several ranks the digit loop and its peer exchanges are still running on the side stream
@@ -612,8 +564,6 @@ class BatchStep:
         bounds = self._bounds(state)
         sig = self._signature(bounds)
         if sig != self._sig:
-            if worker is not None:
-                worker.sync()  # the tables it reads are about to be rebuilt
             self._plan(state, bounds)
             self._sig = sig
             b.run_windows()
@@ -621,8 +571,6 @@ class BatchStep:
             early = False
         else:
             self._update_slots(bounds)
-            if worker is not None:
-                b.ctx.wait_for(worker)  # K2a / slot-free rasters of every piece are done before the rest
         want_rgba = b.d_lut is not None
         if early:
             b.prepare(part=1)

@@ -403,7 +403,7 @@ def _device_tables(figures, dpi):
 
 
 def encode_figures_device(ctx, d_rgba_ptr: int, figures, dpi: float | None = None, max_segments: int = 400_000, consume=None,
-                          timings: dict | None = None, huffman: str = "custom", wait: bool = True, code_cache: dict | None = None,
+                          timings: dict | None = None, wait: bool = True, code_cache: dict | None = None,
                           paths=None, write_threads: int = 16, defer: bool = False):
     """PNG bytes of every figure, composed and DEFLATE-encoded on the GPU.
 
@@ -418,11 +418,11 @@ def encode_figures_device(ctx, d_rgba_ptr: int, figures, dpi: float | None = Non
     ``consume(first_figure_index, parts)``: instead of returning the files, hand every group's files
     -- each a list of buffers, some aliasing pinned scratch that is valid only during the call -- to the
     caller (``write_figures_device`` writes them straight to disk without assembling them in memory).
-    ``timings`` (optional dict) accumulates host seconds per phase.  ``huffman``: "custom" fits a
-    dynamic-Huffman code to the symbol statistics of the first group of figures (one counting pass of
-    the same tokeniser over every 4th scanline segment) and uses it for the whole call; "fixed" uses
-    RFC 1951's fixed code.  ``code_cache`` (a dict the caller keeps): the fitted code is stored there and
-    reused by later calls instead of being fitted again (the chunks of one directory run look alike).
+    ``timings`` (optional dict) accumulates host seconds per phase.  The DEFLATE code is a dynamic-Huffman
+    code fitted to the symbol statistics of the first group of figures (one counting pass of the same
+    tokeniser over every 4th scanline segment) and used for the whole call.  ``code_cache`` (a dict the
+    caller keeps): the fitted code is stored there and reused by later calls instead of being fitted again
+    (the chunks of one directory run look alike).
 
     ``paths`` (one per figure): frame and write the files natively (``csg_png_write_files``: CRC-32 +
     ``writev`` from the pinned buffer on ``write_threads`` native threads, no interpreter lock held) instead of
@@ -496,9 +496,9 @@ def encode_figures_device(ctx, d_rgba_ptr: int, figures, dpi: float | None = Non
         table = np.array([tuple(c) for c in group], dtype=PNG_CANVAS)
         d_canvases = ctx.to_device(table)
         if k == 0:  # the code of this call
-            if huffman == "custom" and code_cache is not None and "tables" in code_cache:
+            if code_cache is not None and "tables" in code_cache:
                 ctx._check(lib.csg_png_set_tables(ctx.handle, code_cache["tables"].ctypes.data))
-            elif huffman == "custom":
+            else:
                 d_counts = dev("counts", 316 * 4)
                 d_counts.zero()
                 ctx._check(lib.csg_png_set_tables(ctx.handle, None))  # the count pass needs valid symbol tables
@@ -508,10 +508,6 @@ def encode_figures_device(ctx, d_rgba_ptr: int, figures, dpi: float | None = Non
                 ctx._check(lib.csg_png_set_tables(ctx.handle, tables.ctypes.data))
                 if code_cache is not None:
                     code_cache["tables"] = tables
-            elif huffman == "fixed":
-                ctx._check(lib.csg_png_set_tables(ctx.handle, None))
-            else:
-                raise ValueError(f"huffman must be 'custom' or 'fixed', not {huffman!r}")
             t0 = tick("code_tables", t0)
         d_slots, d_sizes, d_adler = dev("slots", n_seg * slot), dev("sizes", n_seg * 4), dev("adler", n_seg * 8)
         ctx._check(lib.csg_png_encode(ctx.handle, d_rgba_ptr, d_overlay, d_canvases.ptr, len(group), d_tiles.ptr, None,

@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define CSG_ABI_VERSION 24
+#define CSG_ABI_VERSION 25
 
 #if defined(__GNUC__)
 #define CSG_API __attribute__((visibility("default")))
@@ -169,12 +169,6 @@ CSG_API int64_t csg_sums_elems(int32_t T, int32_t E, int n_groups);
 CSG_API int csg_collapse(csg_ctx* ctx, const csg_file_desc* d_files, int n_files, int total_blocks,
                  const uint8_t* d_pa_bits, const int32_t* d_runs, int n_groups, int max_P, int max_E,
                  int dtype, int layout, int kernel, void* d_sums, uint8_t* d_row_flags);
-/* The same launch over the blocks [block_offset, block_offset + total_blocks) of the file table
- * (stream kernel only): a shard collapsed in a few pieces lets the statistics and rasters of the
- * files already done run on another stream while the next piece streams from HBM. */
-CSG_API int csg_collapse_range(csg_ctx* ctx, const csg_file_desc* d_files, int n_files, int block_offset, int total_blocks,
-                 const uint8_t* d_pa_bits, const int32_t* d_runs, int n_groups, int max_P, int max_E,
-                 int dtype, int layout, int kernel, void* d_sums, uint8_t* d_row_flags);
 
 /* zoom_needed = np.any(~np.isnan(cube[window])) (CS/plotting.py:597-603) from the row flags:
  * d_out[w] = 1 iff some row of window w has bit `bit` set.  Rows are [t0, t0+nt) when
@@ -277,8 +271,8 @@ CSG_API int csg_panel_prepare(csg_ctx* ctx, const csg_panel* d_panels, int n_pan
 
 /* Launches blocks [block_offset, block_offset + total_blocks) of the panel table's block space
  * (a table can be rasterised in several launches, e.g. the panels whose bounds are known first).
- * d_block_panel (may be NULL): panel index of every thread block, i.e. panel p repeated
- * csg_raster_blocks(ne_p, nt_p) times; without it every block binary-searches first_block.
+ * d_block_panel (required): panel index of every thread block, i.e. panel p repeated
+ * csg_raster_blocks(ne_p, nt_p) times.
  * Clamp -> normalise -> 256-entry LUT index -> RGBA8.  d_lut: 259 x 4 bytes (256 colours,
  * under, over, bad).  d_index (uint16, may be NULL) receives Colormap indices 0..255 and
  * 256/257/258 for under/over/bad; d_rgba (may be NULL) the colours.  Row 0 of a panel is
