@@ -112,6 +112,7 @@ __global__ void __launch_bounds__(288)
   if (g > dom_hi) g = dom_hi;
   U lo, hi;  // invariant once bracketed: code(lo) < k <= code(hi)
   U step = 2;
+  constexpr U kMaxStep = (U)1 << (Key<T>::BITS - 2);  // the gallop saturates: a step that wrapped to 0 would never move
   bool found = true;
   if (code(g) >= k) {
     hi = g;
@@ -123,7 +124,7 @@ __global__ void __launch_bounds__(288)
       lo = (hi - dom_lo > step) ? hi - step : dom_lo;
       if (code(lo) < k) break;
       hi = lo;
-      step <<= 2;
+      if (step < kMaxStep) step <<= 2;
     }
   } else {
     lo = g;
@@ -135,7 +136,7 @@ __global__ void __launch_bounds__(288)
       hi = (dom_hi - lo > step) ? lo + step : dom_hi;
       if (code(hi) >= k) break;
       lo = hi;
-      step <<= 2;
+      if (step < kMaxStep) step <<= 2;
     }
   }
   if (!found) {
@@ -191,6 +192,9 @@ __global__ void panel_prepare_kernel(const csg_panel* __restrict__ panels, int n
     nm.t_range = thi - tlo;
     if (nm.status == CSG_NORM_OK && !nm.degenerate && !(is_finite(tlo) && is_finite(thi)))
       nm.status = CSG_NORM_INVALID;
+    // vmin < vmax a few ulps apart, but log10 rounds both to the same double: every normalised value is
+    // (t - t_vmin) / 0 = +-inf or NaN, which LogNorm masks -> "bad", like a NaN bound
+    if (nm.status == CSG_NORM_OK && !nm.degenerate && nm.t_range == 0.0) nm.degenerate = 2;
   } else {
     nm.fill_lo = (double)(T)zmin;
     nm.fill_hi = (double)(T)zmax;
@@ -219,6 +223,11 @@ __global__ void panel_prepare_kernel(const csg_panel* __restrict__ panels, int n
       nm.status = CSG_NORM_VMIN_GT_VMAX;
     else if (is_nan(zmin) || is_nan(zmax))
       nm.degenerate = 2;  // every normalised value is NaN -> "bad" colour
+    else if (!is_finite(nm.t_range))
+      // vmax - vmin = inf (an infinite percentile bound, or finite bounds whose difference overflows):
+      // (v - vmin) / inf is NaN ("bad") where v - vmin is infinite -- every cell when vmin = -inf -- and 0
+      // elsewhere.  Not a monotone step function of v, so no threshold table: the rasteriser tests each cell.
+      nm.degenerate = is_finite(zmin) ? 3 : 2;
   }
   // first-guess coefficients of the rasteriser: #{thresholds <= v} ~ c1 * (log2 v | v) + c0
   nm.c1 = p.log_scale ? (float)(256.0 * 0.30102999566398120 / nm.t_range) : (float)(256.0 / nm.t_range);
@@ -374,12 +383,20 @@ __global__ void __launch_bounds__(kRasterThreads, sizeof(T) == 4 ? 3 : 2)
     uint32_t* out_rgba = rgba ? rgba + out_off : nullptr;
     uint16_t* out_idx = index ? index + out_off : nullptr;
     if (degenerate != 0) {
-      // vmin == vmax: every cell maps to index 0; NaN bound: every cell is "bad"
-      const int idx = degenerate == 1 ? 0 : I_BAD;
-      const int row = degenerate == 1 ? 1 : 258;
+      // 1: vmin == vmax, every cell maps to index 0; 2: NaN bound, every cell is "bad"; 3 (linear, vmax - vmin
+      // = inf): index 0, or "bad" where the in-place subtraction v - vmin is infinite (inf / inf = NaN)
+      const csg_panel_norm* nm = norms + cur_panel;
+      const double vmin = degenerate == 3 ? __ldg(&nm->t_vmin) : 0.0;
       for (unsigned i = first + tid; i < last; i += kRasterThreads) {
-        if (out_rgba) out_rgba[i] = lut_at(row);
-        if (out_idx) out_idx[i] = (uint16_t)idx;
+        bool bad = degenerate == 2;
+        if (degenerate == 3) {
+          const unsigned jj = i / nt, t = i - jj * nt;
+          T v = __ldg(mat + __ldg(cols + jj) * ld + (rows_off < 0 ? t0 + (int)t : __ldg(rows + t)));
+          v = (is_nan(v) || v == (T)(-CUDART_INF)) ? fill_lo : (v == (T)CUDART_INF ? fill_hi : v);
+          bad = !is_finite((T)((double)v - vmin));
+        }
+        if (out_rgba) out_rgba[i] = lut_at(bad ? 258 : 1);
+        if (out_idx) out_idx[i] = (uint16_t)(bad ? I_BAD : 0);
       }
       continue;
     }

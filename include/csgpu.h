@@ -252,7 +252,8 @@ typedef struct {
   double fill_lo, fill_hi; /* substitutes written into the matrix (already rounded to D)          */
   double t_vmin, t_range;  /* log: log10(vmin), log10(vmax)-log10(vmin); linear: vmin, vmax-vmin  */
   int32_t status;          /* CSG_NORM_*                                                          */
-  int32_t degenerate;      /* 1: vmin == vmax -> every cell maps to index 0; 2: NaN bound -> all "bad" */
+  int32_t degenerate;      /* 1: vmin == vmax -> every cell maps to index 0; 2: NaN bound, or log10(vmin) == log10(vmax) -> all "bad";
+                               3: linear, vmax - vmin = inf -> index 0, "bad" where v - vmin is inf */
   float c0, c1;            /* rasteriser's first-guess coefficients (internal)                    */
 } csg_panel_norm;          /* 64 bytes */
 

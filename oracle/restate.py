@@ -265,6 +265,15 @@ def panel(
         zmin, zmax = compute_percentile_bounds(m, 1, 99, z_min, z_max)  # :259
         fp = m[np.isfinite(m) & (m > 0)]
         safe_vmin = np.nanmin(fp) if fp.size > 0 else 1e-10  # :261-262
+    out = clamp_for_imshow(m, z_scale, zmin, zmax, safe_vmin)
+    out.update(x=x, y=y, safe_vmin=float(safe_vmin))
+    return out
+
+
+def clamp_for_imshow(m, z_scale, zmin, zmax, safe_vmin):
+    """The z clamps of ``make_spectrogram`` (``CS/plotting.py:276-278`` log, ``:307-315`` linear) on the
+    matrix handed to ``imshow``, given the percentile bounds and ``safe_vmin`` already resolved."""
+    with np.errstate(invalid="ignore"):
         if z_scale == "log":
             zmin = float(max(zmin, safe_vmin, 1e-10))  # :276
             zmax = float(zmax)
@@ -280,7 +289,7 @@ def panel(
                 zmin = float(np.nanmin(m))
                 zmax = float(np.nanmax(m))
             mode = "linear"
-    return {"matrix": m, "vmin": zmin, "vmax": zmax, "mode": mode, "x": x, "y": y, "safe_vmin": float(safe_vmin)}
+    return {"matrix": m, "vmin": zmin, "vmax": zmax, "mode": mode}
 
 
 # ----------------------------------------------------------------------------
