@@ -17,6 +17,7 @@ Data layout in HBM (DESIGN.md section 3):
 from __future__ import annotations
 
 import ctypes as C
+from collections import namedtuple
 
 import numpy as np
 
@@ -33,6 +34,18 @@ from ._lib import (
     DevBuf,
     np_dtype_code,
 )
+
+
+#: One row of the region, panel and zoom-window tables, with the fields of the ABI mirror dtypes in
+#: their order: ``np.array(rows, dtype=REGION)`` is the table the kernels read.
+RegionRow = namedtuple("RegionRow", REGION.names)
+PanelRow = namedtuple("PanelRow", PANEL.names)
+WindowRow = namedtuple("WindowRow", FLAG_WINDOW.names)
+
+#: ``csg_region.want_pct``: what K2a computes for a region
+WANT_REDUCTIONS, WANT_PERCENTILES, WANT_GEOMETRY = 0, 1, 2
+# a region asked for more than once keeps the most it was asked for
+_WANT_RANK = {WANT_GEOMETRY: 0, WANT_REDUCTIONS: 1, WANT_PERCENTILES: 2}
 
 
 def _align(n: int, a: int = 256) -> int:
@@ -94,8 +107,8 @@ class Batch:
         self.code = np_dtype_code(dtype)
         self.G = int(n_groups)
         self.files: list[dict] = []
-        self._regions: list[tuple] = []
-        self._panels: list[tuple] = []
+        self._regions: list[RegionRow] = []
+        self._panels: list[PanelRow] = []
         self._pool: list[np.ndarray] = []
         self._pool_len = 0
         self._pool_cache: dict[bytes, int] = {}
@@ -122,7 +135,7 @@ class Batch:
         self.d_lut: DevBuf | None = None
         self.d_thr: DevBuf | None = None
         self.d_zvals: DevBuf | None = None
-        self._windows: list[tuple] = []
+        self._windows: list[WindowRow] = []
         self.d_windows: DevBuf | None = None
         self.d_window_any: DevBuf | None = None
         self._zvals: list[float] = []
@@ -359,14 +372,9 @@ class Batch:
         a = self.d_sums.download(self.dtype, n, self.mat_off(file, group) * self.dtype.itemsize)
         return np.ascontiguousarray(a.reshape(f["E"], f["Tp"])[:, : f["T"]].T)
 
-    def all_flags(self) -> np.ndarray:
-        return self.d_flags.download(np.uint8, self._flags_bytes)
-
-    def flags(self, file: int, flags_host: np.ndarray | None = None) -> np.ndarray:
+    def flags(self, file: int) -> np.ndarray:
         f = self.files[file]
-        if flags_host is None:
-            return self.d_flags.download(np.uint8, f["T"], f["flags_off"]) if f["T"] else np.zeros(0, np.uint8)
-        return flags_host[f["flags_off"] : f["flags_off"] + f["T"]]
+        return self.d_flags.download(np.uint8, f["T"], f["flags_off"]) if f["T"] else np.zeros(0, np.uint8)
 
     # ---------------------------------------------------------------- regions
     def _pool_add(self, idx: np.ndarray) -> int:
@@ -389,8 +397,8 @@ class Batch:
         self.d_regions = self.d_panels = self.d_windows = self.d_window_any = None
 
     def add_region(self, file: int, group: int, cols, *, t0: int = 0, nt: int | None = None, rows=None,
-                   want_pct: bool | int = False, p_lo: float = 1.0, p_hi: float = 99.0) -> int:
-        """``want_pct``: 0/False reductions only, 1/True + percentiles, 2 geometry only (no stats)."""
+                   want_pct: bool | int = WANT_REDUCTIONS, p_lo: float = 1.0, p_hi: float = 99.0) -> int:
+        """``want_pct``: ``WANT_REDUCTIONS`` (or False), ``WANT_PERCENTILES`` (or True) or ``WANT_GEOMETRY``."""
         f = self.files[file]
         cols = np.asarray(cols, dtype=np.int32)
         if rows is not None:
@@ -408,9 +416,23 @@ class Batch:
             t0, nt = 0, len(rows)
         cols_off = self._pool_add(cols) if len(cols) else 0
         self._regions.append(
-            (self.mat_off(file, group), f["Tp"], t0, nt, rows_off, cols_off, len(cols), int(want_pct), 0, float(p_lo), float(p_hi))
+            RegionRow(mat_off=self.mat_off(file, group), ld=f["Tp"], t0=t0, nt=nt, rows_off=rows_off, cols_off=cols_off,
+                      ne=len(cols), want_pct=int(want_pct), reserved=0, p_lo=float(p_lo), p_hi=float(p_hi))
         )
         return len(self._regions) - 1
+
+    def require_stats(self, region: int, want_pct: int):
+        """Make K2a compute at least ``want_pct`` for a region, in the order geometry < reductions <
+        percentiles; a region never loses what it was already asked for."""
+        r = self._regions[region]
+        if _WANT_RANK[int(want_pct)] > _WANT_RANK[r.want_pct]:
+            self._regions[region] = r._replace(want_pct=int(want_pct))
+
+    def drop_reductions(self, region: int):
+        """A region whose reductions no panel reads any more becomes geometry only (percentiles stay)."""
+        r = self._regions[region]
+        if r.want_pct == WANT_REDUCTIONS:
+            self._regions[region] = r._replace(want_pct=WANT_GEOMETRY)
 
     def zslot(self, value=None) -> ZSlot:
         """A new slot of the per-step z-bound table (``None`` = not given -> percentile bound)."""
@@ -436,7 +458,7 @@ class Batch:
                 t0, nt, rows_off = int(rows[0]), len(rows), -1
             else:
                 t0, nt, rows_off = 0, len(rows), (self._pool_add(rows) if len(rows) else -1)
-        self._windows.append((f["flags_off"], t0, nt, rows_off, int(bit)))
+        self._windows.append(WindowRow(flags_off=f["flags_off"], t0=t0, nt=nt, rows_off=rows_off, bit=int(bit)))
         return len(self._windows) - 1
 
     def run_windows(self):
@@ -450,6 +472,12 @@ class Batch:
             )
         )
 
+    def window_any(self) -> np.ndarray:
+        """Download the result of :meth:`run_windows`: uint8 per window."""
+        if not self._windows:
+            return np.zeros(0, np.uint8)
+        return self.d_window_any.download(np.uint8, len(self._windows))
+
     def _pool_array(self) -> np.ndarray:
         if getattr(self, "_pool_flat_len", -1) != self._pool_len:
             self._pool_flat = np.concatenate(self._pool) if self._pool else np.zeros(0, np.int32)
@@ -459,39 +487,45 @@ class Batch:
     def region_energy_index(self, region: int) -> np.ndarray:
         """Energy channel of every image row of a region (lowest energy first)."""
         r = self._regions[region]
-        return self._pool_array()[r[5] : r[5] + r[6]]
-
-    def region_time_index(self, region: int) -> np.ndarray:
-        """Time step of every image column of a region."""
-        r = self._regions[region]
-        if r[4] < 0:
-            return np.arange(r[2], r[2] + r[3])
-        return self._pool_array()[r[4] : r[4] + r[3]]
+        return self._pool_array()[r.cols_off : r.cols_off + r.ne]
 
     def region_time_ends(self, region: int) -> tuple[int, int]:
         """Time steps of the first and last image column of a region."""
         r = self._regions[region]
-        if r[4] < 0:
-            return r[2], r[2] + r[3] - 1
+        if r.rows_off < 0:
+            return r.t0, r.t0 + r.nt - 1
         pool = self._pool_array()
-        return int(pool[r[4]]), int(pool[r[4] + r[3] - 1])
+        return int(pool[r.rows_off]), int(pool[r.rows_off + r.nt - 1])
 
     def add_panel(self, region: int, pct_region: int = -1, log_scale: bool = False, z_min=None, z_max=None,
                   stat_region: int = -1) -> int:
         r = self._regions[region]
-        ne, nt = r[6], r[3]
         self._panels.append(
-            (region, pct_region, int(bool(log_scale)), self._raster_blocks,
-             np.nan if z_min is None else float(z_min), np.nan if z_max is None else float(z_max), self._pixels,
-             stat_region, 0, z_min.slot if isinstance(z_min, ZSlot) else -1, z_max.slot if isinstance(z_max, ZSlot) else -1)
+            PanelRow(region=region, pct_region=pct_region, log_scale=int(bool(log_scale)), first_block=self._raster_blocks,
+                     z_min=np.nan if z_min is None else float(z_min), z_max=np.nan if z_max is None else float(z_max),
+                     out_off=self._pixels, stat_region=stat_region, reserved=0,
+                     zmin_slot=z_min.slot if isinstance(z_min, ZSlot) else -1,
+                     zmax_slot=z_max.slot if isinstance(z_max, ZSlot) else -1)
         )
-        self._raster_blocks += self.ctx.lib.csg_raster_blocks(ne, nt)
-        self._pixels += (ne * nt + 3) & ~3  # every panel starts 16-byte aligned: 128-bit RGBA stores
+        self._raster_blocks += self.ctx.lib.csg_raster_blocks(r.ne, r.nt)
+        self._pixels += (r.ne * r.nt + 3) & ~3  # every panel starts 16-byte aligned: 128-bit RGBA stores
         return len(self._panels) - 1
 
+    def set_stat_region(self, panel: int, region: int):
+        """Take a panel's reductions (safe_vmin, nanmin / nanmax) from ``region`` instead of its own region."""
+        self._panels[panel] = self._panels[panel]._replace(stat_region=region)
+
+    def panel_region(self, panel: int) -> int:
+        """The region a panel draws."""
+        return self._panels[panel].region
+
+    def panel_offset(self, panel: int) -> int:
+        """First pixel of a panel in the batch's RGBA / index buffers."""
+        return self._panels[panel].out_off
+
     def panel_shape(self, panel: int) -> tuple[int, int]:
-        r = self._regions[self._panels[panel][0]]
-        return r[6], r[3]
+        r = self._regions[self._panels[panel].region]
+        return r.ne, r.nt
 
     def upload_tables(self):
         """Region / panel / index tables -> device (call after the last add_*)."""
@@ -517,8 +551,7 @@ class Batch:
         free = (logical["zmin_slot"] < 0) & (logical["zmax_slot"] < 0)
         order = np.concatenate([np.flatnonzero(free), np.flatnonzero(~free)])
         dev = logical[order]
-        blocks = np.array([self.ctx.lib.csg_raster_blocks(self._regions[p["region"]][6], self._regions[p["region"]][3])
-                           for p in dev], dtype=np.int64)
+        blocks = np.array([self.ctx.lib.csg_raster_blocks(*self.panel_shape(p)) for p in order], dtype=np.int64)
         first = np.concatenate([[0], np.cumsum(blocks)[:-1]])
         dev["first_block"] = first
         # region-stat references stay valid (they index regions, not panels)
@@ -533,12 +566,6 @@ class Batch:
         thr_bytes = self.ctx.lib.csg_threshold_bytes(n, self.code)
         if self.d_thr is None or self.d_thr.nbytes < thr_bytes:
             self.d_thr = self.ctx.alloc(thr_bytes)
-
-    def set_panel_bounds(self, panel: int, z_min=None, z_max=None):
-        p = list(self._panels[panel])
-        p[4] = np.nan if z_min is None else float(z_min)
-        p[5] = np.nan if z_max is None else float(z_max)
-        self._panels[panel] = tuple(p)
 
     # ------------------------------------------------------------------ stages
     def run_stats(self):
@@ -604,7 +631,10 @@ class Batch:
         """Resolved normalisation of every panel, indexed by panel id."""
         if not self._panels:
             return np.zeros(0, PANEL_NORM)
-        dev = self.d_norms.download(PANEL_NORM, len(self._panels))
+        return self.by_panel(self.d_norms.download(PANEL_NORM, len(self._panels)))
+
+    def by_panel(self, dev: np.ndarray) -> np.ndarray:
+        """Rows of a per-panel table in device order (see :meth:`upload_panels`), reordered by panel id."""
         out = np.empty_like(dev)
         out[self._dev_order] = dev
         return out
@@ -639,13 +669,11 @@ class Batch:
 
     def panel_index(self, panel: int) -> np.ndarray:
         ne, nt = self.panel_shape(panel)
-        off = self._panels[panel][6]
-        return self.d_index.download(np.uint16, ne * nt, off * 2).reshape(ne, nt)
+        return self.d_index.download(np.uint16, ne * nt, self.panel_offset(panel) * 2).reshape(ne, nt)
 
     def panel_rgba(self, panel: int) -> np.ndarray:
         ne, nt = self.panel_shape(panel)
-        off = self._panels[panel][6]
-        return self.d_rgba.download(np.uint8, ne * nt * 4, off * 4).reshape(ne, nt, 4)
+        return self.d_rgba.download(np.uint8, ne * nt * 4, self.panel_offset(panel) * 4).reshape(ne, nt, 4)
 
     def all_rgba(self) -> np.ndarray:
         return self.d_rgba.download(np.uint8, self._pixels * 4)
@@ -660,6 +688,10 @@ class Batch:
     @property
     def n_panels(self) -> int:
         return len(self._panels)
+
+    @property
+    def n_windows(self) -> int:
+        return len(self._windows)
 
     @property
     def n_pixels(self) -> int:
@@ -711,9 +743,10 @@ def matrix_percentiles(matrix: np.ndarray, p_lo, p_hi, ctx: Context | None = Non
     if n == 0:
         return float("nan"), float("nan")
     d_m = ctx.to_device(flat)
-    reg = np.zeros(1, dtype=REGION)
-    reg[0] = (0, n, 0, n, -1, 0, 1, 1, 0, float(p_lo), float(p_hi))  # one energy row holding every cell
-    d_r = ctx.to_device(reg)
+    # one energy row holding every cell
+    reg = RegionRow(mat_off=0, ld=n, t0=0, nt=n, rows_off=-1, cols_off=0, ne=1, want_pct=WANT_PERCENTILES, reserved=0,
+                    p_lo=float(p_lo), p_hi=float(p_hi))
+    d_r = ctx.to_device(np.array([reg], dtype=REGION))
     d_pool = ctx.to_device(np.zeros(1, dtype=np.int32))
     d_out = ctx.alloc(REGION_STATS.itemsize)
     ctx._check(ctx.lib.csg_region_stats_run(ctx.handle, d_m.ptr, np_dtype_code(flat.dtype), d_r.ptr, 1, d_pool.ptr, d_out.ptr))

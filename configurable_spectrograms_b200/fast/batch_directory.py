@@ -35,7 +35,7 @@ from ..logging_utils import configure_log_batch, flush_log_buffer, log_exception
 from .constants import DEFAULT_INSTRUMENT_ORDER, FAST_CDF_DATA_FOLDER_PATH, FAST_OUTPUT_BASE, FAST_PLOTTING_PROGRESS_JSON
 from .extrema import compute_global_extrema
 from .orbit_discovery import _add_to_orbit_list, _classify_error_reason, _parse_year_month, discover_orbit_files
-from .pipeline import BatchStep, ShardPlan
+from .pipeline import BatchStep, ShardPlan, chunk_orbits, ingest_orbits
 from .plotting import figure_from_spec
 from .process_orbit import SAVE_DPI, figure_filename
 
@@ -164,15 +164,6 @@ def _render_threads(n_threads: int) -> int:
         return 1
 
 
-def _chunk_orbits_default() -> int:
-    """Orbits per streaming chunk (``CSG_CHUNK_ORBITS``): a nominal 4-instrument orbit is 84 MB of cubes,
-    so the default keeps one pinned slot / the device staging buffer near 0.7 GB."""
-    try:
-        return max(1, int(os.environ.get("CSG_CHUNK_ORBITS", "8")))
-    except ValueError:
-        return 8
-
-
 def _run_directory(directory_path, output_base, y_scale, z_scale, zoom_duration_minutes, instrument_order, verbose,
                    progress_json_path, ignore_progress_json, colormap, cusp_marker_style, cusp_marker_kwargs, max_workers,
                    flush_batch_size, log_flush_batch_size, max_processing_percentile, override_plots,
@@ -246,17 +237,11 @@ def _run_directory(directory_path, output_base, y_scale, z_scale, zoom_duration_
     shard = ShardPlan(ctx, y_scale, z_scale, zoom_duration_minutes, instrument_order=instrument_order)
     shard.first_orbit_index = lo
     load_errors: dict[int, list[str]] = {}
-    loaded_orbits: list[int] = []
 
-    # ---- phase A: streaming ingest.  Loader threads decode the next chunk's files straight into a pinned
-    # staging slot while the copy engine uploads the previous chunk and K1 collapses it; neither host RAM
-    # nor HBM ever holds more cubes than the slots of the ring (the sums and row flags of every orbit stay)
-    chunk_n = _chunk_orbits_default()
-    chunks = [list(range(a, min(a + chunk_n, len(mine)))) for a in range(0, len(mine), chunk_n)]
-    slot_bytes = int(os.environ.get("CSG_SLOT_BYTES", str(max(1 << 28, chunk_n * 100 * (1 << 20)))))
-    ring = _lib.shared_ring(ctx, n_slots=3, slot_bytes=slot_bytes) if chunks else None
-
-    def load_one(slot, index):
+    # ---- phase A: streaming ingest (pipeline.ingest_orbits): loader threads decode the next chunk's files
+    # into a pinned staging slot while the previous chunk is uploaded and collapsed; the sums and row flags of
+    # every orbit stay in HBM
+    def load_one(index, alloc):
         orbit, files = mine[index]
         wanted = set(scan_needs.get(lo + index, ()))
         if orbit in pending_set:
@@ -270,40 +255,24 @@ def _run_directory(directory_path, output_base, y_scale, z_scale, zoom_duration_
                 detected = get_cdf_file_type(path)
                 if detected is None or detected == "orb":
                     continue
-                ds = load_fast_cdf_dataset(path, data_alloc=lambda shape, dtype: ring.alloc(slot, shape, dtype))
+                ds = load_fast_cdf_dataset(path, data_alloc=alloc)
                 datasets[inst] = ds
                 lines[inst] = get_timestamps_for_orbit(frame, orbit, detected, ds["times"])
             except Exception as exc:
                 err = f"[FAIL] Plotting Orbit {orbit} pitch angle grid for {inst}"
                 log_exception(err, exc, level="error")
                 errors.append(err)
-        return orbit, datasets, lines, errors
+        if errors:
+            load_errors[orbit] = errors
+        return orbit, datasets, lines
+
+    def refused(orbit, exc):  # a cube of another float dtype than the shard's: refused, not cast
+        err = f"[FAIL] Orbit {orbit} processing"
+        log_exception(err, exc, level="error")
+        load_errors.setdefault(orbit, []).append(err)
 
     t_phase = tick("discover_and_resume", t_phase)
-    with ThreadPoolExecutor(max_workers=n_threads) as pool:
-        def submit(k):
-            slot = ring.acquire()
-            return slot, [pool.submit(load_one, slot, i) for i in chunks[k]]
-
-        in_flight = submit(0) if chunks else None
-        for k in range(len(chunks)):
-            slot, futures = in_flight
-            loaded = [f.result() for f in futures]
-            # the next chunk decodes while this one is registered, uploaded and collapsed
-            in_flight = submit(k + 1) if k + 1 < len(chunks) else None
-            for orbit, datasets, lines, errors in loaded:
-                if errors:
-                    load_errors.setdefault(orbit, []).extend(errors)
-                try:
-                    shard.add_orbit(orbit, datasets, lines)
-                except TypeError as exc:  # a cube of another float dtype than the shard's: refused, not cast
-                    err = f"[FAIL] Orbit {orbit} processing"
-                    log_exception(err, exc, level="error")
-                    load_errors.setdefault(orbit, []).append(err)
-                    shard.add_orbit(orbit, {}, {})
-                loaded_orbits.append(orbit)
-            shard.collapse_pending()
-            ring.release(slot)
+    ingest_orbits(shard, range(len(mine)), load_one, refused, n_threads=n_threads)
     if world > 1:
         # one pool, one key width: every rank computes in the same dtype.  A rank without orbits of its own
         # (more GPUs than orbits) adopts its peers'; ranks that read cubes of different float dtypes cannot
@@ -317,14 +286,8 @@ def _run_directory(directory_path, output_base, y_scale, z_scale, zoom_duration_
         if shard._dtype is None and kinds:
             shard._dtype = np.dtype(kinds[0])
             shard._batch = None
-    if not chunks:  # such a rank still joins the extrema exchange, with empty outputs of K1
+    if not mine:  # such a rank still joins the extrema exchange, with empty outputs of K1
         shard.collapse_pending()
-    if ring is not None:
-        if ring.overflow_bytes:
-            log_exception(f"[INGEST] {ring.overflow_bytes} bytes of cubes did not fit the pinned slots "
-                          f"({slot_bytes} bytes each; CSG_SLOT_BYTES / CSG_CHUNK_ORBITS) and were uploaded from pageable memory",
-                          level="message")
-        ring.drain()  # the ring belongs to the context and serves the next call too
     # ranks that loaded only part of the sequence still index it globally
     if not need_extrema:
         shard.first_orbit_index = 0
@@ -343,8 +306,9 @@ def _run_directory(directory_path, output_base, y_scale, z_scale, zoom_duration_
     # ---- phase C: the figures, chunk by chunk: K2a + K3 for the chunk's panels, the figures planned on host
     # threads from panel references, composed and PNG-encoded on the device (K4: no raster ever crosses PCIe
     # uncompressed), files written, progress recorded -- an interrupt loses at most the chunk in flight
-    loaded_set = set(loaded_orbits)
+    loaded_set = {orbit for orbit, _files in mine}
     my_pending = [o for o in pending if o in loaded_set]
+    chunk_n = chunk_orbits()
     submissions = (False, True) if need_extrema else (False,)
     lut = get_lut(colormap)
     b = shard.batch

@@ -621,44 +621,28 @@ def compute_global_extrema(
     if shard is None:
         needs = orbits_the_scan_needs(sequence, instrument_order, y_scale, z_scale, state, log_floor_cutoff, log_floor_value)
         if needs:
-            from concurrent.futures import ThreadPoolExecutor
-
             from .. import _lib
-            from .pipeline import ShardPlan
+            from .pipeline import ShardPlan, ingest_orbits
 
-            ctx = _lib.default_context()
-            shard = ShardPlan(ctx, y_scale, z_scale, instrument_order=instrument_order)
+            shard = ShardPlan(_lib.default_context(), y_scale, z_scale, instrument_order=instrument_order)
             shard.first_orbit_index = 0
-            chunk_n = max(1, int(os.environ.get("CSG_CHUNK_ORBITS", "8")))
-            ring = _lib.shared_ring(ctx, n_slots=3, slot_bytes=int(os.environ.get("CSG_SLOT_BYTES", str(max(1 << 28, chunk_n * 100 * (1 << 20))))))
 
-            def load_one(slot, oi):
+            def load_one(oi, alloc):
                 datasets = {}
                 for inst in needs.get(oi, ()):
                     path = orbit_files[orbits[oi]].get(inst)
                     if path is None:
                         continue
                     try:
-                        datasets[inst] = load_fast_cdf_dataset(path, data_alloc=lambda shape, dtype: ring.alloc(slot, shape, dtype))
+                        datasets[inst] = load_fast_cdf_dataset(path, data_alloc=alloc)
                     except Exception as exc:
                         log_exception(f"[EXTREMA] Ingest failure inst={inst} orbit={orbits[oi]} file={path}", exc, level="message")
-                return datasets
+                return orbits[oi], datasets, None
 
-            try:
-                with ThreadPoolExecutor(max_workers=4) as pool:
-                    for a in range(0, len(orbits), chunk_n):
-                        slot = ring.acquire()
-                        loaded = list(pool.map(lambda oi: load_one(slot, oi), range(a, min(a + chunk_n, len(orbits)))))
-                        for oi, datasets in zip(range(a, a + len(loaded)), loaded):
-                            try:
-                                shard.add_orbit(orbits[oi], datasets)
-                            except TypeError as exc:
-                                log_exception(f"[EXTREMA] Ingest failure orbit={orbits[oi]}", exc, level="message")
-                                shard.add_orbit(orbits[oi], {})
-                        shard.collapse_pending()
-                        ring.release(slot)
-            finally:
-                ring.drain()
+            def refused(orbit, exc):
+                log_exception(f"[EXTREMA] Ingest failure orbit={orbit}", exc, level="message")
+
+            ingest_orbits(shard, range(len(orbits)), load_one, refused)
     if shard is None:
         # nothing reaches the scan (everything re-used or complete): only the bookkeeping runs
         totals = {i: sum(1 for _, h in sequence if i in h) for i in instrument_order}

@@ -14,12 +14,13 @@ inline) so that panels, bounds and figure/file naming are identical.
 
 from __future__ import annotations
 
+import os
 from dataclasses import dataclass, field
 
 import numpy as np
 
 from .. import _lib
-from ..engine import Batch
+from ..engine import WANT_GEOMETRY, WANT_PERCENTILES, WANT_REDUCTIONS, Batch
 from .constants import DEFAULT_INSTRUMENT_ORDER, DEFAULT_PITCH_ANGLE_CATEGORIES, PITCH_ANGLE_ROW_KEYS
 
 
@@ -100,7 +101,6 @@ class ShardPlan:
         self._region_cache: dict = {}
         self._cols_cache: dict = {}
         self._full_stats: dict = {}  # (file, group) -> percentile region over the [0,4000] eV cells, every row
-        self._flags_host = None
         self._window_cache: dict = {}
         self._full_region_of: dict = {}  # region id -> (file, group) for full panels over every time row
 
@@ -164,9 +164,6 @@ class ShardPlan:
         the last call; their cubes are not kept, neither on the host nor in HBM."""
         return self.batch.collapse_pending()
 
-    def fetch_flags(self):
-        self._flags_host = self.batch.all_flags()
-
     # ------------------------------------------------------------ phase 2: panels
     def _energy_cols(self, file: int, lo, hi):
         """Columns kept by ``(E >= lo) & (E <= hi)`` (builder order, no flip) and the same
@@ -193,12 +190,7 @@ class ShardPlan:
                 rid = self.batch.add_region(file, group, cols, rows=rows, want_pct=want_pct)
             self._region_cache[key] = rid
         else:
-            r = list(self.batch._regions[rid])
-            # 2 = geometry only < 0 = reductions < 1 = reductions + percentiles
-            order = {2: 0, 0: 1, 1: 2}
-            if order[int(want_pct)] > order[r[7]]:
-                r[7] = int(want_pct)
-                self.batch._regions[rid] = tuple(r)
+            self.batch.require_stats(rid, want_pct)
         return rid
 
     def _panel(self, region, pct_region, z_min, z_max, stat_region=-1):
@@ -266,7 +258,7 @@ class ShardPlan:
         pct = -1
         if z_lo is None or z_hi is None:
             # compute_percentile_bounds(matrix_full_plot, 1, 99, z_min, z_max) on the builder matrix
-            pct = self._region(file, group, builder_cols, "full", (0, len(meta["times"])), True)
+            pct = self._region(file, group, builder_cols, "full", (0, len(meta["times"])), WANT_PERCENTILES)
         # make_spectrogram always clips energy to [0, 4000] here: y_axis_min/max are not
         # forwarded by generic_plot_multirow_optional_zoom (plotting.py:618-636 vs :104-105)
         plain, cols = self._energy_cols(file, 0, 4000)
@@ -279,14 +271,14 @@ class ShardPlan:
             n_rows = rows[1] if isinstance(rows, tuple) else len(rows)
             if n_rows:
                 shared = self._full_stats.get((file, group), -1) if isinstance(rows, tuple) else -1
-                reg = self._region(file, group, cols, rk, rows, 2 if shared >= 0 else 0)
+                reg = self._region(file, group, cols, rk, rows, WANT_GEOMETRY if shared >= 0 else WANT_REDUCTIONS)
                 if isinstance(rows, tuple):
                     self._full_region_of[reg] = (file, group)
                 row.full_panel = self._panel(reg, pct, z_lo, z_hi, shared)
             if zoom is not None:
                 rk, rows = self._rows_zoom(file, zoom)
                 if len(rows):
-                    reg = self._region(file, group, cols, rk, rows, False)
+                    reg = self._region(file, group, cols, rk, rows, WANT_REDUCTIONS)
                     row.zoom_panel = self._panel(reg, pct, z_lo, z_hi)
         row.vmin, row.vmax = z_lo, z_hi
         fig.rows.append(row)
@@ -364,33 +356,37 @@ class ShardPlan:
         reads any more become geometry only -- K2a touches every cell set once instead of twice."""
         b = self.batch
         own = set()
-        for pid, p in enumerate(b._panels):
-            region, stat_region = p[0], p[7]
+        for (region, _pct, _lo, _hi, stat_region), pid in self._panel_cache.items():  # every panel of the plan
             if stat_region < 0:
                 shared = self._full_stats.get(self._full_region_of.get(region))
                 if shared is not None and shared != region:
-                    q = list(p)
-                    q[7] = shared
-                    b._panels[pid] = tuple(q)
+                    b.set_stat_region(pid, shared)
                     continue
                 own.add(region)
-        for rid, r in enumerate(b._regions):
-            if r[7] == 0 and rid not in own and rid in self._full_region_of:
-                q = list(r)
-                q[7] = 2
-                b._regions[rid] = tuple(q)
+        for rid in self._full_region_of:
+            if rid not in own:
+                b.drop_reductions(rid)
 
     def upload_tables(self):
         self.share_full_stats()
         self.batch.upload_tables()
 
     def run_panels(self, lut259=None, want_index=True):
+        """K2a, panel norms and K3 over the uploaded tables (``lut259=None``: the LUT already set)."""
         b = self.batch
         b.run_stats()
         b.prepare()
         if lut259 is not None:
             b.set_lut(lut259)
         b.rasterise(want_rgba=lut259 is not None or b.d_lut is not None, want_index=want_index)
+
+    def run_once(self, lut259, want_index=True):
+        """Compute every planned figure of a collapsed shard once: tables, zoom windows, :meth:`run_panels`,
+        then the figures' ``zoom_needed`` flags (the rasters stay on the device)."""
+        self.upload_tables()
+        self.batch.run_windows()
+        self.run_panels(lut259, want_index)
+        self.resolve_zoom_flags(self.batch.window_any())
 
     def pool_items(self, steps_by_inst: dict[str, list[int]]):
         """POOL_ITEM table for the scanned (orbit index) steps of every instrument."""
@@ -412,6 +408,64 @@ class ShardPlan:
             inst_len[ii] = pos
         items = np.array(rows, dtype=POOL_ITEM) if rows else np.zeros(0, POOL_ITEM)
         return items, inst_len, owners
+
+
+def chunk_orbits() -> int:
+    """Orbits per streaming chunk (``CSG_CHUNK_ORBITS``, default 8; a malformed value means the default): a
+    nominal 4-instrument orbit is 84 MB of cubes, so the default keeps one pinned slot / the device staging
+    buffer near 0.7 GB."""
+    try:
+        return max(1, int(os.environ.get("CSG_CHUNK_ORBITS", "8")))
+    except ValueError:
+        return 8
+
+
+def ingest_orbits(shard: ShardPlan, indices, load, refused, n_threads: int = 4):
+    """Streaming ingest: add the orbits ``indices`` to ``shard`` and collapse them, :func:`chunk_orbits` at a time.
+
+    ``load(index, alloc) -> (orbit, datasets, lines)`` runs on one of ``n_threads`` loader threads and decodes
+    the orbit's cubes into ``alloc(shape, dtype)``: pinned memory of the chunk's staging slot.  Chunk k+1 is
+    decoded while chunk k is uploaded and collapsed (``ShardPlan.collapse_pending``), so neither host RAM nor
+    HBM holds more cubes than the three slots of the context's ring (``CSG_SLOT_BYTES`` each).  An orbit whose
+    cubes ``add_orbit`` refuses (a float dtype other than the shard's) goes to ``refused(orbit, exc)`` and is
+    added without files."""
+    from concurrent.futures import ThreadPoolExecutor
+    from functools import partial
+
+    from ..logging_utils import log_exception
+
+    indices = list(indices)
+    if not indices:
+        return
+    chunk_n = chunk_orbits()
+    chunks = [indices[a : a + chunk_n] for a in range(0, len(indices), chunk_n)]
+    slot_bytes = int(os.environ.get("CSG_SLOT_BYTES", str(max(1 << 28, chunk_n * 100 * (1 << 20)))))
+    ring = _lib.shared_ring(shard.ctx, n_slots=3, slot_bytes=slot_bytes)
+    try:
+        with ThreadPoolExecutor(max_workers=n_threads) as pool:
+            def submit(chunk):
+                slot = ring.acquire()
+                return slot, [pool.submit(load, i, partial(ring.alloc, slot)) for i in chunk]
+
+            in_flight = submit(chunks[0])
+            for k in range(len(chunks)):
+                slot, futures = in_flight
+                loaded = [f.result() for f in futures]
+                in_flight = submit(chunks[k + 1]) if k + 1 < len(chunks) else None
+                for orbit, datasets, lines in loaded:
+                    try:
+                        shard.add_orbit(orbit, datasets, lines)
+                    except TypeError as exc:
+                        refused(orbit, exc)
+                        shard.add_orbit(orbit, {}, {})
+                shard.collapse_pending()
+                ring.release(slot)
+    finally:
+        ring.drain()  # the ring belongs to the context and serves the next call too
+    if ring.overflow_bytes:
+        log_exception(f"[INGEST] {ring.overflow_bytes} bytes of cubes did not fit the pinned slots "
+                      f"({slot_bytes} bytes each; CSG_SLOT_BYTES / CSG_CHUNK_ORBITS) and were uploaded from pageable memory",
+                      level="message")
 
 
 class BatchStep:
@@ -505,8 +559,7 @@ class BatchStep:
         sh.upload_tables()
         if self.lut is not None:
             b.set_lut(self.lut)
-        n_win = len(b._windows)
-        self._win_pin = b.ctx.pinned(max(n_win, 1))
+        self._win_pin = b.ctx.pinned(max(b.n_windows, 1))
 
     def _update_slots(self, bounds):
         b = self.shard.batch
@@ -578,8 +631,8 @@ class BatchStep:
         else:
             b.prepare()
             b.rasterise(want_rgba=want_rgba, want_index=self.want_index)
-        if b._windows:
-            b.ctx._check(b.ctx.lib.csg_d2h(b.ctx.handle, self._win_pin.ptr, b.d_window_any.ptr, len(b._windows)))
+        if b.n_windows:
+            b.ctx._check(b.ctx.lib.csg_d2h(b.ctx.handle, self._win_pin.ptr, b.d_window_any.ptr, b.n_windows))
         self.state = state
         return state
 
@@ -587,25 +640,29 @@ class BatchStep:
         """Wait for the step and fill the figures' ``zoom_needed`` flags."""
         b = self.shard.batch
         b.ctx.sync()
-        if b._windows:
-            self.shard.resolve_zoom_flags(self._win_pin.view(np.uint8, len(b._windows)))
+        if b.n_windows:
+            self.shard.resolve_zoom_flags(self._win_pin.view(np.uint8, b.n_windows))
         return self.state
 
 
 def _k3_shared_blocks() -> int:
     """K3 blocks per SM while the extrema chain runs beside it (``CSG_K3_SHARED_BLOCKS``, default 2; 0 = no cap)."""
-    import os
-
     try:
         return max(0, int(os.environ.get("CSG_K3_SHARED_BLOCKS", "2")))
     except ValueError:
         return 2
 
 
-def check_norm_status(norm_row, what: str):
-    """Raise what matplotlib would raise at draw time for an invalid panel normalisation."""
+def check_norm_status(norm_row, what: str | None = None):
+    """Raise what matplotlib would raise at draw time for an invalid panel normalisation; ``what`` names
+    the panel and adds its bounds to the message."""
     st = int(norm_row["status"])
     if st == _lib.NORM_VMIN_GT_VMAX:
-        raise ValueError(f"vmin must be less or equal to vmax ({what}: vmin={norm_row['vmin']}, vmax={norm_row['vmax']})")
-    if st == _lib.NORM_INVALID:
-        raise ValueError(f"Invalid vmin or vmax ({what}: vmin={norm_row['vmin']}, vmax={norm_row['vmax']})")
+        msg = "vmin must be less or equal to vmax"
+    elif st == _lib.NORM_INVALID:
+        msg = "Invalid vmin or vmax"
+    else:
+        return
+    if what is not None:
+        msg += f" ({what}: vmin={norm_row['vmin']}, vmax={norm_row['vmax']})"
+    raise ValueError(msg)

@@ -27,12 +27,12 @@ __all__ = ["FAST_plot_pitch_angle_grid", "FAST_plot_instrument_grid", "figure_fr
 
 
 def figure_from_spec(shard: ShardPlan, spec: FigureSpec, colormap="viridis", cusp_marker_style="both",
-                     cusp_marker_kwargs=None, norms=None, rgba_flat=None, index_flat=None, device_rasters=False):
+                     cusp_marker_kwargs=None, norms=None, device_rasters=False):
     """Compose the figure ``generic_plot_multirow_optional_zoom`` would return for one planned
     figure (reference ``plotting.py:583-698``) from the shard's finished rasters.
 
-    ``norms`` / ``rgba_flat`` / ``index_flat``: the batch's downloaded tables (bulk D2H by the
-    batch driver); fetched per panel when omitted.  ``device_rasters``: the panels stay in HBM
+    ``norms``: the batch's downloaded normalisations (``Batch.norms``), fetched when omitted; the
+    rasters are downloaded per panel.  ``device_rasters``: the panels stay in HBM
     (``figure.DeviceRaster`` references into the batch's RGBA buffer) and the figure is meant for
     ``png.encode_figures_device``.  Raises the ``ValueError`` matplotlib would raise at draw time
     for an invalid normalisation.
@@ -52,20 +52,9 @@ def figure_from_spec(shard: ShardPlan, spec: FigureSpec, colormap="viridis", cus
             axes[i, j] = fig.add_subplot(n_rows, n_cols, i * n_cols + j + 1)
 
     def raster(pid):
-        ne, nt = b.panel_shape(pid)
-        off = b._panels[pid][6]
         if device_rasters:
-            return DeviceRaster(off, ne, nt), None
-        if rgba_flat is not None:
-            rgba = rgba_flat[off * 4 : (off + ne * nt) * 4].reshape(ne, nt, 4)
-        else:
-            rgba = b.panel_rgba(pid)
-        index = None
-        if index_flat is not None:
-            index = index_flat[off : off + ne * nt].reshape(ne, nt)
-        elif rgba_flat is None and b.d_index is not None:
-            index = b.panel_index(pid)
-        return rgba, index
+            return DeviceRaster(b.panel_offset(pid), *b.panel_shape(pid)), None
+        return b.panel_rgba(pid), (b.panel_index(pid) if b.d_index is not None else None)
 
     log_scale = shard.z_scale == "log"
     for i, row in enumerate(spec.rows):
@@ -76,7 +65,7 @@ def figure_from_spec(shard: ShardPlan, spec: FigureSpec, colormap="viridis", cus
             check_norm_status(nm, f"orbit {spec.orbit} {spec.kind} {row.label}")
             rgba, index = raster(pid)
             # the axes only need the ends of the panel's time and energy ranges (extent, limits, markers)
-            region = b._panels[pid][0]
+            region = b.panel_region(pid)
             t_first, t_last = b.region_time_ends(region)
             e_index = b.region_energy_index(region)
             y_kept = row.energy[e_index[[0, -1]]] if len(e_index) > 2 else row.energy[e_index]
@@ -120,12 +109,7 @@ class _Ends:
 def _run_single(shard: ShardPlan, spec: FigureSpec, colormap, cusp_marker_style, cusp_marker_kwargs):
     if not spec.rows:
         return None, None
-    b = shard.batch
-    shard.upload_tables()
-    b.run_windows()
-    shard.run_panels(get_lut(colormap), want_index=True)
-    if b._windows:
-        shard.resolve_zoom_flags(b.d_window_any.download(np.uint8, len(b._windows)))
+    shard.run_once(get_lut(colormap), want_index=True)
     return figure_from_spec(shard, spec, colormap, cusp_marker_style, cusp_marker_kwargs)
 
 

@@ -14,8 +14,6 @@ import os
 import time as _time
 from typing import Any
 
-import numpy as np
-
 from .. import _lib
 from ..cdf_utils import get_cdf_file_type, get_timestamps_for_orbit, load_fast_cdf_dataset
 from ..colormaps import get_lut
@@ -137,12 +135,8 @@ def FAST_process_single_orbit(
             shard.upload()
             shard.collapse()
             specs = plan_orbit_figures(shard, shard.orbits[0], global_extrema)
+            shard.run_once(get_lut(colormap), want_index=False)
             b = shard.batch
-            shard.upload_tables()
-            b.run_windows()
-            shard.run_panels(get_lut(colormap), want_index=False)
-            if b._windows:
-                shard.resolve_zoom_flags(b.d_window_any.download(np.uint8, len(b._windows)))
             norms = b.norms()
             group_start, group_key = _time.time(), None
             for spec in specs:

@@ -25,6 +25,7 @@ from .colormaps import get_lut
 from .constants import AXIS_LABEL_FONT_SIZE, PLOT_FIGURE_HEIGHT_INCHES, PLOT_FIGURE_WIDTH_INCHES, TICK_LABEL_FONT_SIZE
 from .cusp_marking import draw_cusp_both_markers, draw_cusp_bracket_marker, draw_cusp_line_markers
 from .engine import Batch
+from .fast.pipeline import check_norm_status, zoom_window
 from .figure import FigureCanvas, SpectrogramFigure, close_all_axes_and_clear
 from .logging_utils import log_message
 
@@ -223,11 +224,7 @@ def _resolved_bounds(norm, stats, log_scale):
     """``(vmin, vmax)`` of a panel's resolved normalisation; raises what matplotlib raises when the figure is
     drawn with an invalid one, and logs the reference's warning for a log panel that holds non-positive cells
     (``:264-275``)."""
-    status = int(norm["status"])
-    if status == _lib.NORM_VMIN_GT_VMAX:
-        raise ValueError("vmin must be less or equal to vmax")
-    if status == _lib.NORM_INVALID:
-        raise ValueError("Invalid vmin or vmax")
+    check_norm_status(norm)
     z_lo, z_hi = float(norm["vmin"]), float(norm["vmax"])
     if log_scale and stats is not None:
         if stats["n_pos"] < stats["n_valid"] + stats["n_nan"] or not (np.isfinite(z_lo) and z_hi > z_lo > 0):
@@ -282,7 +279,7 @@ class SpectrogramGroup:
             try:
                 z_lo, z_hi = _resolved_bounds(norms[panel], stats[region] if log_scale else None, log_scale)
                 ne, nt = batch.panel_shape(panel)
-                draw_panel(axis_object, DeviceRaster(batch._panels[panel][6], ne, nt), None, z_lo, z_hi, log_scale, x_axis_plot,
+                draw_panel(axis_object, DeviceRaster(batch.panel_offset(panel), ne, nt), None, z_lo, z_hi, log_scale, x_axis_plot,
                            y_kept, **annotate)
                 axis_object.images[-1].batch = batch  # which RGBA buffer the raster lives in
                 outcome.append(None)
@@ -429,16 +426,6 @@ def generic_plot_spectrogram_set(
     return fig, canvas
 
 
-def zoom_window_from_lines(vertical_lines, zoom_duration_minutes):
-    """(centre, duration) of the zoom column, or ``None`` without lines (reference ``:586-596``)."""
-    if not vertical_lines:
-        return None
-    if len(vertical_lines) == 1:
-        return vertical_lines[0], zoom_duration_minutes * 60
-    centre = 0.5 * (vertical_lines[0] + vertical_lines[1])
-    return centre, max(zoom_duration_minutes * 60, abs(vertical_lines[1] - vertical_lines[0]) * 1.5)
-
-
 def generic_plot_multirow_optional_zoom(
     datasets,
     vertical_lines=None,
@@ -467,7 +454,7 @@ def generic_plot_multirow_optional_zoom(
         return None, None
     zoom_needed = False
     centre = duration = None
-    zoom = zoom_window_from_lines(vertical_lines, zoom_duration_minutes) if vertical_lines is not None and len(vertical_lines) > 0 else None
+    zoom = zoom_window(vertical_lines, zoom_duration_minutes) if vertical_lines is not None and len(vertical_lines) > 0 else None
     if zoom is not None:
         centre, duration = zoom
         left, right = centre - duration / 2, centre + duration / 2

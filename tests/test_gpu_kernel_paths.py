@@ -250,7 +250,7 @@ def _check_panels(b, specs, lut, rgba=None, index=None):
             continue
         assert nm["status"] == 0, p
         ne, nt = b.panel_shape(p)
-        off = b._panels[p][6]
+        off = b.panel_offset(p)
         if index is not None:
             assert np.array_equal(index[off : off + ne * nt].reshape(ne, nt), out[0]), (p, ne, nt, log, zlo, zhi)
         if rgba is not None:
@@ -471,7 +471,7 @@ def test_rasterise_linear_panels_with_infinite_range(ctx, dtype):
         assert not np.isfinite(norms["vmax"] - norms["vmin"]).any()
     assert _check_panels(b, specs, lut, rgba=b.all_rgba(), index=b.all_index()) == len(cases)
     idx = b.all_index()
-    off, (ne, nt) = b._panels[2][6], b.panel_shape(2)
+    off, (ne, nt) = b.panel_offset(2), b.panel_shape(2)
     assert {0, 258} <= set(np.unique(idx[off : off + ne * nt]))  # both colours of the infinite range occur
 
 
@@ -590,8 +590,7 @@ def test_threshold_table_and_lookup_at_colour_boundaries(ctx, dtype):
     norms = b.norms()
     n = b.n_panels
     dev = b.d_thr.download(D, n * 264).reshape(n, 264)[:, :257]
-    table = np.empty_like(dev)
-    table[b._dev_order] = dev
+    table = b.by_panel(dev)
     for p, ((log, zlo, zhi), (vmin, thr), Mr) in enumerate(zip(panels, expect, specs)):
         nm = norms[p]
         assert nm["status"] == 0 and nm["vmin"] == vmin and nm["vmax"] == zhi, (p, nm)

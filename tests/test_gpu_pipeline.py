@@ -54,10 +54,7 @@ def test_pitch_angle_grid_matches_reference_captures(ctx):
             shard.upload()
             shard.collapse()
             fig = shard.plan_pitch_angle_grid(shard.orbits[0], "ees", variant, **kw)
-            shard.upload_tables()
-            shard.batch.run_windows()
-            shard.run_panels(lut, want_index=True)
-            shard.resolve_zoom_flags(shard.batch.d_window_any.download(np.uint8, len(shard.batch._windows)))
+            shard.run_once(lut, want_index=True)
             assert fig.zoom_needed
             norms = shard.batch.norms()
             assert len(fig.rows) == 4 and len(ref) == 8
@@ -86,10 +83,7 @@ def test_instrument_grid_matches_reference_captures(ctx):
         shard.upload()
         shard.collapse()
         fig = shard.plan_instrument_grid(shard.orbits[0], tag, global_extrema=ge)
-        shard.upload_tables()
-        shard.batch.run_windows()
-        shard.run_panels(lut, want_index=True)
-        shard.resolve_zoom_flags(shard.batch.d_window_any.download(np.uint8, len(shard.batch._windows)))
+        shard.run_once(lut, want_index=True)
         assert fig.zoom_needed
         norms = shard.batch.norms()
         assert len(ref) == 2 * len(fig.rows)
