@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 # CSG_LIBRARY: another build of the same ABI (A/B experiments: a kernel variant compiled with a different -D)
 LIB_PATH = os.environ.get("CSG_LIBRARY") or os.path.join(HERE, "libcsgpu.so")
 
-ABI_VERSION = 25
+ABI_VERSION = 26
 F32, F64 = 0, 1
 LAYOUT_TPE, LAYOUT_TEP = 0, 1
 K1_GENERIC, K1_STREAM = 0, 1
@@ -118,9 +118,9 @@ FLAG_WINDOW = np.dtype(
 assert FLAG_WINDOW.itemsize == 24
 PNG_TILE = np.dtype(
     [("rgba_off", "<i8"), ("ne", "<i4"), ("nt", "<i4"), ("x", "<i4"), ("y", "<i4"), ("w", "<i4"), ("h", "<i4"),
-     ("vline_first", "<i4"), ("vline_count", "<i4"), ("flags", "<i4"), ("pad", "<i4")], align=True
+     ("vline_first", "<i4"), ("vline_count", "<i4"), ("flags", "<i4"), ("row_map", "<i4")], align=True
 )
-TILE_OVERLAY, TILE_TOP_ORIGIN = 1, 2
+TILE_OVERLAY, TILE_TOP_ORIGIN, TILE_ROW_MAP = 1, 2, 4
 PNG_ZERO_SEGMENT = np.dtype([("n_raw", "<i4"), ("len", "<i4"), ("bytes", "u1", (56,))], align=True)
 assert PNG_ZERO_SEGMENT.itemsize == 64
 PNG_FILE = np.dtype(
@@ -209,11 +209,11 @@ SIGNATURES = {
     "csg_pool_reduce_max": (_i, [_vp, _vp, _i, _i, _vp]),
     "csg_png_fixed_tables": (_i, [_vp]),
     "csg_png_set_tables": (_i, [_vp, _vp]),
-    "csg_png_count": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _i, _i, _vp, _vp, _i]),
+    "csg_png_count": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _i, _i, _vp, _vp, _i, _vp]),
     "csg_png_max_segment_tiles": (C.c_int32, []),
     "csg_png_slot_bytes": (C.c_int32, []),
     "csg_png_segments": (C.c_int32, [C.c_int32, C.c_int32]),
-    "csg_png_encode": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i]),
+    "csg_png_encode": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp]),
     "csg_png_compact": (_i, [_vp, _vp, _vp, _vp, _i, _vp]),
     "csg_png_write_files": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _i]),
     "csg_peer_create": (_i, [_vp, _i, _i, _sz, _vp, _vp]),

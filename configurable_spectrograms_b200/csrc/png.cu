@@ -4,7 +4,8 @@
 // fig.savefig, CS/generic_batch.py:108-113); there nearly all wall time goes into Agg and zlib.
 // Here the colour-mapped panels (K3) already sit in HBM, so a figure never exists as raw pixels
 // anywhere: one kernel evaluates the mosaic for the scanline it encodes -- every tile is a source
-// raster (a K3 panel in d_rgba, flipped to origin="lower"; or a host-drawn annotation sprite in the
+// raster (a K3 panel in d_rgba, flipped to origin="lower" -- or, on a log energy axis, placed row by row
+// through the host's row map; or a host-drawn annotation sprite in the
 // overlay atlas) resampled nearest-neighbour into its rectangle on the canvas, the way
 // imshow(aspect="auto") fills an axes box at display resolution (CS/plotting.py:280-287,606-611:
 // 4800 x 2400 pixels for the FAST grids); cusp lines burnt in; background in the gaps -- the
@@ -51,6 +52,7 @@ constexpr int kMergedWords = kPieces * kTokWords + kHeaderWords + 4;
 // figures of 4800x2400: 115.6 / 96.8 / 85.5 ms with 4 / 2 / 1 warps per block (achieved occupancy was 13.7 % of a
 // theoretical 25 % with 4).
 constexpr int kWarpsPerBlock = CSG_K4_WARPS;
+constexpr int kTileRowMap = 4;       // csg_png_tile.flags: rows come from d_row_maps (TILE_ROW_MAP in csgpu.h)
 
 // The code tables of one batch of figures (csg_png_tables in csgpu.h): either RFC 1951's fixed codes
 // or a custom (dynamic-block) code built by the host from the batch's own symbol counts.  Codes are
@@ -111,7 +113,7 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32)
                       const csg_png_vline* __restrict__ vlines, const int32_t* __restrict__ rows, int n_segments,
                       unsigned char* __restrict__ slots, int slot_bytes, int32_t* __restrict__ sizes,
                       uint32_t* __restrict__ adler, unsigned* __restrict__ counts, int count_stride, int* __restrict__ error,
-                      const csg_png_zero_segment* __restrict__ zero_table, int n_zero) {
+                      const csg_png_zero_segment* __restrict__ zero_table, int n_zero, const int32_t* __restrict__ row_maps) {
   // counts != NULL: no output, only the symbol statistics of every count_stride-th segment
   // (literal / length symbols 0..285, then distance symbols 0..29) for the host's custom code
   extern __shared__ __align__(16) unsigned char s_dyn[];
@@ -169,8 +171,18 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32)
       if (hit) {
         const int at = n + __popc(m & ((1u << lane) - 1u));
         if (at < kSegTiles) {
-          const int r_top = nearest(r - t.y, __fdiv_rn((float)t.ne, (float)t.h), t.ne - 1);  // source row, counted from the top
-          const int src_row = (t.flags & 2) ? r_top : t.ne - 1 - r_top;  // rasters store the lowest energy first
+          int src_row;
+          if (t.flags & kTileRowMap) {  // a panel on a log energy axis: the host lists the storage row of every canvas row
+            int k = 0;
+            if (row_maps)
+              k = __ldg(row_maps + t.row_map + (r - t.y));
+            else if (error)
+              atomicExch(error, -(1 + lo));  // the host raises: the tile's map table is missing
+            src_row = min(max(k, 0), t.ne - 1);
+          } else {
+            const int r_top = nearest(r - t.y, __fdiv_rn((float)t.ne, (float)t.h), t.ne - 1);  // source row, counted from the top
+            src_row = (t.flags & 2) ? r_top : t.ne - 1 - r_top;  // rasters store the lowest energy first
+          }
           SegTile e;
           e.x0 = (unsigned short)max(t.x, x0), e.x1 = (unsigned short)min(t.x + t.w, x0 + npx);
           e.tx = (unsigned short)t.x, e.nt_minus_1 = t.nt - 1;
@@ -509,7 +521,8 @@ int csg_png_set_tables(csg_ctx* ctx, const csg_png_tables* tables) {
 static int png_launch(csg_ctx* ctx, const uint8_t* d_rgba, const uint8_t* d_overlay, const csg_png_canvas* d_canvases,
                       int n_canvases, const csg_png_tile* d_tiles, const csg_png_vline* d_vlines, const int32_t* d_rows,
                       int n_segments, uint8_t* d_slots, int32_t* d_sizes, uint32_t* d_adler, uint32_t* d_counts,
-                      int count_stride, int32_t* d_error, const csg_png_zero_segment* d_zero, int n_zero) {
+                      int count_stride, int32_t* d_error, const csg_png_zero_segment* d_zero, int n_zero,
+                      const int32_t* d_row_maps) {
   if (!ctx_tables_ready(ctx)) {
     const int st = csg_png_set_tables(ctx, nullptr);
     if (st != CSG_OK) return st;
@@ -523,7 +536,7 @@ static int png_launch(csg_ctx* ctx, const uint8_t* d_rgba, const uint8_t* d_over
   }
   png_encode_kernel<<<blocks, kWarpsPerBlock * 32, kEncodeSmem, ctx->stream>>>(
       (const uint32_t*)d_rgba, (const uint32_t*)d_overlay, d_canvases, n_canvases, d_tiles, d_vlines, d_rows, n_segments, d_slots,
-      csg_png_slot_bytes(), d_sizes, d_adler, d_counts, count_stride, d_error, d_zero, d_zero ? n_zero : 0);
+      csg_png_slot_bytes(), d_sizes, d_adler, d_counts, count_stride, d_error, d_zero, d_zero ? n_zero : 0, d_row_maps);
   CSG_LAUNCH_CHECK(ctx, "png_encode_kernel");
   return CSG_OK;
 }
@@ -531,23 +544,24 @@ static int png_launch(csg_ctx* ctx, const uint8_t* d_rgba, const uint8_t* d_over
 int csg_png_encode(csg_ctx* ctx, const uint8_t* d_rgba, const uint8_t* d_overlay, const csg_png_canvas* d_canvases,
                    int n_canvases, const csg_png_tile* d_tiles, const csg_png_vline* d_vlines, const int32_t* d_rows,
                    int n_segments, uint8_t* d_slots, int32_t* d_sizes, uint32_t* d_adler, int32_t* d_error,
-                   const csg_png_zero_segment* d_zero, int n_zero) {
+                   const csg_png_zero_segment* d_zero, int n_zero, const int32_t* d_row_maps) {
   if (!ctx) return CSG_ERR_ARG;
   if (n_canvases <= 0 || n_segments <= 0) return CSG_OK;
   if (!d_rgba || !d_canvases || !d_tiles || !d_rows || !d_slots || !d_sizes || !d_adler)
     return csg_fail(ctx, CSG_ERR_ARG, "NULL argument");
   return png_launch(ctx, d_rgba, d_overlay, d_canvases, n_canvases, d_tiles, d_vlines, d_rows, n_segments, d_slots, d_sizes,
-                    d_adler, nullptr, 1, d_error, d_zero, n_zero);
+                    d_adler, nullptr, 1, d_error, d_zero, n_zero, d_row_maps);
 }
 
 int csg_png_count(csg_ctx* ctx, const uint8_t* d_rgba, const uint8_t* d_overlay, const csg_png_canvas* d_canvases,
                   int n_canvases, const csg_png_tile* d_tiles, const csg_png_vline* d_vlines, const int32_t* d_rows,
-                  int n_segments, int stride, uint32_t* d_counts, const csg_png_zero_segment* d_zero, int n_zero) {
+                  int n_segments, int stride, uint32_t* d_counts, const csg_png_zero_segment* d_zero, int n_zero,
+                  const int32_t* d_row_maps) {
   if (!ctx) return CSG_ERR_ARG;
   if (n_canvases <= 0 || n_segments <= 0) return CSG_OK;
   if (!d_rgba || !d_canvases || !d_tiles || !d_rows || !d_counts || stride < 1) return csg_fail(ctx, CSG_ERR_ARG, "bad argument");
   return png_launch(ctx, d_rgba, d_overlay, d_canvases, n_canvases, d_tiles, d_vlines, d_rows, n_segments, nullptr, nullptr,
-                    nullptr, d_counts, stride, nullptr, d_zero, n_zero);
+                    nullptr, d_counts, stride, nullptr, d_zero, n_zero, d_row_maps);
 }
 
 int csg_png_compact(csg_ctx* ctx, const uint8_t* d_slots, const int32_t* d_sizes, const int64_t* d_offsets, int n_segments,

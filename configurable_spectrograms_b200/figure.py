@@ -29,7 +29,7 @@ from datetime import datetime, timedelta, timezone
 import numpy as np
 
 from . import png
-from ._lib import PNG_TILE, TILE_OVERLAY, TILE_TOP_ORIGIN
+from ._lib import PNG_TILE, TILE_OVERLAY, TILE_ROW_MAP, TILE_TOP_ORIGIN
 from .overlay import ATLAS
 
 _COLORS = {
@@ -63,14 +63,37 @@ def nearest_index(n_dst: int, n_src: int) -> np.ndarray:
 
 _change_rows_cache: dict = {}
 _content_rows_cache: dict = {}
+_row_map_cache: dict = {}
 
 
-def _change_rows(ne: int, h: int) -> np.ndarray:
-    """Destination rows (0-based, inside a tile ``h`` pixels high) at which the source row changes."""
-    key = (ne, h)
+def log_row_map(ne: int, h: int, y_lo: float, y_hi: float) -> tuple:
+    """``(key, map)``: the storage row (0 = the extent's ``y_lo`` end) that every canvas row of a panel ``h``
+    pixels high shows when its ``ne`` evenly spaced rows are drawn on a log axis from ``y_lo`` (bottom) to
+    ``y_hi`` (top), the way Agg resamples ``imshow`` through ``set_yscale("log")``.  Canvas row ``d`` (0 = top)
+    is sampled at its centre, ``f = (h - d - 0.5) / h`` of the way up, in float64.  Cached: the panels of a
+    grid share one map, and ``key`` names it in the content-row caches."""
+    key = (int(ne), int(h), float(y_lo), float(y_hi))
+    hit = _row_map_cache.get(key)
+    if hit is None:
+        f = (h - np.arange(h, dtype=np.float64) - 0.5) / h
+        l0, l1 = math.log10(y_lo), math.log10(y_hi)
+        value = 10.0 ** (l0 + f * (l1 - l0))
+        k = np.floor((value - y_lo) / (y_hi - y_lo) * ne)
+        rows = np.clip(k, 0, ne - 1).astype(np.int32)
+        rows.flags.writeable = False
+        if len(_row_map_cache) > 4096:
+            _row_map_cache.clear()
+        hit = _row_map_cache[key] = (key, rows)
+    return hit
+
+
+def _change_rows(ne: int, h: int, row_map: tuple | None = None) -> np.ndarray:
+    """Destination rows (0-based, inside a tile ``h`` pixels high) at which the source row changes: nearest
+    neighbour, or the rows of ``row_map`` (a :func:`log_row_map`)."""
+    key = (ne, h) if row_map is None else (ne, h, row_map[0])
     hit = _change_rows_cache.get(key)
     if hit is None:
-        idx = nearest_index(h, ne)
+        idx = nearest_index(h, ne) if row_map is None else row_map[1]
         hit = _change_rows_cache[key] = np.concatenate([[0], np.flatnonzero(np.diff(idx)) + 1]).astype(np.int32)
         if len(_change_rows_cache) > 4096:
             _change_rows_cache.clear()
@@ -145,6 +168,7 @@ class PanelAxes:
         self.yscale = "linear"
         self.tick_labelsize = None
         self.tick_length = None
+        self.minor_tick_length = None
         self.colorbar: Colorbar | None = None
         self.row_label_pad = 0
 
@@ -192,6 +216,8 @@ class PanelAxes:
         if kw.get("which", "major") == "major":
             self.tick_labelsize = kw.get("labelsize", self.tick_labelsize)
             self.tick_length = kw.get("length", self.tick_length)
+        elif kw["which"] == "minor":
+            self.minor_tick_length = kw.get("length", self.minor_tick_length)
 
     def axvline(self, x, **kw):
         line = {"kind": "vline", "x": float(x), **kw}
@@ -252,6 +278,18 @@ def linear_ticks(lo: float, hi: float, max_ticks: int = 6):
     return [first + k * step for k in range(int((hi - first) / step + 1e-9) + 1)]
 
 
+def log_minor_ticks(lo: float, hi: float) -> list[float]:
+    """Unlabelled minor ticks of a log axis, ``LogLocator(subs="auto")``: ``m * 10**k`` (m = 2..9) inside
+    ``[lo, hi]``, none when the axis covers more than 10 decades (matplotlib's ``numdec > 10``)."""
+    lo, hi = min(lo, hi), max(lo, hi)
+    if not (lo > 0 and math.isfinite(hi)) or lo == hi:
+        return []
+    if math.floor(math.log10(hi)) - math.ceil(math.log10(lo)) > 10:
+        return []
+    decades = range(math.floor(math.log10(lo)), math.floor(math.log10(hi)) + 1)
+    return [m * 10.0**k for k in decades for m in range(2, 10) if lo <= m * 10.0**k <= hi]
+
+
 def _format_number(v: float) -> str:
     if v == 0:
         return "0"
@@ -268,12 +306,14 @@ _OVERLAY_FLAGS = TILE_OVERLAY | TILE_TOP_ORIGIN
 class FigureTiles:
     """The tile list of one figure: what both composers consume."""
 
-    __slots__ = ("W", "H", "records", "sources", "background")
+    __slots__ = ("W", "H", "records", "sources", "background", "row_maps")
 
     def __init__(self, W, H, background):
         self.W, self.H, self.background = int(W), int(H), background
         self.records: list[tuple] = []  # PNG_TILE fields, in drawing priority (the first tile covering a pixel wins)
         self.sources: dict = {}         # record index -> DeviceRaster | ndarray, for the panel rasters
+        self.row_maps: list[tuple] = []  # the distinct log_row_map()s of the panels; a TILE_ROW_MAP record's
+        # last field is its index here until table() turns it into an offset
 
     def sprite(self, ref, x, y, w=None, h=None):
         off, sh, sw = ref
@@ -291,14 +331,29 @@ class FigureTiles:
         if x1 > x0 and y1 > y0:
             self.records.append((ATLAS.solid(color)[0], 1, 1, x0, y0, x1 - x0, y1 - y0, 0, 0, _OVERLAY_FLAGS, 0))
 
-    def raster(self, source, ne, nt, x, y, w, h):
+    def raster(self, source, ne, nt, x, y, w, h, row_map=None):
+        """A panel; ``row_map`` (a :func:`log_row_map` of height ``h``) places its rows instead of the nearest
+        row and the origin="lower" flip."""
         if w <= 0 or h <= 0 or ne <= 0 or nt <= 0:
             return
         off = source.offset if isinstance(source, DeviceRaster) else 0
+        flags = slot = 0
+        if row_map is not None:
+            keys = [m[0] for m in self.row_maps]
+            if row_map[0] not in keys:
+                self.row_maps.append(row_map)
+                keys.append(row_map[0])
+            flags, slot = TILE_ROW_MAP, keys.index(row_map[0])
         self.sources[len(self.records)] = source
-        self.records.append((off, ne, nt, int(x), int(y), int(w), int(h), 0, 0, 0, 0))
+        self.records.append((off, ne, nt, int(x), int(y), int(w), int(h), 0, 0, flags, slot))
 
-    def table(self) -> np.ndarray:
+    def map_of(self, k: int) -> tuple:
+        """The row map of record ``k`` (a TILE_ROW_MAP tile)."""
+        return self.row_maps[self.records[k][10]]
+
+    def table(self, map_offsets=None) -> np.ndarray:
+        """The records as ``PNG_TILE`` rows.  A TILE_ROW_MAP tile's ``row_map`` is the offset of its map in the
+        concatenation of ``row_maps``, or ``map_offsets[i]`` for map ``i`` when the caller places them."""
         if not self.records:
             return np.zeros(0, dtype=PNG_TILE)
         # (a structured array straight from the tuples is built field by field per record: 3x slower)
@@ -308,14 +363,22 @@ class FigureTiles:
         out = np.empty(len(flat), dtype=PNG_TILE)
         out["rgba_off"] = flat[:, 0]
         out.view(np.int32).reshape(len(flat), PNG_TILE.itemsize // 4)[:, 2:] = flat[:, 1:]
+        if self.row_maps:
+            if map_offsets is None:
+                map_offsets = np.cumsum([0] + [len(m[1]) for m in self.row_maps[:-1]])
+            mapped = (out["flags"] & TILE_ROW_MAP) != 0
+            out["row_map"][mapped] = np.asarray(map_offsets, dtype=np.int64)[out["row_map"][mapped]]
         return out
 
     def content_rows(self, table: np.ndarray | None = None) -> np.ndarray:
         """Ascending scanlines whose content may differ from the line above: where a tile starts, ends or
         moves on to another source row (the device encodes these; the runs in between repeat)."""
         t = self.table() if table is None else table
-        # rows depend on the vertical geometry only, which the figures of one kind share
-        key = (self.H, t["y"].tobytes(), t["h"].tobytes(), t["ne"].tobytes()) if len(t) else (self.H,)
+        # rows depend on the vertical geometry only, which the figures of one kind share -- and on the row map
+        # of every panel on a log axis (a linear panel of the same geometry changes rows elsewhere)
+        mapped = np.flatnonzero(t["flags"] & TILE_ROW_MAP) if self.row_maps else np.zeros(0, np.int64)
+        maps = tuple((int(k), self.map_of(int(k))[0]) for k in mapped)
+        key = (self.H, t["y"].tobytes(), t["h"].tobytes(), t["ne"].tobytes(), maps) if len(t) else (self.H,)
         hit = _content_rows_cache.get(key)
         if hit is not None:
             return hit
@@ -325,13 +388,18 @@ class FigureTiles:
             y, h, ne = t["y"].astype(np.int64), t["h"].astype(np.int64), t["ne"].astype(np.int64)
             mark[np.minimum(y, self.H)] = True
             mark[np.minimum(y + h, self.H)] = True
+            for k in mapped:
+                rows = _change_rows(int(ne[k]), int(h[k]), self.map_of(int(k))) + int(y[k])
+                mark[rows[rows <= self.H]] = True
+            h = h.copy()
+            h[mapped] = -1  # handled above
             one_to_one = (ne == h) & (h > 1)
             if one_to_one.any():  # sprites at their own size: every row is new (+1 / -1 over their spans)
                 delta = np.zeros(self.H + 2, dtype=np.int32)
                 np.add.at(delta, np.minimum(y[one_to_one], self.H), 1)
                 np.add.at(delta, np.minimum(y[one_to_one] + h[one_to_one], self.H), -1)
                 mark[:-1] |= np.cumsum(delta[:-1]) > 0
-            for k in np.flatnonzero((ne != h) & (ne > 1)):  # resampled rasters and ramps: a few per figure
+            for k in np.flatnonzero((ne != h) & (ne > 1) & (h > 0)):  # resampled rasters and ramps: a few per figure
                 rows = _change_rows(int(ne[k]), int(h[k])) + int(y[k])
                 mark[rows[rows <= self.H]] = True
         rows = np.flatnonzero(mark[: self.H]).astype(np.int32)
@@ -373,6 +441,7 @@ def _static_block(ax: "PanelAxes", img: RasterImage, cw: int, ch: int, pt: float
     black = (0, 0, 0, 255)
     tick_px = max(6, int(round((ax.tick_labelsize or 10) * pt)))
     tick_len = max(2, int(round((ax.tick_length or 4) * pt)))
+    minor_len = max(1, int(round((ax.minor_tick_length or 2) * pt)))
     line_w = max(1, int(round(0.8 * pt)))
     solid = ATLAS.solid(black)[0]
     tiles: list[tuple] = []
@@ -390,7 +459,7 @@ def _static_block(ax: "PanelAxes", img: RasterImage, cw: int, ch: int, pt: float
 
     ylabel = ATLAS.text(ax.yaxis.label.text, label_px(ax.yaxis.label), rotate=True) if ax.yaxis.label.text else None
     xlabel = ATLAS.text(ax.xaxis.label.text, label_px(ax.xaxis.label)) if ax.xaxis.label.text else None
-    log_y = ax.yscale == "log" and y_lo > 0 and y_hi > 0
+    log_y = ax.yscale == "log" and y_lo > 0 and y_hi > 0 and y_lo != y_hi
     if ax.yticks is not None:
         yt = [float(v) for v in ax.yticks]
         yl = list(ax.yticklabels) if ax.yticklabels is not None else [_format_number(v) for v in yt]
@@ -436,6 +505,10 @@ def _static_block(ax: "PanelAxes", img: RasterImage, cw: int, ch: int, pt: float
         if by - 0.5 <= py <= by + bh + 0.5:
             rect(bx - line_w - tick_len, int(round(py - line_w / 2)), tick_len, line_w)
             sprite(ref, bx - line_w - tick_len - pad - ref[2], int(round(py - ref[1] / 2)))
+    if log_y:
+        for v in log_minor_ticks(y_lo, y_hi):
+            py = by + bh - (math.log10(v) - math.log10(y_lo)) / (math.log10(y_hi) - math.log10(y_lo)) * bh
+            rect(bx - line_w - minor_len, int(round(py - line_w / 2)), minor_len, line_w)
     if ylabel:
         sprite(ylabel, pad, int(by + bh / 2 - ylabel[1] / 2))
     if xlabel:
@@ -561,7 +634,7 @@ class SpectrogramFigure:
         # (width, height, word sprites): a title changes with every orbit, its words and its height do not
         title = ATLAS.text_parts(ax.title, max(6, int(round((ax.title_fontsize or 12) * pt)))) if ax.title else None
         title_h = title[1] if title else 0
-        key = (int(cw), int(ch), pt, pad, ax.tick_labelsize, ax.tick_length, ax.yaxis.label.text, ax.yaxis.label.fontsize,
+        key = (int(cw), int(ch), pt, pad, ax.tick_labelsize, ax.tick_length, ax.minor_tick_length, ax.yaxis.label.text, ax.yaxis.label.fontsize,
                ax.xaxis.label.text, ax.xaxis.label.fontsize, title_h,
                None if ax.yticks is None else tuple(ax.yticks), None if ax.yticklabels is None else tuple(ax.yticklabels),
                ax.yscale, y_lo, y_hi, cb is not None,
@@ -660,7 +733,12 @@ class SpectrogramFigure:
         ix1 = int(round(min(max(bx + (float(ex[1]) - x_lo) * scale, bx), bx + bw)))
         if ix1 - ix0 < 1:
             ix0, ix1 = bx, bx + bw
-        out.raster(img.rgba, ne, nt, ix0, by, ix1 - ix0, bh)
+        # a log energy axis: the rows are placed through the log transform (imshow + set_yscale("log")); with
+        # a non-positive or empty extent, or a single row, matplotlib has no warp to show and the rows stay linear
+        row_map = None
+        if ax.yscale == "log" and 0 < y_lo < math.inf and 0 < y_hi < math.inf and y_lo != y_hi and ne >= 2:
+            row_map = log_row_map(ne, bh, y_lo, y_hi)
+        out.raster(img.rgba, ne, nt, ix0, by, ix1 - ix0, bh, row_map)
 
     # --------------------------------------------------------------- composing
     def compose(self, dpi: float | None = None) -> np.ndarray:
@@ -671,14 +749,17 @@ class SpectrogramFigure:
         canvas[:] = t.background
         atlas = ATLAS.pixels()
         for k in range(len(t.records) - 1, -1, -1):  # the first tile of the list ends up on top
-            off, ne, nt, x, y, w, h, _vf, _vc, flags, _pad = t.records[k]
+            off, ne, nt, x, y, w, h, _vf, _vc, flags, _map = t.records[k]
             src = t.sources.get(k)
             if isinstance(src, DeviceRaster):
                 raise TypeError("this panel lives on the device: encode the figure with png.encode_figures_device")
             source = atlas[off : off + ne * nt].view(np.uint8).reshape(ne, nt, 4) if flags & TILE_OVERLAY else src
-            rows = nearest_index(h, ne)
-            if not flags & TILE_TOP_ORIGIN:
-                rows = ne - 1 - rows  # rasters store the lowest energy first (imshow origin="lower")
+            if flags & TILE_ROW_MAP:
+                rows = t.map_of(k)[1]  # storage rows, lowest energy = 0, like the device reads them
+            else:
+                rows = nearest_index(h, ne)
+                if not flags & TILE_TOP_ORIGIN:
+                    rows = ne - 1 - rows  # rasters store the lowest energy first (imshow origin="lower")
             canvas[y : y + h, x : x + w] = source[rows][:, nearest_index(w, nt)]
         return canvas
 

@@ -372,9 +372,11 @@ def zero_segment_table(widths) -> np.ndarray:
 
 
 def _device_tables(figures, dpi):
-    """Tile / canvas / row tables of a list of figures.  Returns ``(canvases, tiles, rows, per_figure)`` with
-    ``canvases`` a list of mutable rows of ``PNG_CANVAS`` (``seg_first`` is filled per group), ``tiles`` one
-    ``PNG_TILE`` array, ``rows`` one int32 array of content rows and ``per_figure`` = [(W, H, content rows)]."""
+    """Tile / canvas / row tables of a list of figures.  Returns ``(canvases, tiles, rows, row_maps, per_figure)``
+    with ``canvases`` a list of mutable rows of ``PNG_CANVAS`` (``seg_first`` is filled per group), ``tiles`` one
+    ``PNG_TILE`` array, ``rows`` one int32 array of content rows, ``row_maps`` the int32 row maps of the panels
+    on a log energy axis (each distinct map once; ``None`` when there are none) and ``per_figure`` =
+    [(W, H, content rows)]."""
     from ._lib import PNG_TILE
     from .figure import DeviceRaster
 
@@ -383,13 +385,19 @@ def _device_tables(figures, dpi):
         return r | (g << 8) | (b << 16) | (a << 24)
 
     canvases, tile_parts, row_parts, per_figure = [], [], [], []
-    n_tiles = n_rows = 0
+    map_at, map_parts = {}, []  # row-map key -> offset in the concatenated maps
+    n_tiles = n_rows = n_map = 0
     for fig in figures:
         t = fig.tiles(dpi)
         for src in t.sources.values():
             if not isinstance(src, DeviceRaster):
                 raise TypeError("encode_figures_device needs panels drawn from device rasters (figure.DeviceRaster)")
-        table = t.table()
+        for key, rows in t.row_maps:
+            if key not in map_at:
+                map_at[key] = n_map
+                map_parts.append(rows)
+                n_map += len(rows)
+        table = t.table([map_at[key] for key, _rows in t.row_maps])
         rows = t.content_rows(table)
         canvases.append([t.W, t.H, n_tiles, len(table), pack(t.background), 0, (t.W + 1023) // 1024, n_rows])
         tile_parts.append(table)
@@ -399,7 +407,8 @@ def _device_tables(figures, dpi):
         n_rows += len(rows)
     tiles = np.concatenate(tile_parts) if n_tiles else np.zeros(1, PNG_TILE)
     rows = np.concatenate(row_parts) if n_rows else np.zeros(1, np.int32)
-    return canvases, tiles, rows, per_figure
+    row_maps = np.concatenate(map_parts).astype(np.int32) if n_map else None
+    return canvases, tiles, rows, row_maps, per_figure
 
 
 def encode_figures_device(ctx, d_rgba_ptr: int, figures, dpi: float | None = None, max_segments: int = 400_000, consume=None,
@@ -451,7 +460,7 @@ def encode_figures_device(ctx, d_rgba_ptr: int, figures, dpi: float | None = Non
     lib = ctx.lib
     figures = list(figures)
     t0 = time.perf_counter()
-    canvases, tiles, rows, per_figure = _device_tables(figures, dpi)
+    canvases, tiles, rows, row_maps, per_figure = _device_tables(figures, dpi)
     slot = int(lib.csg_png_slot_bytes())
     scratch = ctx.__dict__.setdefault("_png_scratch", {})
     if scratch.get("deferred") is not None:
@@ -466,6 +475,8 @@ def encode_figures_device(ctx, d_rgba_ptr: int, figures, dpi: float | None = Non
         return buf
 
     d_tiles, d_rows = ctx.to_device(tiles), ctx.to_device(rows)
+    d_row_maps = ctx.to_device(row_maps) if row_maps is not None else None
+    maps_ptr = d_row_maps.ptr if d_row_maps is not None else None
     zero_table = zero_segment_table([c[0] for c in canvases]) if canvases else np.zeros(0, dtype=np.uint8)
     d_zero = ctx.to_device(zero_table) if len(zero_table) else None
     zero_args = (d_zero.ptr if d_zero is not None else None, len(zero_table))
@@ -503,7 +514,7 @@ def encode_figures_device(ctx, d_rgba_ptr: int, figures, dpi: float | None = Non
                 d_counts.zero()
                 ctx._check(lib.csg_png_set_tables(ctx.handle, None))  # the count pass needs valid symbol tables
                 ctx._check(lib.csg_png_count(ctx.handle, d_rgba_ptr, d_overlay, d_canvases.ptr, len(group), d_tiles.ptr, None,
-                                             d_rows.ptr, n_seg, 4, d_counts.ptr, *zero_args))
+                                             d_rows.ptr, n_seg, 4, d_counts.ptr, *zero_args, maps_ptr))
                 tables = np.ascontiguousarray(custom_tables(d_counts.download(np.uint32, 316)))
                 ctx._check(lib.csg_png_set_tables(ctx.handle, tables.ctypes.data))
                 if code_cache is not None:
@@ -511,7 +522,7 @@ def encode_figures_device(ctx, d_rgba_ptr: int, figures, dpi: float | None = Non
             t0 = tick("code_tables", t0)
         d_slots, d_sizes, d_adler = dev("slots", n_seg * slot), dev("sizes", n_seg * 4), dev("adler", n_seg * 8)
         ctx._check(lib.csg_png_encode(ctx.handle, d_rgba_ptr, d_overlay, d_canvases.ptr, len(group), d_tiles.ptr, None,
-                                      d_rows.ptr, n_seg, d_slots.ptr, d_sizes.ptr, d_adler.ptr, d_error.ptr, *zero_args))
+                                      d_rows.ptr, n_seg, d_slots.ptr, d_sizes.ptr, d_adler.ptr, d_error.ptr, *zero_args, maps_ptr))
         tick("encode_launch", t0)
         return (k, group, n_seg, d_canvases, d_slots, d_sizes, d_adler)
 
@@ -522,6 +533,8 @@ def encode_figures_device(ctx, d_rgba_ptr: int, figures, dpi: float | None = Non
         sizes = d_sizes.download(np.int32, n_seg, sync=False)
         bad = d_error.download(np.int32, 1, sync=False)
         adler = d_adler.download(np.uint32, 2 * n_seg).reshape(n_seg, 2)  # synchronises
+        if bad[0] < 0:
+            raise ValueError(f"figure {k - int(bad[0]) - 1}: a tile reads a row map, but no row-map table was given")
         if bad[0]:
             raise ValueError(f"figure {k + int(bad[0]) - 1}: more than {int(lib.csg_png_max_segment_tiles())} tiles meet in one "
                              "1024-pixel scanline segment")
@@ -596,7 +609,7 @@ def encode_figures_device(ctx, d_rgba_ptr: int, figures, dpi: float | None = Non
         settle_failed()
         raise
     if open_state is not None:
-        keep_alive = {"tables": (d_tiles, d_rows, d_zero)}  # device tables the open kernel reads
+        keep_alive = {"tables": (d_tiles, d_rows, d_zero, d_row_maps)}  # device tables the open kernel reads
 
         def complete_open():
             try:

@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define CSG_ABI_VERSION 25
+#define CSG_ABI_VERSION 26
 
 #if defined(__GNUC__)
 #define CSG_API __attribute__((visibility("default")))
@@ -473,8 +473,10 @@ typedef struct {
   int32_t w, h;      /* size on the canvas: source index = floor((d + 0.5) * n_src / n_dst), float32         */
   int32_t vline_first, vline_count; /* cusp lines burnt into this tile (d_vlines)                            */
   int32_t flags;     /* bit 0: source in the overlay atlas; bit 1: source row 0 is the TOP row (a K3 raster
-                        stores the lowest energy first and is flipped: imshow origin="lower")                */
-  int32_t pad;
+                        stores the lowest energy first and is flipped: imshow origin="lower"); bit 2
+                        (TILE_ROW_MAP): canvas row r shows storage row d_row_maps[row_map + (r - y)], clamped
+                        to [0, ne-1], instead of the nearest row and the flip (a panel on a log energy axis)  */
+  int32_t row_map;   /* with bit 2: offset of the tile's h-entry map in d_row_maps                           */
 } csg_png_tile; /* 48 bytes */
 typedef struct {
   int32_t col, half; /* canvas columns col-half .. col+half, relative to the tile's left edge              */
@@ -522,10 +524,12 @@ typedef struct {
 CSG_API int csg_png_fixed_tables(csg_png_tables* out);                        /* RFC 1951 fixed code    */
 CSG_API int csg_png_set_tables(csg_ctx* ctx, const csg_png_tables* tables);  /* NULL: the fixed code   */
 /* Symbol statistics of every stride-th segment: d_counts[286 + 30] (uint32, zeroed by the caller) +=
- * literal / length symbol counts, then distance symbol counts.  Nothing is encoded. */
+ * literal / length symbol counts, then distance symbol counts.  Nothing is encoded.  d_row_maps as for
+ * csg_png_encode (the counts must see the pixels the encode pass will encode). */
 CSG_API int csg_png_count(csg_ctx* ctx, const uint8_t* d_rgba, const uint8_t* d_overlay, const csg_png_canvas* d_canvases,
                   int n_canvases, const csg_png_tile* d_tiles, const csg_png_vline* d_vlines, const int32_t* d_rows,
-                  int n_segments, int stride, uint32_t* d_counts, const csg_png_zero_segment* d_zero, int n_zero);
+                  int n_segments, int stride, uint32_t* d_counts, const csg_png_zero_segment* d_zero, int n_zero,
+                  const int32_t* d_row_maps);
 CSG_API int32_t csg_png_slot_bytes(void);                    /* capacity of one segment's output slot        */
 CSG_API int32_t csg_png_segments(int32_t W, int32_t n_rows); /* segments of n_rows listed scanlines of width W */
 CSG_API int32_t csg_png_max_segment_tiles(void);             /* tiles one segment may intersect               */
@@ -533,11 +537,14 @@ CSG_API int32_t csg_png_max_segment_tiles(void);             /* tiles one segmen
  * d_slots[n_segments][slot_bytes]: the encoded segments; d_sizes[n_segments]: their byte counts;
  * d_adler[n_segments][2]: (sum of bytes, sum of (n - t) * byte_t) mod 65521 of the filtered bytes;
  * d_error (int32, may be NULL, zeroed by the caller): 1 + the canvas in which more than
- * csg_png_max_segment_tiles() tiles met in one segment (its output is wrong: the host raises). */
+ * csg_png_max_segment_tiles() tiles met in one segment, or -(1 + the canvas) in which a TILE_ROW_MAP tile
+ * met a NULL d_row_maps (either way its output is wrong: the host raises).
+ * d_row_maps (int32, may be NULL when no tile sets TILE_ROW_MAP): the row maps of the tiles that do. */
 CSG_API int csg_png_encode(csg_ctx* ctx, const uint8_t* d_rgba, const uint8_t* d_overlay, const csg_png_canvas* d_canvases,
                    int n_canvases, const csg_png_tile* d_tiles, const csg_png_vline* d_vlines, const int32_t* d_rows,
                    int n_segments, uint8_t* d_slots, int32_t* d_sizes, uint32_t* d_adler, int32_t* d_error,
-                   const csg_png_zero_segment* d_zero, int n_zero); /* d_zero may be NULL */
+                   const csg_png_zero_segment* d_zero, int n_zero, /* d_zero may be NULL */
+                   const int32_t* d_row_maps);
 /* d_packed + d_offsets[s] <- slot s (d_offsets: exclusive prefix sum of d_sizes, from the host). */
 CSG_API int csg_png_compact(csg_ctx* ctx, const uint8_t* d_slots, const int32_t* d_sizes, const int64_t* d_offsets,
                     int n_segments, uint8_t* d_packed);
