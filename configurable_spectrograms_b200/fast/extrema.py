@@ -19,7 +19,8 @@ import json
 import math
 import os
 from collections.abc import Iterable
-from typing import Any
+from dataclasses import dataclass
+from typing import Any, NamedTuple
 
 import numpy as np
 
@@ -47,13 +48,28 @@ def _extrema_overrides(global_extrema, inst, y_scale, z_scale):
     return tuple(out)
 
 
+def _last_done(state, y_scale, z_scale) -> int:
+    """The last orbit the cached walk of this (y, z) combo finished (-1: none or unreadable)."""
+    stored = state.get(f"{y_scale}_{z_scale}_last_orbit", -1)
+    return int(stored) if isinstance(stored, (int, float)) else -1
+
+
+def _merge(prev_e, prev_z, cand_e, cand_z):
+    """One step's running-max merge as the reference stores it: ``(y_max, z_max)``, an int capped at
+    4000 and a float (the JSON cache is compared and written as is, so the types are part of the result)."""
+    merged_e = max(float(prev_e), cand_e) if isinstance(prev_e, (int, float)) else cand_e
+    merged_z = max(float(prev_z), cand_z) if isinstance(prev_z, (int, float)) else cand_z
+    return int(min(4000, math.ceil(merged_e))), float(math.ceil(merged_z))
+
+
 def _walk(sequence, instrument_order, y_scale, z_scale, state, totals, log_floor_cutoff, log_floor_value,
-          on_scan, on_step_done=None):
+          on_scan, on_step_done=None, *, range_max=None):
     """The reference's orbit x instrument loop (``:183-331``) with the scan abstracted.
 
     ``sequence``: [(orbit, {inst: handle})] ascending.  ``on_scan(inst, orbit_index, handle)``
     is called where the reference loads a file and updates its pools, and must return
-    ``(candidate_energy_max, candidate_intensity_max, intensity_min_store)``.
+    ``(candidate_energy_max, candidate_intensity_max, intensity_min_store)``.  ``range_max(inst, first,
+    stop)``: the same for the largest candidates of steps first..stop (None: unknown), to fold a chain.
     """
 
     def safe_log(value):  # :151-161
@@ -69,10 +85,10 @@ def _walk(sequence, instrument_order, y_scale, z_scale, state, totals, log_floor
 
     orbit_numbers = [o for o, _ in sequence]
     last_key = f"{y_scale}_{z_scale}_last_orbit"
-    stored = state.get(last_key, -1)
-    last_done = int(stored) if isinstance(stored, (int, float)) else -1
+    last_done = _last_done(state, y_scale, z_scale)
     y_log, z_log = y_scale == "log", z_scale == "log"
-    if on_step_done is None and _walk_chains(sequence, instrument_order, y_scale, z_scale, state, totals, last_done, on_scan):
+    if on_step_done is None and _walk_chains(sequence, instrument_order, y_scale, z_scale, state, totals, last_done,
+                                             on_scan, range_max):
         return state
     # key strings of every instrument, built once (the loop below runs orbits x instruments times)
     keys = []
@@ -105,13 +121,11 @@ def _walk(sequence, instrument_order, y_scale, z_scale, state, totals, log_floor
                     on_step_done(reuse=True)
                 continue
             cand_e, cand_z, z_min_store = on_scan(inst, orbit_index, handles.get(inst))
-            prev_e, prev_z = state.get(k_ymax), state.get(k_zmax)
-            merged_e = max(float(prev_e), cand_e) if isinstance(prev_e, (int, float)) else cand_e
-            merged_z = max(float(prev_z), cand_z) if isinstance(prev_z, (int, float)) else cand_z
+            y_max, z_max = _merge(state.get(k_ymax), state.get(k_zmax), cand_e, cand_z)
             state[k_ymin] = 0
-            state[k_ymax] = int(min(4000, math.ceil(merged_e)))
+            state[k_ymax] = y_max
             state[k_zmin] = z_min_store
-            state[k_zmax] = float(math.ceil(merged_z))
+            state[k_zmax] = z_max
             state[progress_key] = {
                 "processed_index": orbit_index,
                 "total": totals[inst],
@@ -130,8 +144,7 @@ def chain_ranges(sequence, instrument_order, y_scale, z_scale, state, totals, la
     covers -- when the walk is nothing but independent max-merge chains (see
     :func:`_walk_chains`); ``None`` when some step re-uses, skips or completes differently."""
     if last_done is None:
-        stored = state.get(f"{y_scale}_{z_scale}_last_orbit", -1)
-        last_done = int(stored) if isinstance(stored, (int, float)) else -1
+        last_done = _last_done(state, y_scale, z_scale)
     if not sequence or not instrument_order or (y_scale == "linear" and z_scale == "linear"):
         return None
     for inst in instrument_order:
@@ -152,43 +165,34 @@ def chain_ranges(sequence, instrument_order, y_scale, z_scale, state, totals, la
     return first, {inst: min(last_index, max(first, totals[inst] - 1)) for inst in instrument_order}
 
 
-def _walk_chains(sequence, instrument_order, y_scale, z_scale, state, totals, last_done, on_scan) -> bool:
+def _walk_chains(sequence, instrument_order, y_scale, z_scale, state, totals, last_done, on_scan, range_max) -> bool:
     """The loop of :func:`_walk` when every (orbit, instrument) step is a plain scan step: nothing
     is re-used from the linear/linear keys, nothing is complete, nobody watches the intermediate
     states.  Then the instruments are independent max-merge chains and only their last writes
     survive, so each chain runs on local variables and ``state`` is written once -- the same
-    arithmetic in the same order per instrument, without ~25 dict operations per step.
-    Returns False (state untouched) when the preconditions do not hold."""
+    arithmetic in the same order per instrument, without ~25 dict operations per step, or with
+    ``range_max`` one merge per chain.  Returns False (state untouched) when the preconditions do not hold."""
     ranges = chain_ranges(sequence, instrument_order, y_scale, z_scale, state, totals, last_done)
     if ranges is None:
         return False
     first, stops = ranges
     results = {}
     last_executed = first
-    range_max = getattr(on_scan, "range_max", None)
     for inst in instrument_order:
         stem = f"{inst}_{y_scale}_{z_scale}"
         prev_e, prev_z = state.get(f"{stem}_y_max"), state.get(f"{stem}_z_max")
-        # the per-step loop below runs first..stop: it breaks after the step that makes the
-        # instrument "complete" (orbit_index + 1 >= total, :315-319), and always runs one step
         stop = stops[inst]
         folded = range_max(inst, first, stop) if range_max is not None else None
         if folded is not None:
             # ceil and min(4000, .) are monotone, so folding the max-merge over the steps equals
             # one merge with the largest candidate: min(4000, ceil(max(prev, c_first..c_stop)))
             cand_e, cand_z, z_min_store = folded
-            merged_e = max(float(prev_e), cand_e) if isinstance(prev_e, (int, float)) else cand_e
-            merged_z = max(float(prev_z), cand_z) if isinstance(prev_z, (int, float)) else cand_z
-            prev_e = int(min(4000, math.ceil(merged_e)))
-            prev_z = float(math.ceil(merged_z))
+            prev_e, prev_z = _merge(prev_e, prev_z, cand_e, cand_z)
         else:
             z_min_store = 0
             for orbit_index in range(first, stop + 1):
                 cand_e, cand_z, z_min_store = on_scan(inst, orbit_index, sequence[orbit_index][1].get(inst))
-                merged_e = max(float(prev_e), cand_e) if isinstance(prev_e, (int, float)) else cand_e
-                merged_z = max(float(prev_z), cand_z) if isinstance(prev_z, (int, float)) else cand_z
-                prev_e = int(min(4000, math.ceil(merged_e)))
-                prev_z = float(math.ceil(merged_z))
+                prev_e, prev_z = _merge(prev_e, prev_z, cand_e, cand_z)
         results[inst] = (stem, prev_e, prev_z, z_min_store, stop)
         last_executed = max(last_executed, stop)
     # the writes of the last step of every chain
@@ -267,8 +271,21 @@ def shared_energy_table(energy):
     return e0, keys, idx
 
 
+class _EnergyPlan(NamedTuple):
+    """One instrument's part of :func:`_energy_plan`."""
+
+    present: list  # scanned steps (orbit indices) whose file some rank holds
+    rows: np.ndarray  # their rows in the gathered per-file count table
+    energies: list  # their energy tables (equal tables folded into one object)
+    steps: np.ndarray  # every scanned step of the instrument
+    pos: np.ndarray  # position of every present step inside `steps`
+    ascending: bool  # `steps` strictly ascending
+    table: tuple | None  # shared_energy_table() when every present file shares one table
+
+
 def _energy_plan(shard, comm, instrument_order, steps, owners, first):
-    """Who holds the per-energy counts of every scanned step (static per plan; exchanged once)."""
+    """Who holds the per-energy counts of every scanned step (static per plan; exchanged once):
+    ``({inst: _EnergyPlan}, count rows per rank, max_E)``."""
     local = [(inst, oi + first, shard.file_meta[file]["energy"]) for inst, oi, file in owners]
     parts = comm.allgather_object(local) if comm.size > 1 else [local]
     n_max = max((len(p) for p in parts), default=0)
@@ -291,42 +308,88 @@ def _energy_plan(shard, comm, instrument_order, steps, owners, first):
                     break
             else:
                 uniq.append(e)
-        # static index maps of the per-step candidate fill (extrema_finish): position of every
-        # present step inside steps[inst]
+        # static index maps of the per-step candidate fill (extrema_finish)
         steps_arr = np.asarray(steps[inst], dtype=np.int64)
         pos = np.searchsorted(steps_arr, np.asarray(present, dtype=np.int64)) if present else np.zeros(0, np.int64)
         ascending = bool(np.all(np.diff(steps_arr) > 0)) if len(steps_arr) > 1 else True
         table = shared_energy_table(en[0]) if en and all(e is en[0] for e in en) else None
-        plan[inst] = (present, np.asarray([where[(inst, oi)] for oi in present], dtype=np.int64), en, steps_arr, pos, ascending, table)
+        rows = np.asarray([where[(inst, oi)] for oi in present], dtype=np.int64)
+        plan[inst] = _EnergyPlan(present, rows, en, steps_arr, pos, ascending, table)
     return plan, n_max, max_E
 
 
-def _device_y_tables(instrument_order, eplan, max_E):
-    """Static energy tables for ``csg_pool_energy_candidates`` -- or None when some instrument's
-    files do not share one table of distinct, NaN-free energies (the host path handles those)."""
+def _device_y_tables(instrument_order, eplan, max_E, ranges, owners, first):
+    """Static energy tables for ``csg_pool_energy_candidates`` over the chains of
+    :func:`chain_ranges` -- or None when there are no chains, or some instrument's files do not
+    share one table of distinct, NaN-free energies (the host path handles those)."""
+    if ranges is None:
+        return None
+    first_step, stops = ranges
     n_inst = len(instrument_order)
     order = np.zeros((n_inst, max_E), dtype=np.int32)
     keys = np.zeros((n_inst, max_E), dtype=np.float64)
     n_keys = np.zeros(n_inst, dtype=np.int32)
-    covered = {}
+    zero = {}
     for ii, inst in enumerate(instrument_order):
-        present, _rows, _en, steps_arr, pos, ascending, table = eplan[inst]
-        if not ascending:
+        ep = eplan[inst]
+        if not ep.ascending:
             return None
-        cov = np.zeros(int(steps_arr.max()) + 1 if len(steps_arr) else 0, dtype=bool)
-        if present:
-            if table is None:
+        cov = np.zeros(int(ep.steps.max()) + 1 if len(ep.steps) else 0, dtype=bool)
+        if ep.present:
+            if ep.table is None:
                 return None
-            e0, uniq, _idx = table
+            e0, uniq, _idx = ep.table
             if len(uniq) != len(e0) or len(e0) > max_E or np.isnan(e0).any():
                 return None
             o = np.argsort(e0, kind="stable")
             order[ii, : len(e0)], keys[ii, : len(e0)], n_keys[ii] = o, e0[o], len(e0)
-            idx = np.full(len(steps_arr), -1, dtype=np.int64)
-            idx[pos] = 1
-            cov[steps_arr] = np.maximum.accumulate(idx) >= 0
-        covered[inst] = cov
-    return {"order": order, "keys": keys, "n_keys": n_keys, "covered": covered}
+            idx = np.full(len(ep.steps), -1, dtype=np.int64)
+            idx[ep.pos] = 1
+            cov[ep.steps] = np.maximum.accumulate(idx) >= 0
+        # some step of the chain sees the 0.0 candidate (no file yet)
+        part = cov[first_step : stops[inst] + 1]
+        zero[inst] = not (len(part) == stops[inst] + 1 - first_step and bool(part.all()))
+    # positions of this rank that take part in each chain (global orbit index <= stop)
+    limit = np.array([sum(1 for i2, oi, _f in owners if i2 == inst and oi + first <= stops[inst]) for inst in instrument_order],
+                     dtype=np.int32)
+    return {"order": order, "keys": keys, "n_keys": n_keys, "limit": limit, "zero": zero}
+
+
+class _ExtremaPlan(NamedTuple):
+    """One entry of ``shard._extrema_plan_cache``: what depends only on the orbit sequence and the cache state."""
+
+    sequence: list  # held so that its id(), part of the cache key, cannot be recycled while the entry lives
+    totals: dict
+    items: np.ndarray  # this rank's POOL_ITEM rows
+    inst_len: np.ndarray
+    eplan: dict  # {inst: _EnergyPlan}
+    n_max: int  # count rows per rank in the gathered per-file count table
+    max_E: int
+    ytab: dict | None  # _device_y_tables()
+
+
+@dataclass
+class PendingExtrema:
+    """The selection :func:`extrema_enqueue` left running, and what :func:`extrema_finish` needs to redeem it."""
+
+    shard: Any
+    selector: Any  # pool_select.DevicePoolSelector
+    comm: Any
+    sequence: list
+    instrument_order: tuple
+    y_scale: str
+    z_scale: str
+    state: dict
+    totals: dict
+    compute_mins: bool
+    log_floor_cutoff: float
+    log_floor_value: float
+    requests: list
+    items: np.ndarray  # items, inst_len, max_E: the host-driven fallback's input
+    inst_len: np.ndarray
+    max_E: int
+    eplan: dict
+    ydev: dict | None  # the y candidates were max-merged on the device with these tables
 
 
 def extrema_enqueue(shard, sequence, instrument_order, y_scale, z_scale, state, *, compute_mins=False,
@@ -373,26 +436,11 @@ def extrema_enqueue(shard, sequence, instrument_order, y_scale, z_scale, state, 
         eplan, n_max, max_E = _energy_plan(shard, comm, instrument_order, steps, owners, first)
         max_E = (max_E + 3) & ~3  # count rows pack to 16 bytes (exchange payloads)
         ranges = chain_ranges(sequence, instrument_order, y_scale, z_scale, state, totals)
-        ytab = _device_y_tables(instrument_order, eplan, max_E) if ranges is not None else None
-        if ytab is not None:
-            first_step, stops = ranges
-            # positions of this rank that take part in each chain (global orbit index <= stop)
-            ytab["limit"] = np.array(
-                [sum(1 for i2, oi, _f in owners if i2 == inst and oi + first <= stops[inst]) for inst in instrument_order],
-                dtype=np.int32)
-            ytab["zero"] = {}
-            for inst in instrument_order:
-                cov = ytab["covered"][inst]
-                seg = np.zeros(stops[inst] + 1 - first_step, dtype=bool)
-                part = cov[first_step : stops[inst] + 1]
-                seg[: len(part)] = part
-                ytab["zero"][inst] = not bool(seg.all())  # some step of the chain sees the 0.0 candidate
+        ytab = _device_y_tables(instrument_order, eplan, max_E, ranges, owners, first)
         if len(cache) > 8:
             cache.clear()
-        # the entry holds `sequence` itself, so its id() cannot be recycled while the entry lives
-        hit = cache[key] = (sequence, steps, totals, items, inst_len, owners, eplan, n_max, max_E, ytab)
-    _, steps, totals, items, inst_len, owners, eplan, n_max, max_E, ytab = hit
-    ydev = ytab if not per_step else None
+        hit = cache[key] = _ExtremaPlan(sequence, totals, items, inst_len, eplan, n_max, max_E, ytab)
+    ydev = hit.ytab if not per_step else None
     requests = [{"inst": ii, "p": max_percentile, "mode": "running_max"} for ii in range(len(instrument_order))]
     if compute_mins:
         requests += [{"inst": ii, "p": 1, "mode": "last"} for ii in range(len(instrument_order))]
@@ -403,135 +451,99 @@ def extrema_enqueue(shard, sequence, instrument_order, y_scale, z_scale, state, 
         setattr(shard, attr, selector)
     if overlap:
         selector.ctx.wait_for(shard.batch.ctx)  # the collapsed sums (K1) are complete before the histograms read them
-    selector.enqueue(shard.batch.dtype, items, len(instrument_order), inst_len, max_E, requests, comm=comm,
-                     count_rows=n_max, ydev=ydev)
-    return {
-        "shard": shard, "sequence": sequence, "instrument_order": instrument_order, "y_scale": y_scale, "z_scale": z_scale,
-        "state": state, "compute_mins": compute_mins, "log_floor_cutoff": log_floor_cutoff,
-        "log_floor_value": log_floor_value, "comm": comm, "steps": steps, "totals": totals, "first": first,
-        "items": items, "inst_len": inst_len, "owners": owners, "requests": requests, "max_E": max_E, "selector": selector,
-        "eplan": eplan, "n_max": n_max, "ydev": ydev,
-    }
+    selector.enqueue(shard.batch.dtype, hit.items, len(instrument_order), hit.inst_len, hit.max_E, requests, comm=comm,
+                     count_rows=hit.n_max, ydev=ydev)
+    return PendingExtrema(
+        shard=shard, selector=selector, comm=comm, sequence=sequence, instrument_order=instrument_order,
+        y_scale=y_scale, z_scale=z_scale, state=state, totals=hit.totals, compute_mins=compute_mins,
+        log_floor_cutoff=log_floor_cutoff, log_floor_value=log_floor_value, requests=requests, items=hit.items,
+        inst_len=hit.inst_len, max_E=hit.max_E, eplan=hit.eplan, ydev=ydev,
+    )
 
 
-def extrema_finish(pending, on_step_done=None):
-    """Wait for the selection's read-backs and run the reference's bookkeeping walk on the results."""
-    from ..pool_select import GpuPoolBackend, prefix_percentiles
+def extrema_finish(pending: PendingExtrema, on_step_done=None):
+    """Wait for the selection's read-backs and run the reference's bookkeeping walk on the results.
 
-    shard, comm = pending["shard"], pending["comm"]
-    instrument_order, steps = pending["instrument_order"], pending["steps"]
-    requests, compute_mins = pending["requests"], pending["compute_mins"]
-    selector = pending["selector"]
-    if pending.get("ydev") is not None:
-        return _finish_device_y(pending, on_step_done)
-    # ---- y extrema: per-step energy candidates from every rank's per-file positive counts
-    # (available after the first histogram pass; this overlaps the digit loop on the GPU)
-    all_counts, npos = selector.result_counts()  # multi-rank: every rank's rows (device all-gather)
-    n_seq = len(pending["sequence"])
-    cand_e: dict[str, np.ndarray] = {}  # per orbit index: the candidate the reference's step would see
-    for inst in instrument_order:
-        present, rows, energies, steps_arr, pos, ascending, table = pending["eplan"][inst]
-        dense = np.zeros(n_seq, dtype=np.float64)
-        if present and ascending:
-            ce = energy_candidates(energies, all_counts[rows], as_array=True, shared_table=table)
-            # steps without a file repeat the previous candidate (0.0 before the first file)
-            idx = np.full(len(steps_arr), -1, dtype=np.int64)
-            idx[pos] = np.arange(len(present))
-            filled = np.maximum.accumulate(idx)
-            dense[steps_arr] = np.where(filled >= 0, ce[np.maximum(filled, 0)], 0.0)
-        elif present:
-            by_step = dict(zip(present, energy_candidates(energies, all_counts[rows])))
-            running = 0.0
-            for oi in steps[inst]:
-                running = by_step.get(oi, running)
-                dense[oi] = running
-        cand_e[inst] = dense
-    # ---- z extrema: the device selection
-    values = selector.result_values()
-    if values is None:
-        # more distinct candidate buckets survived than the device table holds: same kernels,
-        # digit loop driven from the host (arbitrary candidate counts)
-        backend = getattr(shard, "_pool_backend", None)
-        if backend is None:
-            backend = shard._pool_backend = GpuPoolBackend(shard.batch)
-        values, _, _ = prefix_percentiles(
-            backend, shard.batch.dtype, pending["items"], len(instrument_order), pending["inst_len"], pending["max_E"],
-            requests, comm=comm,
-        )
-    n_inst = len(instrument_order)
-    per_inst = {}
-    for ii, inst in enumerate(instrument_order):
-        z = values[ii]
-        z_min = 0
-        if compute_mins:
-            zm = values[n_inst + ii]
-            z_min = float(zm) if zm is not None else 0
-        per_inst[inst] = (cand_e[inst], float(z) if z is not None else 0.0, z_min)
-
-    def scan(inst, orbit_index, handle):
-        ce, z, z_min = per_inst[inst]
-        return float(ce[orbit_index]), z, z_min
-
-    def range_max(inst, first, stop):
-        """Largest candidates over the steps first..stop (None: NaN candidates, walk step by step)."""
-        ce, z, z_min = per_inst[inst]
-        top = float(ce[first : stop + 1].max())
-        if top != top or z != z:
-            return None
-        return top, z, z_min
-
-    scan.range_max = range_max
-    return _walk(pending["sequence"], instrument_order, pending["y_scale"], pending["z_scale"], pending["state"],
-                 pending["totals"], pending["log_floor_cutoff"], pending["log_floor_value"], scan, on_step_done)
-
-
-def _finish_device_y(pending, on_step_done):
-    """:func:`extrema_finish` when both extrema were max-merged on the device: one read-back of
-    ``n_requests + n_instruments`` numbers, then one merge per instrument."""
-    if on_step_done is not None:
+    The y candidates are per step, from every rank's per-file counts -- or, when
+    :func:`extrema_enqueue` max-merged them on the device, one per instrument."""
+    device_y = pending.ydev is not None
+    if device_y and on_step_done is not None:
         raise ValueError("extrema_enqueue(per_step=False) cannot report the state after every step")
+    order = pending.instrument_order
+    if not device_y:
+        # the per-file counts are read back after the first histogram pass: the per-step candidates
+        # are built while the digit loop runs on the GPU, before anything waits for the values
+        all_counts, _npos = pending.selector.result_counts()  # multi-rank: every rank's rows (device all-gather)
+        cand_e = {}  # {inst: [orbit index] -> the candidate the reference's step sees}
+        for inst in order:
+            ep = pending.eplan[inst]
+            dense = np.zeros(len(pending.sequence), dtype=np.float64)
+            if ep.present and ep.ascending:
+                ce = energy_candidates(ep.energies, all_counts[ep.rows], as_array=True, shared_table=ep.table)
+                # steps without a file repeat the previous candidate (0.0 before the first file)
+                idx = np.full(len(ep.steps), -1, dtype=np.int64)
+                idx[ep.pos] = np.arange(len(ep.present))
+                filled = np.maximum.accumulate(idx)
+                dense[ep.steps] = np.where(filled >= 0, ce[np.maximum(filled, 0)], 0.0)
+            elif ep.present:
+                by_step = dict(zip(ep.present, energy_candidates(ep.energies, all_counts[ep.rows])))
+                running = 0.0
+                for oi in ep.steps.tolist():
+                    running = by_step.get(oi, running)
+                    dense[oi] = running
+            cand_e[inst] = dense
+    values = _selected_values(pending)
+    n_inst = len(order)
+    z, z_min = {}, {}
+    for ii, inst in enumerate(order):
+        z[inst] = float(values[ii]) if values[ii] is not None else 0.0
+        zm = values[n_inst + ii] if pending.compute_mins else None
+        z_min[inst] = float(zm) if zm is not None else 0
+    if device_y:
+        top = {}
+        for inst, y in zip(order, pending.selector.result_y_candidates()):
+            if y is None:
+                y = 0.0  # no file took part: every step of the chain saw the empty-pool candidate
+            elif pending.ydev["zero"][inst]:
+                y = max(y, 0.0)
+            top[inst] = y
+
+        def scan(inst, orbit_index, handle):
+            raise AssertionError("per-step scan requested from a device-merged selection")
+
+        def range_max(inst, first, stop):
+            return top[inst], z[inst], z_min[inst]
+    else:
+
+        def scan(inst, orbit_index, handle):
+            return float(cand_e[inst][orbit_index]), z[inst], z_min[inst]
+
+        def range_max(inst, first, stop):
+            """Largest candidates over the steps first..stop (None: NaN candidates, walk step by step)."""
+            y = float(cand_e[inst][first : stop + 1].max())
+            if y != y or z[inst] != z[inst]:
+                return None
+            return y, z[inst], z_min[inst]
+
+    return _walk(pending.sequence, order, pending.y_scale, pending.z_scale, pending.state, pending.totals,
+                 pending.log_floor_cutoff, pending.log_floor_value, scan, on_step_done, range_max=range_max)
+
+
+def _selected_values(pending: PendingExtrema) -> list:
+    """One value per request (None: empty pool): the device selection's, or -- when more candidate
+    buckets survived than its slot table holds -- the same kernels with the digit loop driven from
+    the host, on a backend kept as ``shard._pool_backend``."""
     from ..pool_select import GpuPoolBackend, prefix_percentiles
 
-    shard, comm = pending["shard"], pending["comm"]
-    instrument_order, requests = pending["instrument_order"], pending["requests"]
-    selector, ydev = pending["selector"], pending["ydev"]
-    values = selector.result_values()
-    ycands = selector.result_y_candidates()
-    if values is None:  # slot-table overflow: same kernels, digit loop driven from the host
+    values = pending.selector.result_values()
+    if values is None:
+        shard = pending.shard
         backend = getattr(shard, "_pool_backend", None)
         if backend is None:
             backend = shard._pool_backend = GpuPoolBackend(shard.batch)
-        values, _, _ = prefix_percentiles(
-            backend, shard.batch.dtype, pending["items"], len(instrument_order), pending["inst_len"], pending["max_E"],
-            requests, comm=comm,
-        )
-    n_inst = len(instrument_order)
-    per_inst = {}
-    for ii, inst in enumerate(instrument_order):
-        z = values[ii]
-        z_min = 0
-        if pending["compute_mins"]:
-            zm = values[n_inst + ii]
-            z_min = float(zm) if zm is not None else 0
-        top = ycands[ii]
-        if top is None:
-            top = 0.0  # no file took part: every step of the chain saw the empty-pool candidate
-        elif ydev["zero"][inst]:
-            top = max(top, 0.0)
-        per_inst[inst] = (top, float(z) if z is not None else 0.0, z_min)
-
-    def scan(inst, orbit_index, handle):
-        raise AssertionError("per-step scan requested from a device-merged selection")
-
-    scan.range_max = lambda inst, first, stop: per_inst[inst]
-    state = pending["state"]
-    totals = pending["totals"]
-    stored = state.get(f"{pending['y_scale']}_{pending['z_scale']}_last_orbit", -1)
-    last_done = int(stored) if isinstance(stored, (int, float)) else -1
-    if not _walk_chains(pending["sequence"], instrument_order, pending["y_scale"], pending["z_scale"], state, totals,
-                        last_done, scan):
-        raise AssertionError("chain preconditions changed between enqueue and finish")
-    return state
+        values, _, _ = prefix_percentiles(backend, shard.batch.dtype, pending.items, len(pending.instrument_order),
+                                          pending.inst_len, pending.max_E, pending.requests, comm=pending.comm)
+    return values
 
 
 def extrema_from_shard(shard, sequence, instrument_order, y_scale, z_scale, state, *, compute_mins=False,

@@ -24,6 +24,8 @@ form the gloo tests exercise with a numpy kernel stand-in).
 
 from __future__ import annotations
 
+from collections import namedtuple
+
 import numpy as np
 
 from . import _lib
@@ -109,6 +111,15 @@ class _Grow:
             buf = self.pin[name] = self.ctx.pinned(max(int(nbytes * 1.25), 256))
         return buf
 
+    def put(self, name: str, arr: np.ndarray) -> _lib.DevBuf:
+        """Upload a small array through pinned staging into the device buffer ``name`` (on the stream)."""
+        arr = np.ascontiguousarray(arr)
+        pin = self.pinned(name, arr.nbytes)
+        pin.array[: arr.nbytes] = arr.view(np.uint8).reshape(-1)
+        dev = self.device(name, arr.nbytes)
+        self.ctx._check(self.ctx.lib.csg_h2d(self.ctx.handle, dev.ptr, pin.ptr, arr.nbytes))
+        return dev
+
 
 class GpuPoolBackend:
     """The four pool kernels over a :class:`engine.Batch`'s sums buffer (persistent scratch)."""
@@ -119,15 +130,6 @@ class GpuPoolBackend:
         self.mem = _Grow(batch.ctx)
         self._items_key = None
         self.n_items = 0
-
-    # -- small transfers through pinned staging
-    def _put(self, name: str, arr: np.ndarray) -> _lib.DevBuf:
-        arr = np.ascontiguousarray(arr)
-        pin = self.mem.pinned(name, arr.nbytes)
-        pin.array[: arr.nbytes] = arr.view(np.uint8).reshape(-1)
-        dev = self.mem.device(name, arr.nbytes)
-        self.ctx._check(self.ctx.lib.csg_h2d(self.ctx.handle, dev.ptr, pin.ptr, arr.nbytes))
-        return dev
 
     def _get(self, name: str, dev: _lib.DevBuf, dtype, count: int, sync=True) -> np.ndarray:
         nbytes = np.dtype(dtype).itemsize * count
@@ -143,8 +145,8 @@ class GpuPoolBackend:
         self.n_items = len(items)
         self.n_inst, self.max_pos, self.max_E = n_inst, max(max_pos, 1), max(max_E, 1)
         if key != self._items_key:
-            self.d_items = self._put("items", items) if len(items) else None
-            self.d_inst_len = self._put("inst_len", np.ascontiguousarray(inst_len, dtype=np.int32))
+            self.d_items = self.mem.put("items", items) if len(items) else None
+            self.d_inst_len = self.mem.put("inst_len", np.ascontiguousarray(inst_len, dtype=np.int32))
             self._items_key = key
 
     def hist_first(self, bits: int):
@@ -173,7 +175,7 @@ class GpuPoolBackend:
         nbytes = self.n_inst * self.max_pos * n_slots * nb * 4
         self.d_hist = self.mem.device("hist1", nbytes)
         self.ctx._check(self.ctx.lib.csg_memset(self.ctx.handle, self.d_hist.ptr, 0, nbytes))
-        d_pref = self._put("pref", np.ascontiguousarray(slot_prefix, dtype=np.uint64))
+        d_pref = self.mem.put("pref", np.ascontiguousarray(slot_prefix, dtype=np.uint64))
         if self.n_items:
             self.ctx._check(
                 self.ctx.lib.csg_pool_hist_refine(
@@ -200,8 +202,8 @@ class GpuPoolBackend:
     def locate(self, queries: np.ndarray, base: np.ndarray | None) -> np.ndarray:
         if len(queries) == 0:
             return queries
-        d_q = self._put("queries", queries)
-        d_base = self._put("base", np.ascontiguousarray(base, dtype=np.uint32)) if base is not None else None
+        d_q = self.mem.put("queries", queries)
+        d_base = self.mem.put("base", np.ascontiguousarray(base, dtype=np.uint32)) if base is not None else None
         self.ctx._check(
             self.ctx.lib.csg_pool_locate(
                 self.ctx.handle, self.d_hist.ptr, self.max_pos, self.n_slots, self.bits,
@@ -232,14 +234,6 @@ class DevicePoolSelector:
         self.mem = _Grow(self.ctx)
         self._static_key = None
         self._pending = None
-
-    def _put(self, name: str, arr: np.ndarray) -> _lib.DevBuf:
-        arr = np.ascontiguousarray(arr)
-        pin = self.mem.pinned(name, arr.nbytes)
-        pin.array[: arr.nbytes] = arr.view(np.uint8).reshape(-1)
-        dev = self.mem.device(name, arr.nbytes)
-        self.ctx._check(self.ctx.lib.csg_h2d(self.ctx.handle, dev.ptr, pin.ptr, arr.nbytes))
-        return dev
 
     def enqueue(self, dtype, items: np.ndarray, n_inst: int, inst_len: np.ndarray, max_E: int, requests: list[dict],
                 comm=None, count_rows: int | None = None, exchange=None, ydev: dict | None = None, dry: bool = False):
@@ -286,7 +280,7 @@ class DevicePoolSelector:
     def _payload_bytes(self, D, n_inst, max_E, n_items, count_rows, n_req, R, device_y):
         S = self.N_SLOTS
         bits0 = digit_plan(D)[0][1]
-        rows = max(n_items, 1) if (R == 1 or count_rows is None) else max(int(count_rows), n_items, 1)
+        rows = _count_rows(n_items, R, count_rows)
         sizes = [
             _al(n_inst * ((1 << bits0) + max(int(max_E), 1)) * 4, 16),
             n_inst * S * 1024 * 4,
@@ -328,20 +322,20 @@ class DevicePoolSelector:
             reqs = np.zeros(max(n_req, 1), dtype=POOL_REQUEST)
             for r, rq in enumerate(requests):
                 reqs[r] = (rq["inst"], 0 if rq["mode"] == "running_max" else 1, float(rq["p"]))
-            self.d_items = self._put("items", items) if n_items else None
-            self.d_inst_len = self._put("inst_len", np.ascontiguousarray(inst_len, dtype=np.int32))
-            self.d_reqs = self._put("reqs", reqs)
+            self.d_items = self.mem.put("items", items) if n_items else None
+            self.d_inst_len = self.mem.put("inst_len", np.ascontiguousarray(inst_len, dtype=np.int32))
+            self.d_reqs = self.mem.put("reqs", reqs)
             if device_y:
-                self.d_order = self._put("y_order", np.ascontiguousarray(ydev["order"], dtype=np.int32))
-                self.d_keys = self._put("y_keys", np.ascontiguousarray(ydev["keys"], dtype=np.float64))
-                self.d_nkeys = self._put("y_nkeys", np.ascontiguousarray(ydev["n_keys"], dtype=np.int32))
-                self.d_limit = self._put("y_limit", np.ascontiguousarray(ydev["limit"], dtype=np.int32))
+                self.d_order = self.mem.put("y_order", np.ascontiguousarray(ydev["order"], dtype=np.int32))
+                self.d_keys = self.mem.put("y_keys", np.ascontiguousarray(ydev["keys"], dtype=np.float64))
+                self.d_nkeys = self.mem.put("y_nkeys", np.ascontiguousarray(ydev["n_keys"], dtype=np.int32))
+                self.d_limit = self.mem.put("y_limit", np.ascontiguousarray(ydev["limit"], dtype=np.int32))
             self._static_key = key
         shift0, bits0 = plan[0]
         nb0 = 1 << bits0
         hist0 = mem.device("hist0", n_inst * max_pos * nb0 * 4)
         run(lib.csg_memset, h, hist0.ptr, 0, n_inst * max_pos * nb0 * 4)
-        rows = max(n_items, 1) if (R == 1 or count_rows is None) else max(int(count_rows), n_items, 1)
+        rows = _count_rows(n_items, R, count_rows)
         d_counts = mem.device("counts", rows * max_E * 4)
         d_npos = mem.device("npos", max(n_items, 1) * 4)
         d_ehist = None
@@ -449,22 +443,22 @@ class DevicePoolSelector:
         record(self.EVENT_SLOT)
         if not dry:
             self._last_exchange = ex
-            self._pending = (pin, views, n_req, n_items, max_E, n_count_rows, n_inst, device_y)
+            self._pending = _Readback(pin, views, n_req, n_inst, max_E, n_count_rows, device_y)
 
     def _view(self, name, dt):
-        pin, views = self._pending[0], self._pending[1]
+        pin, views = self._pending.pin, self._pending.views
         return pin.view(dt, views[name][1] // np.dtype(dt).itemsize, views[name][0])
 
     def result_counts(self):
         """(counts[n_items][max_E], npos[n_items]) -- available right after the first histogram pass."""
-        _, _, _, n_items, max_E, n_count_rows, _, device_y = self._pending
-        if device_y:
+        p = self._pending
+        if p.device_y:
             raise _lib.CsgError("per-file counts are not read back when the y candidates are computed on the device")
         self.ctx.event_sync(self.EVENT_SLOT - 1)
-        return self._view("counts", np.int32).reshape(n_count_rows, max_E).copy(), self._view("npos", np.int32).copy()
+        return self._view("counts", np.int32).reshape(p.n_count_rows, p.max_E).copy(), self._view("npos", np.int32).copy()
 
     def _out(self):
-        n_req, n_inst = self._pending[2], self._pending[6]
+        n_req, n_inst = self._pending.n_req, self._pending.n_inst
         self.ctx.event_sync(self.EVENT_SLOT)
         out = self._view("out", np.float64)
         flags = out[n_req + n_inst : n_req + n_inst + 4]
@@ -473,30 +467,37 @@ class DevicePoolSelector:
             if ex is not None and hasattr(ex, "clear_error"):
                 ex.clear_error()
             raise _lib.CsgError(f"peer exchange timed out waiting for rank {int(out[n_req + n_inst + 4]) - 1}")
-        return out, flags
+        return out[:n_req], out[n_req : n_req + n_inst], flags
 
     def result_values(self):
         """One float per request (None: empty pool), or None when the slot table overflowed."""
-        n_req = self._pending[2]
-        out, flags = self._out()
+        values, _, flags = self._out()
         if flags[1]:  # slot overflow: later digits ran on a truncated table, their flags mean nothing
             self.overflows = self.__dict__.get("overflows", 0) + 1
             return None
         if flags[0] or flags[2]:
             raise _lib.CsgError("device pool selection: a rank fell outside its bucket (histogram / scan mismatch)")
-        return [float(v) if np.isfinite(v) else None for v in out[:n_req]]
+        return [float(v) if np.isfinite(v) else None for v in values]
 
     def result_y_candidates(self):
         """Largest 99 %-coverage energy per instrument over the positions below ``limit`` (None:
         no position took part on any rank).  Only with ``ydev``."""
-        n_req, n_inst = self._pending[2], self._pending[6]
-        out, _ = self._out()
-        return [float(v) if v != -np.inf else None for v in out[n_req : n_req + n_inst]]
+        _, ycand, _ = self._out()
+        return [float(v) if v != -np.inf else None for v in ycand]
 
     def result(self):
         """(values | None on slot overflow, counts, npos); waits for the read-backs only."""
         counts, npos = self.result_counts()
         return self.result_values(), counts, npos
+
+
+# where the last DevicePoolSelector.enqueue lands its read-backs (views: {name: (byte offset, bytes)} in pin)
+_Readback = namedtuple("_Readback", "pin views n_req n_inst max_E n_count_rows device_y")
+
+
+def _count_rows(n_items: int, n_ranks: int, count_rows: int | None) -> int:
+    """Rows of this rank's per-file count table (several ranks: what every rank adds to the gather)."""
+    return max(n_items, 1) if (n_ranks == 1 or count_rows is None) else max(int(count_rows), n_items, 1)
 
 
 def _al(n: int, a: int = 64) -> int:

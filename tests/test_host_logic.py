@@ -160,8 +160,7 @@ def test_walk_chain_fast_path_equals_step_loop():
                 return (max(table[(inst, k)][0] for k in range(a, b + 1)), max(table[(inst, k)][1] for k in range(a, b + 1)),
                         table[(inst, b)][2])
 
-            folded_scan.range_max = range_max
-            folded = X._walk(sequence, order, ys, zs, json_copy(start), totals, 0.1, -1.0, folded_scan)
+            folded = X._walk(sequence, order, ys, zs, json_copy(start), totals, 0.1, -1.0, folded_scan, range_max=range_max)
             assert folded == slow, (trial, ys, zs)
 
 
@@ -282,7 +281,7 @@ def test_device_merged_extrema_equal_the_per_step_walk():
                 pending = X.extrema_enqueue(sh, sequence, order, ys, zs, json_copy(start), max_percentile=99.0,
                                             compute_mins=trial % 2 == 0, per_step=per_step)
                 if not per_step:
-                    assert pending["ydev"] is not None, "the chain preconditions hold for every case generated here"
+                    assert pending.ydev is not None, "the chain preconditions hold for every case generated here"
                 results.append(X.extrema_finish(pending))
             assert results[0] == results[1], (trial, ys, zs, results)
 
