@@ -22,6 +22,7 @@ import json
 import os
 import signal
 from concurrent.futures import ThreadPoolExecutor
+from dataclasses import dataclass
 from typing import Any
 
 import numpy as np
@@ -133,6 +134,23 @@ def FAST_plot_spectrograms_directory(
                 pass
 
 
+@dataclass
+class _Chunk:
+    """A chunk's K4 state between its encode and its progress records."""
+
+    encode: Any  # the open png.DeferredEncode of its last group, None once read back (or with nothing to draw)
+    writes: list  # futures of the framing + writing of its files
+    paths: list
+    planned: list  # (result, saves) per submission
+    n_jobs: int
+    seconds: float  # wall time so far
+
+    def read_back(self) -> None:
+        """Wait for the encode kernel and hand the last group to the writers."""
+        if self.encode is not None:
+            self.writes, self.encode = self.encode.complete(), None
+
+
 class _OpenEncode:
     """Leaves no deferred K4 encode open when the chunk loop is left by an exception (an interrupt): the next
     call in this process finds the encoder context free."""
@@ -144,10 +162,10 @@ class _OpenEncode:
         return self
 
     def __exit__(self, kind, _value, _trace):
-        state = self._current()
-        if kind is not None and state is not None and hasattr(state[0], "abandon"):
+        chunk = self._current()
+        if kind is not None and chunk is not None and chunk.encode is not None:
             try:
-                state[0].abandon()
+                chunk.encode.abandon()
             except Exception:
                 pass
         return False
@@ -348,21 +366,20 @@ def _run_directory(directory_path, output_base, y_scale, z_scale, zoom_duration_
     encoding = writing = None
     n_chunk = 0
 
-    def settle(chunk_state, since_flush):
+    def settle(chunk: _Chunk, since_flush):
         """The host half of a chunk ends here: its PNG files are on disk (the framing and writing ran on the
         encoder's finisher thread while the next chunk was ingested and planned), then the soft timeouts and
         the progress records -- in that order, so that progress never names an orbit whose files are missing."""
-        writes, paths, planned, n_jobs, seconds = chunk_state
         t_wait = _time.perf_counter()
-        for fut in writes:
+        for fut in chunk.writes:
             fut.result()
-        seconds += _time.perf_counter() - t_wait
-        for path in paths:
+        seconds = chunk.seconds + _time.perf_counter() - t_wait
+        for path in chunk.paths:
             log_exception(f"[SAVED] {path}", level="message")
         # soft timeouts, checked after the work like the reference's (process_orbit.py:203-211,276-283): a
         # chunk's wall time is shared evenly between its submissions
-        share = seconds / max(1, n_jobs)
-        for result, _s in planned:
+        share = seconds / max(1, chunk.n_jobs)
+        for result, _s in chunk.planned:
             if share > orbit_timeout_seconds and result["status"] == "ok":
                 log_exception(f"[TIMEOUT] Orbit {result['orbit']} exceeded {orbit_timeout_seconds:.0f}s total.", level="message")
                 result["status"], result["timeout_type"] = "timeout", "orbit"
@@ -447,25 +464,21 @@ def _run_directory(directory_path, output_base, y_scale, z_scale, zoom_duration_
                 writing = None
                 t_phase = tick("png_wait_previous_chunk", t_phase)
             if encoding is not None:  # the last chunk: its kernel ran while this one was planned
-                if not isinstance(encoding[0], list):
-                    encoding[0] = encoding[0].complete()
+                encoding.read_back()
                 writing, encoding = encoding, None
                 t_phase = tick("png_read_back", t_phase)
+            handle = None  # nothing to draw: the chunk still takes its turn, so that progress is recorded in orbit order
             if saves:
                 encoder_ctx.wait_for(ctx)  # (the rasters are complete: step.finish() above; ordering kept explicit)
                 handle = write_figures_device(encoder_ctx, b.d_rgba.ptr, saves, max_workers=n_threads, dpi=SAVE_DPI,
-                                              timings=png_timings, wait=False, defer=True, code_cache=code_cache,
-                                              max_segments=1_000_000)
+                                              timings=png_timings, defer=True, code_cache=code_cache, max_segments=1_000_000)
                 for _path, fig in saves:
                     close_all_axes_and_clear(fig)
-                encoding = [handle, [path for path, _f in saves], planned, len(jobs), _time.perf_counter() - t_chunk]
-            else:  # nothing to draw: the chunk still takes its turn, so that progress is recorded in orbit order
-                encoding = [[], [], planned, len(jobs), _time.perf_counter() - t_chunk]
+            encoding = _Chunk(handle, [], [path for path, _f in saves], planned, len(jobs), _time.perf_counter() - t_chunk)
             t_phase = tick("png_encode", t_phase)
         for state in (writing, encoding):  # oldest first: progress is recorded in orbit order
             if state is not None:
-                if not isinstance(state[0], list):
-                    state[0] = state[0].complete()
+                state.read_back()
                 since_flush = settle(state, since_flush)
         t_phase = tick("png_wait_last_chunk", t_phase)
 

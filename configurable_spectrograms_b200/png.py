@@ -7,7 +7,9 @@ Two encoders, one file format (8-bit RGBA, non-interlaced):
   rasters are host arrays (the single-figure entry points);
 * :func:`encode_figures_device` / :func:`write_figures_device` -- figures whose panels are K3 rasters
   in HBM are composed, Up-filtered and DEFLATE-encoded on the GPU (``csrc/png.cu``); only the
-  compressed bytes cross PCIe.  The host adds the zlib header / trailer and the PNG chunk framing.
+  compressed bytes cross PCIe.  The host adds the zlib header / trailer and the PNG chunk framing.  It
+  returns the PNG bytes, writes the files and waits, or writes them deferred (``defer=True``: the last
+  group's kernel still runs when the call returns).
 
 Both decode to the same pixels (``tests/test_gpu_api.py``); the host composer is the oracle of the
 device one.
@@ -17,8 +19,10 @@ from __future__ import annotations
 
 import os
 import struct
+import time
 import zlib
 from concurrent.futures import ThreadPoolExecutor
+from typing import NamedTuple
 
 import numpy as np
 
@@ -82,15 +86,6 @@ def decode_rgba(data: bytes) -> np.ndarray:
             if up[r] and r > 0:
                 out[r] += out[r - 1]
     return out.reshape(h, w, 4)
-
-
-def write_many(jobs, compress_level: int = 6, max_workers: int = 8) -> None:
-    """``jobs``: iterable of (path, image).  Encodes and writes on a thread pool."""
-    jobs = list(jobs)
-    if not jobs:
-        return
-    with ThreadPoolExecutor(max_workers=max(1, min(max_workers, len(jobs)))) as pool:
-        list(pool.map(lambda j: write_rgba(j[0], j[1], compress_level), jobs))
 
 
 # ----------------------------------------------------------------------------------------
@@ -371,22 +366,24 @@ def zero_segment_table(widths) -> np.ndarray:
     return table
 
 
-def _device_tables(figures, dpi):
-    """Tile / canvas / row tables of a list of figures.  Returns ``(canvases, tiles, rows, row_maps, per_figure)``
-    with ``canvases`` a list of mutable rows of ``PNG_CANVAS`` (``seg_first`` is filled per group), ``tiles`` one
-    ``PNG_TILE`` array, ``rows`` one int32 array of content rows, ``row_maps`` the int32 row maps of the panels
-    on a log energy axis (each distinct map once; ``None`` when there are none) and ``per_figure`` =
-    [(W, H, content rows)]."""
-    from ._lib import PNG_TILE
+class DeviceTables(NamedTuple):
+    """What K4 reads of a list of figures (:func:`_device_tables`)."""
+
+    canvases: np.ndarray  # PNG_CANVAS, one row per figure; seg_first counts from the figure's group (_groups)
+    tiles: np.ndarray  # PNG_TILE, every figure's tiles in figure order
+    rows: np.ndarray  # int32 content rows: figure k's are rows[row_first : row_first + n_rows[k]]
+    n_rows: np.ndarray  # content rows per figure
+    row_maps: np.ndarray | None  # int32 row maps of the panels on a log energy axis, each distinct map once
+
+
+def _device_tables(figures, dpi) -> DeviceTables:
+    """Tile / canvas / row tables of a list of figures (an empty tile or row table is one zero entry)."""
+    from ._lib import PNG_CANVAS, PNG_TILE
     from .figure import DeviceRaster
 
-    def pack(c):
-        r, g, b, a = c
-        return r | (g << 8) | (b << 16) | (a << 24)
-
-    canvases, tile_parts, row_parts, per_figure = [], [], [], []
+    widths, heights, backgrounds, tile_parts, row_parts = [], [], [], [], []
     map_at, map_parts = {}, []  # row-map key -> offset in the concatenated maps
-    n_tiles = n_rows = n_map = 0
+    n_map = 0
     for fig in figures:
         t = fig.tiles(dpi)
         for src in t.sources.values():
@@ -398,22 +395,236 @@ def _device_tables(figures, dpi):
                 map_parts.append(rows)
                 n_map += len(rows)
         table = t.table([map_at[key] for key, _rows in t.row_maps])
-        rows = t.content_rows(table)
-        canvases.append([t.W, t.H, n_tiles, len(table), pack(t.background), 0, (t.W + 1023) // 1024, n_rows])
+        r, g, b, a = t.background
+        widths.append(t.W)
+        heights.append(t.H)
+        backgrounds.append(r | (g << 8) | (b << 16) | (a << 24))
         tile_parts.append(table)
-        row_parts.append(rows)
-        per_figure.append((t.W, t.H, rows))
-        n_tiles += len(table)
-        n_rows += len(rows)
-    tiles = np.concatenate(tile_parts) if n_tiles else np.zeros(1, PNG_TILE)
-    rows = np.concatenate(row_parts) if n_rows else np.zeros(1, np.int32)
+        row_parts.append(t.content_rows(table))
+    n_tiles = np.array([len(t) for t in tile_parts], dtype=np.int64)
+    n_rows = np.array([len(r) for r in row_parts], dtype=np.int64)
+    canvases = np.zeros(len(figures), dtype=PNG_CANVAS)
+    canvases["W"], canvases["H"], canvases["background"] = widths, heights, backgrounds
+    canvases["tile_first"], canvases["tile_count"] = np.cumsum(n_tiles) - n_tiles, n_tiles
+    canvases["segs_per_row"] = (canvases["W"] + 1023) // 1024
+    canvases["row_first"] = np.cumsum(n_rows) - n_rows
+    tiles = np.concatenate(tile_parts) if n_tiles.sum() else np.zeros(1, PNG_TILE)
+    rows = np.concatenate(row_parts) if n_rows.sum() else np.zeros(1, np.int32)
     row_maps = np.concatenate(map_parts).astype(np.int32) if n_map else None
-    return canvases, tiles, rows, row_maps, per_figure
+    return DeviceTables(canvases, tiles, rows, n_rows, row_maps)
 
 
-def encode_figures_device(ctx, d_rgba_ptr: int, figures, dpi: float | None = None, max_segments: int = 400_000, consume=None,
-                          timings: dict | None = None, wait: bool = True, code_cache: dict | None = None,
-                          paths=None, write_threads: int = 16, defer: bool = False):
+class _Group(NamedTuple):
+    """Figures ``first .. stop - 1`` of a call: one encode kernel."""
+
+    first: int
+    stop: int
+    n_seg: int  # their scanline segments
+
+
+def _groups(canvases, n_rows, max_segments: int) -> list[_Group]:
+    """Split the figures, in order, into groups of at most ``max_segments`` scanline segments and number every
+    canvas' segments from its group's first (``seg_first``).  A group takes at least one figure, so a figure
+    larger than the budget is a group of its own."""
+    segs = (canvases["segs_per_row"].astype(np.int64) * n_rows).tolist()
+    groups, seg_first = [], []
+    first = n_seg = 0
+    for k, s in enumerate(segs):
+        if k > first and n_seg + s > max_segments:
+            groups.append(_Group(first, k, n_seg))
+            first, n_seg = k, 0
+        seg_first.append(n_seg)
+        n_seg += s
+    if segs:
+        groups.append(_Group(first, len(segs), n_seg))
+    canvases["seg_first"] = seg_first
+    return groups
+
+
+def _tick(timings, name, t0):
+    if timings is not None:
+        timings[name] = timings.get(name, 0.0) + time.perf_counter() - t0
+    return time.perf_counter()
+
+
+class _Encoder:
+    """K4's host state on one context, kept across calls: the grow-only device scratch, the two pinned read-back
+    buffers with the futures of the host work that reads them, the finisher thread that frames and hands over the
+    groups, its framer pool, and the open deferred encode.  Groups are pipelined: while the finisher frames
+    (CRC-32) and hands over group g from one pinned buffer, the caller already encodes, compacts and reads back
+    group g + 1 into the other one -- across calls too."""
+
+    def __init__(self, ctx):
+        self.ctx = ctx
+        self.scratch: dict = {}
+        self.pinned: list = [None, None]
+        self.in_flight: list = [None, None]  # the future of the host work reading pinned buffer 0 / 1
+        self.groups = 0  # groups read back on this context: the parity of the next pinned buffer
+        self.finisher = ThreadPoolExecutor(max_workers=1, thread_name_prefix="csg-png")
+        self.framers = ThreadPoolExecutor(max_workers=16, thread_name_prefix="csg-crc")
+        self.deferred: DeferredEncode | None = None
+
+    @staticmethod
+    def of(ctx) -> "_Encoder":
+        enc = ctx.__dict__.get("_png_encoder")
+        if enc is None:
+            enc = ctx._png_encoder = _Encoder(ctx)
+        return enc
+
+    def dev(self, name: str, nbytes: int):
+        buf = self.scratch.get(name)
+        if buf is None or buf.nbytes < nbytes:
+            buf = self.scratch[name] = self.ctx.alloc(int(nbytes * 1.2) + 256)
+        return buf
+
+
+class _Launched(NamedTuple):
+    """A group whose encode kernel is enqueued.  It holds what the kernel reads: its canvas table, and through
+    ``call`` the call's tiles, content rows, zero-segment table and row maps."""
+
+    call: "_Call"
+    group: _Group
+    d_canvases: object
+    d_slots: object
+    d_sizes: object
+    d_adler: object
+
+
+class _Call:
+    """One :func:`encode_figures_device` call: its device tables, the groups it launches and reads back, and the
+    futures of their host work."""
+
+    def __init__(self, enc: _Encoder, d_rgba_ptr: int, tables: DeviceTables, timings, code_cache, paths, write_threads):
+        from .overlay import ATLAS
+
+        ctx = enc.ctx
+        self.enc, self.ctx, self.lib, self.tables = enc, ctx, ctx.lib, tables
+        self.d_rgba_ptr, self.timings, self.code_cache = d_rgba_ptr, timings, code_cache
+        self.paths, self.write_threads = paths, write_threads
+        self.slot = int(self.lib.csg_png_slot_bytes())
+        self.d_tiles, self.d_rows = ctx.to_device(tables.tiles), ctx.to_device(tables.rows)
+        self.d_row_maps = ctx.to_device(tables.row_maps) if tables.row_maps is not None else None
+        zero_table = zero_segment_table(tables.canvases["W"]) if len(tables.canvases) else np.zeros(0, dtype=np.uint8)
+        self.d_zero = ctx.to_device(zero_table) if len(zero_table) else None
+        self.zero_args = (self.d_zero.ptr if self.d_zero is not None else None, len(zero_table))
+        self.maps_ptr = self.d_row_maps.ptr if self.d_row_maps is not None else None
+        self.d_overlay = ATLAS.device_ptr(ctx)
+        self.d_error = enc.dev("error", 4)
+        self.d_error.zero()
+        self.futures: list = []
+        self.results: dict[int, list] = {}
+
+    def tick(self, name, t0):
+        return _tick(self.timings, name, t0)
+
+    def launch(self, group: _Group) -> _Launched:
+        """The group's canvas table, the code of the call (first group), the encode kernel: nothing waits for the
+        GPU except the one-time count pass."""
+        ctx, lib, enc, n_seg = self.ctx, self.lib, self.enc, group.n_seg
+        t0 = time.perf_counter()
+        d_canvases = ctx.to_device(self.tables.canvases[group.first : group.stop])
+        n_canvases = group.stop - group.first
+        if group.first == 0:  # the code of this call
+            if self.code_cache is not None and "tables" in self.code_cache:
+                ctx._check(lib.csg_png_set_tables(ctx.handle, self.code_cache["tables"].ctypes.data))
+            else:
+                d_counts = enc.dev("counts", 316 * 4)
+                d_counts.zero()
+                ctx._check(lib.csg_png_set_tables(ctx.handle, None))  # the count pass needs valid symbol tables
+                ctx._check(lib.csg_png_count(ctx.handle, self.d_rgba_ptr, self.d_overlay, d_canvases.ptr, n_canvases,
+                                             self.d_tiles.ptr, None, self.d_rows.ptr, n_seg, 4, d_counts.ptr,
+                                             *self.zero_args, self.maps_ptr))
+                tables = np.ascontiguousarray(custom_tables(d_counts.download(np.uint32, 316)))
+                ctx._check(lib.csg_png_set_tables(ctx.handle, tables.ctypes.data))
+                if self.code_cache is not None:
+                    self.code_cache["tables"] = tables
+            t0 = self.tick("code_tables", t0)
+        d_slots, d_sizes, d_adler = enc.dev("slots", n_seg * self.slot), enc.dev("sizes", n_seg * 4), enc.dev("adler", n_seg * 8)
+        ctx._check(lib.csg_png_encode(ctx.handle, self.d_rgba_ptr, self.d_overlay, d_canvases.ptr, n_canvases, self.d_tiles.ptr,
+                                      None, self.d_rows.ptr, n_seg, d_slots.ptr, d_sizes.ptr, d_adler.ptr, self.d_error.ptr,
+                                      *self.zero_args, self.maps_ptr))
+        self.tick("encode_launch", t0)
+        return _Launched(self, group, d_canvases, d_slots, d_sizes, d_adler)
+
+    def complete(self, launched: _Launched) -> None:
+        """Sizes back (waits for the kernel), compaction, read-back into a pinned buffer, hand-over to the finisher."""
+        ctx, lib, enc = self.ctx, self.lib, self.enc
+        group, n_seg = launched.group, launched.group.n_seg
+        t0 = time.perf_counter()
+        sizes = launched.d_sizes.download(np.int32, n_seg, sync=False)
+        bad = self.d_error.download(np.int32, 1, sync=False)
+        adler = launched.d_adler.download(np.uint32, 2 * n_seg).reshape(n_seg, 2)  # synchronises
+        if bad[0] < 0:
+            raise ValueError(f"figure {group.first - int(bad[0]) - 1}: a tile reads a row map, but no row-map table was given")
+        if bad[0]:
+            raise ValueError(f"figure {group.first + int(bad[0]) - 1}: more than {int(lib.csg_png_max_segment_tiles())} tiles "
+                             "meet in one 1024-pixel scanline segment")
+        t0 = self.tick("encode_kernel_and_sizes", t0)
+        offsets = np.zeros(n_seg + 1, dtype=np.int64)
+        np.cumsum(sizes, out=offsets[1:])
+        total = int(offsets[-1])
+        d_off = enc.dev("offsets", n_seg * 8)
+        d_off.upload(offsets[:-1])
+        d_packed = enc.dev("packed", total)
+        ctx._check(lib.csg_png_compact(ctx.handle, launched.d_slots.ptr, launched.d_sizes.ptr, d_off.ptr, n_seg, d_packed.ptr))
+        parity = enc.groups & 1
+        if enc.in_flight[parity] is not None:
+            enc.in_flight[parity].result()  # the group that last used this pinned buffer is handed over
+            enc.in_flight[parity] = None
+            t0 = self.tick("wait_for_host", t0)
+        pin = enc.pinned[parity]
+        if pin is None or pin.nbytes < total:
+            pin = enc.pinned[parity] = ctx.pinned(int(total * 1.2) + 4096)
+        ctx._check(lib.csg_d2h(ctx.handle, pin.ptr, d_packed.ptr, total))
+        ctx.sync()
+        self.tick("compact_and_d2h", t0)
+        enc.in_flight[parity] = enc.finisher.submit(self._finish, group, pin.array, offsets, adler)
+        self.futures.append(enc.in_flight[parity])
+        enc.groups += 1
+
+    def _finish(self, group: _Group, packed, offsets, adler) -> None:
+        """The host work of a read-back group, on the finisher thread: its files framed and written natively, or
+        framed into bytes."""
+        t1 = time.perf_counter()
+        canvases = self.tables.canvases[group.first : group.stop]
+        n_rows = self.tables.n_rows[group.first : group.stop]
+        if self.paths is not None:
+            write_files_native(self.lib, self.paths[group.first : group.stop], canvases, n_rows, self.tables.rows, packed,
+                               offsets, adler, self.write_threads)
+            self.tick("frame_and_write_native", t1)
+            return
+        rows = self.tables.rows
+
+        def frame(canvas, n):
+            first = int(canvas["row_first"])
+            return assemble_png(int(canvas["W"]), int(canvas["H"]), rows[first : first + int(n)], int(canvas["segs_per_row"]),
+                                packed, offsets, int(canvas["seg_first"]), adler)
+
+        parts = list(self.enc.framers.map(frame, canvases, n_rows))
+        t1 = self.tick("framing_crc", t1)
+        self.results[group.first] = [b"".join(p) for p in parts]
+        self.tick("consume", t1)  # the join keeps this phase name, so bench lines stay comparable
+
+    def settle(self) -> None:
+        """Leave no host work of a failed or abandoned call behind."""
+        for fut in self.futures:
+            try:
+                fut.result()
+            except Exception:
+                pass
+
+    def wait(self) -> list:
+        """Every group's host work done: the PNG files (an empty list when they were written)."""
+        t0 = time.perf_counter()
+        for fut in self.futures:
+            fut.result()
+        self.tick("wait_for_host", t0)
+        return [blob for first in sorted(self.results) for blob in self.results[first]]
+
+
+def encode_figures_device(ctx, d_rgba_ptr: int, figures, dpi: float | None = None, max_segments: int = 400_000,
+                          timings: dict | None = None, code_cache: dict | None = None, paths=None, write_threads: int = 16,
+                          defer: bool = False):
     """PNG bytes of every figure, composed and DEFLATE-encoded on the GPU.
 
     ``figures``: :class:`figure.SpectrogramFigure` objects whose panels were drawn from
@@ -424,9 +635,6 @@ def encode_figures_device(ctx, d_rgba_ptr: int, figures, dpi: float | None = Non
     (:func:`zero_run`).  Figures are processed in groups of at most ``max_segments`` scanline segments
     (scratch: 4.6 KB each).
 
-    ``consume(first_figure_index, parts)``: instead of returning the files, hand every group's files
-    -- each a list of buffers, some aliasing pinned scratch that is valid only during the call -- to the
-    caller (``write_figures_device`` writes them straight to disk without assembling them in memory).
     ``timings`` (optional dict) accumulates host seconds per phase.  The DEFLATE code is a dynamic-Huffman
     code fitted to the symbol statistics of the first group of figures (one counting pass of the same
     tokeniser over every 4th scanline segment) and used for the whole call.  ``code_cache`` (a dict the
@@ -435,248 +643,91 @@ def encode_figures_device(ctx, d_rgba_ptr: int, figures, dpi: float | None = Non
 
     ``paths`` (one per figure): frame and write the files natively (``csg_png_write_files``: CRC-32 +
     ``writev`` from the pinned buffer on ``write_threads`` native threads, no interpreter lock held) instead of
-    building them here; nothing is returned or handed to ``consume`` then.
+    building them here; the call returns an empty list once they are written.
 
-    ``defer=True`` (with ``wait=False``): the LAST group's encode kernel is only launched; the call returns a
+    ``defer=True`` (needs ``paths``): the LAST group's encode kernel is only launched; the call returns a
     :class:`DeferredEncode` whose ``complete()`` reads the sizes back, compacts, copies out and hands the
     group to the finisher thread -- the caller does host work (plans the next chunk) while the kernel runs,
-    and must call ``complete()`` before the next encode on this context.
-
-    ``wait=False`` (needs ``consume`` or ``paths``): return as soon as the last group is read back, with the futures of
-    the host work (framing + ``consume``) still running on the context's finisher thread; the caller
-    collects them (``future.result()``) before it relies on the files.  The next call on the same context
-    may start meanwhile -- the two pinned read-back buffers are fenced by those futures.
+    and must call ``complete()`` or ``abandon()`` before the next encode on this context.  The files are
+    complete once every future ``complete()`` returns has its ``result()``.
     """
-    import time
-
-    def tick(name, t0):
-        if timings is not None:
-            timings[name] = timings.get(name, 0.0) + time.perf_counter() - t0
-        return time.perf_counter()
-
-    from ._lib import PNG_CANVAS
-    from .overlay import ATLAS
-
-    lib = ctx.lib
     figures = list(figures)
     t0 = time.perf_counter()
-    canvases, tiles, rows, row_maps, per_figure = _device_tables(figures, dpi)
-    slot = int(lib.csg_png_slot_bytes())
-    scratch = ctx.__dict__.setdefault("_png_scratch", {})
-    if scratch.get("deferred") is not None:
+    tables = _device_tables(figures, dpi)
+    enc = _Encoder.of(ctx)
+    if enc.deferred is not None:
         raise RuntimeError("a deferred encode is still open on this context: call its complete() first")
-    if defer and wait:
-        raise ValueError("defer=True needs wait=False")
-
-    def dev(name, nbytes):
-        buf = scratch.get(name)
-        if buf is None or buf.nbytes < nbytes:
-            buf = scratch[name] = ctx.alloc(int(nbytes * 1.2) + 256)
-        return buf
-
-    d_tiles, d_rows = ctx.to_device(tiles), ctx.to_device(rows)
-    d_row_maps = ctx.to_device(row_maps) if row_maps is not None else None
-    maps_ptr = d_row_maps.ptr if d_row_maps is not None else None
-    zero_table = zero_segment_table([c[0] for c in canvases]) if canvases else np.zeros(0, dtype=np.uint8)
-    d_zero = ctx.to_device(zero_table) if len(zero_table) else None
-    zero_args = (d_zero.ptr if d_zero is not None else None, len(zero_table))
-    d_overlay = ATLAS.device_ptr(ctx)
-    d_error = dev("error", 4)
-    d_error.zero()
-    t0 = tick("tile_tables", t0)
-    # Groups are pipelined: while a background thread frames (CRC-32) and hands over group g from one pinned
-    # buffer, this thread already encodes, compacts and reads back group g + 1 into the other one.  The
-    # thread and the fences of the two buffers belong to the context, so the pipeline runs across calls too.
-    if not wait and consume is None and paths is None:
-        raise ValueError("wait=False needs a consume callback or paths (the files are handed over, not returned)")
+    if defer and paths is None:
+        raise ValueError("defer=True needs paths (the files are written, not returned)")
     if paths is not None and len(paths) != len(figures):
         raise ValueError(f"{len(paths)} paths for {len(figures)} figures")
-    results: dict[int, list] = {}
-    pipe = scratch.get("finisher")
-    if pipe is None:
-        pipe = scratch["finisher"] = {"pool": ThreadPoolExecutor(max_workers=1, thread_name_prefix="csg-png"),
-                                      "framers": ThreadPoolExecutor(max_workers=16, thread_name_prefix="csg-crc"),
-                                      "in_flight": [None, None], "groups": 0}
-    finisher, framers, in_flight = pipe["pool"], pipe["framers"], pipe["in_flight"]  # in_flight: the future reading pinned buffer 0 / 1
-    mine: list = []
-
-    def launch(k, group, n_seg):
-        """Tables of the group, the code of the call (first group), the encode kernel: nothing waits for the GPU
-        except the one-time count pass."""
-        t0 = time.perf_counter()
-        table = np.array([tuple(c) for c in group], dtype=PNG_CANVAS)
-        d_canvases = ctx.to_device(table)
-        if k == 0:  # the code of this call
-            if code_cache is not None and "tables" in code_cache:
-                ctx._check(lib.csg_png_set_tables(ctx.handle, code_cache["tables"].ctypes.data))
-            else:
-                d_counts = dev("counts", 316 * 4)
-                d_counts.zero()
-                ctx._check(lib.csg_png_set_tables(ctx.handle, None))  # the count pass needs valid symbol tables
-                ctx._check(lib.csg_png_count(ctx.handle, d_rgba_ptr, d_overlay, d_canvases.ptr, len(group), d_tiles.ptr, None,
-                                             d_rows.ptr, n_seg, 4, d_counts.ptr, *zero_args, maps_ptr))
-                tables = np.ascontiguousarray(custom_tables(d_counts.download(np.uint32, 316)))
-                ctx._check(lib.csg_png_set_tables(ctx.handle, tables.ctypes.data))
-                if code_cache is not None:
-                    code_cache["tables"] = tables
-            t0 = tick("code_tables", t0)
-        d_slots, d_sizes, d_adler = dev("slots", n_seg * slot), dev("sizes", n_seg * 4), dev("adler", n_seg * 8)
-        ctx._check(lib.csg_png_encode(ctx.handle, d_rgba_ptr, d_overlay, d_canvases.ptr, len(group), d_tiles.ptr, None,
-                                      d_rows.ptr, n_seg, d_slots.ptr, d_sizes.ptr, d_adler.ptr, d_error.ptr, *zero_args, maps_ptr))
-        tick("encode_launch", t0)
-        return (k, group, n_seg, d_canvases, d_slots, d_sizes, d_adler)
-
-    def complete(state):
-        """Sizes back (waits for the kernel), compaction, read-back into a pinned buffer, hand-over."""
-        k, group, n_seg, _d_canvases, d_slots, d_sizes, d_adler = state
-        t0 = time.perf_counter()
-        sizes = d_sizes.download(np.int32, n_seg, sync=False)
-        bad = d_error.download(np.int32, 1, sync=False)
-        adler = d_adler.download(np.uint32, 2 * n_seg).reshape(n_seg, 2)  # synchronises
-        if bad[0] < 0:
-            raise ValueError(f"figure {k - int(bad[0]) - 1}: a tile reads a row map, but no row-map table was given")
-        if bad[0]:
-            raise ValueError(f"figure {k + int(bad[0]) - 1}: more than {int(lib.csg_png_max_segment_tiles())} tiles meet in one "
-                             "1024-pixel scanline segment")
-        t0 = tick("encode_kernel_and_sizes", t0)
-        offsets = np.zeros(n_seg + 1, dtype=np.int64)
-        np.cumsum(sizes, out=offsets[1:])
-        total = int(offsets[-1])
-        d_off = dev("offsets", n_seg * 8)
-        d_off.upload(offsets[:-1])
-        d_packed = dev("packed", total)
-        ctx._check(lib.csg_png_compact(ctx.handle, d_slots.ptr, d_sizes.ptr, d_off.ptr, n_seg, d_packed.ptr))
-        parity = pipe["groups"] & 1
-        if in_flight[parity] is not None:
-            in_flight[parity].result()  # the group that last used this pinned buffer is on disk
-            in_flight[parity] = None
-            t0 = tick("wait_for_host", t0)
-        name = f"pinned{parity}"
-        pin = scratch.get(name)
-        if pin is None or pin.nbytes < total:
-            pin = scratch[name] = ctx.pinned(int(total * 1.2) + 4096)
-        ctx._check(lib.csg_d2h(ctx.handle, pin.ptr, d_packed.ptr, total))
-        ctx.sync()
-        t0 = tick("compact_and_d2h", t0)
-
-        def finish(first=k, group=group, jobs=per_figure[k : k + len(group)], packed=pin.array, offsets=offsets, adler=adler):
-            t1 = time.perf_counter()
-            if paths is not None:
-                write_files_native(lib, paths[first : first + len(group)], group, jobs, rows, packed, offsets, adler, write_threads)
-                tick("frame_and_write_native", t1)
-                return
-            parts = list(framers.map(lambda job: assemble_png(job[1][0], job[1][1], job[1][2], job[0][6], packed, offsets, job[0][5], adler),
-                                     zip(group, jobs)))
-            t1 = tick("framing_crc", t1)
-            if consume is not None:
-                consume(first, parts)  # the buffers alias pinned scratch that the group after next overwrites
-            else:
-                results[first] = [b"".join(p) for p in parts]
-            tick("consume", t1)
-
-        in_flight[parity] = finisher.submit(finish)
-        mine.append(in_flight[parity])
-        pipe["groups"] += 1
-
-    def settle_failed():
-        for fut in mine:  # leave no work of a failed call behind
-            try:
-                fut.result()
-            except Exception:
-                pass
-
-    k = 0
-    open_state = None
+    call = _Call(enc, d_rgba_ptr, tables, timings, code_cache, paths, write_threads)
+    _tick(timings, "tile_tables", t0)
+    groups = _groups(tables.canvases, tables.n_rows, max_segments)
+    last = groups.pop() if defer and groups else None
     try:
-        while k < len(figures):
-            # ---- the next group of figures that fits the segment budget
-            group, n_seg = [], 0
-            while k + len(group) < len(figures):
-                c = canvases[k + len(group)]
-                segs = c[6] * len(per_figure[k + len(group)][2])
-                if group and n_seg + segs > max_segments:
-                    break
-                c[5] = n_seg
-                group.append(c)
-                n_seg += segs
-            state = launch(k, group, n_seg)
-            k += len(group)
-            if defer and k >= len(figures):
-                open_state = state
-                break
-            complete(state)
+        for group in groups:
+            call.complete(call.launch(group))
+        if last is not None:
+            last = call.launch(last)
     except BaseException:
-        settle_failed()
+        call.settle()
         raise
-    if open_state is not None:
-        keep_alive = {"tables": (d_tiles, d_rows, d_zero, d_row_maps)}  # device tables the open kernel reads
-
-        def complete_open():
-            try:
-                complete(open_state)
-            except BaseException:
-                settle_failed()
-                raise
-            finally:
-                scratch["deferred"] = None
-                keep_alive.clear()
-            return mine
-
-        def abandon_open():
-            try:
-                ctx.sync()  # the kernel still reads the tables kept alive here
-            finally:
-                scratch["deferred"] = None
-                keep_alive.clear()
-                settle_failed()
-
-        handle = DeferredEncode(complete_open, abandon_open)
-        scratch["deferred"] = handle
-        return handle
-    if not wait:
-        return mine
-    t0 = time.perf_counter()
-    for fut in mine:
-        fut.result()
-    tick("wait_for_host", t0)
-    return [blob for first in sorted(results) for blob in results[first]]
+    if not defer:
+        return call.wait()
+    handle = DeferredEncode(last)
+    if last is not None:
+        enc.deferred = handle
+    return handle
 
 
 class DeferredEncode:
-    """The open end of ``encode_figures_device(..., defer=True)``: ``complete()`` finishes the last group and
-    returns the futures of every group's host work (framing + writing)."""
+    """The open end of ``encode_figures_device(..., defer=True)``: its last group, whose encode kernel may still
+    run.  ``complete()`` finishes that group and returns the futures of every group's host work (framing +
+    writing)."""
 
-    def __init__(self, complete, abandon=None):
-        self._complete, self._abandon = complete, abandon
-        self.futures: list | None = None
+    def __init__(self, last: _Launched | None):
+        self._last = last
+        self.futures: list | None = None if last is not None else []
 
     def complete(self) -> list:
-        if self._complete is not None:
-            fn, self._complete, self._abandon = self._complete, None, None
-            self.futures = fn()
+        last, self._last = self._last, None
+        if last is not None:
+            call = last.call
+            try:
+                call.complete(last)
+            except BaseException:
+                call.settle()
+                raise
+            finally:
+                call.enc.deferred = None
+            self.futures = call.futures
         return self.futures or []
 
     def abandon(self) -> None:
         """Give the last group up (an interrupted run): wait for its kernel, release the context for the next
         encode; the groups already handed over finish as usual."""
-        if self._abandon is not None:
-            fn, self._complete, self._abandon = self._abandon, None, None
-            fn()
+        last, self._last = self._last, None
+        if last is not None:
+            call = last.call
+            try:
+                call.ctx.sync()  # the kernel still reads the tables `last` holds
+            finally:
+                call.enc.deferred = None
+                call.settle()
 
 
-def write_files_native(lib, paths, group, jobs, rows, packed, offsets, adler, n_threads: int = 16) -> None:
-    """Frame and write one group's files through ``csg_png_write_files``.  ``group``: the canvases' table rows
-    (``[W, H, tile_first, tile_count, background, seg_first, segs_per_row, row_first]``); ``jobs``:
-    ``(W, H, content rows)`` per figure; ``rows``: every canvas' content rows, concatenated."""
+def write_files_native(lib, paths, canvases, n_rows, rows, packed, offsets, adler, n_threads: int = 16) -> None:
+    """Frame and write one group's files through ``csg_png_write_files``.  ``canvases``: the figures' ``PNG_CANVAS``
+    rows; ``n_rows``: their content rows each; ``rows``: every canvas' content rows, concatenated."""
     from ._lib import PNG_FILE, CsgError
 
-    table = np.zeros(len(group), dtype=PNG_FILE)
-    encoded = [os.fsencode(p) + b"\0" for p in paths]
-    keep = [np.frombuffer(e, dtype=np.uint8) for e in encoded]
-    for entry, c, job, name in zip(table, group, jobs, keep):
-        entry["path"] = name.ctypes.data
-        entry["row_first"], entry["seg_first"] = c[7], c[5]
-        entry["width"], entry["height"], entry["n_rows"], entry["segs_per_row"] = c[0], c[1], len(job[2]), c[6]
+    table = np.zeros(len(canvases), dtype=PNG_FILE)
+    keep = [np.frombuffer(os.fsencode(p) + b"\0", dtype=np.uint8) for p in paths]
+    table["path"] = [name.ctypes.data for name in keep]
+    table["row_first"], table["seg_first"] = canvases["row_first"], canvases["seg_first"]
+    table["width"], table["height"] = canvases["W"], canvases["H"]
+    table["n_rows"], table["segs_per_row"] = n_rows, canvases["segs_per_row"]
     rows = np.ascontiguousarray(rows, dtype=np.int32)
     offsets = np.ascontiguousarray(offsets, dtype=np.int64)
     adler = np.ascontiguousarray(adler, dtype=np.uint32)
@@ -691,12 +742,11 @@ def write_files_native(lib, paths, group, jobs, rows, packed, offsets, adler, n_
 
 def write_figures_device(ctx, d_rgba_ptr: int, jobs, max_workers: int = 8, **kwargs):
     """``jobs``: iterable of (path, figure).  Device encode; every group's files are framed and written
-    straight from the pinned read-back buffer by native threads (``csg_png_write_files``).  With
-    ``wait=False`` the call returns the futures of the framing + writing still under way (see
-    :func:`encode_figures_device`); the files are complete once every ``future.result()`` has returned."""
+    straight from the pinned read-back buffer by native threads (``csg_png_write_files``).  Returns ``[]`` once
+    the files are written, or with ``defer=True`` the :class:`DeferredEncode` of the last group (see
+    :func:`encode_figures_device`)."""
     jobs = list(jobs)
     if not jobs:
         return []
-    out = encode_figures_device(ctx, d_rgba_ptr, [fig for _p, fig in jobs], paths=[str(p) for p, _f in jobs],
-                                write_threads=max(1, int(max_workers)), **kwargs)
-    return out if kwargs.get("wait") is False else []  # (futures, or a DeferredEncode with defer=True)
+    return encode_figures_device(ctx, d_rgba_ptr, [fig for _p, fig in jobs], paths=[str(p) for p, _f in jobs],
+                                 write_threads=max(1, int(max_workers)), **kwargs)

@@ -250,6 +250,45 @@ def test_directory_driver_streams_in_small_chunks(tmp_path, monkeypatch):
         assert np.array_equal(a, c), name
 
 
+def test_directory_driver_interrupted_run_frees_the_encoder(tmp_path, monkeypatch):
+    """An interrupt while the second chunk of 2 orbits is planned, with the first chunk's encode still open
+    (``png.DeferredEncode``): the call raises and gives that encode up, progress names no orbit whose PNGs are
+    missing, and a second call in the same process encodes again and writes what an uninterrupted run writes."""
+    from configurable_spectrograms_b200 import png
+    import configurable_spectrograms_b200.fast.batch_directory as BD
+
+    _write_tree(tmp_path)
+    monkeypatch.chdir(tmp_path)
+    monkeypatch.setenv("CSG_CHUNK_ORBITS", "2")
+    gold = load_json("extrema_tree.json")
+    _run_driver(output_base="./full/", progress_json_path="./full.json")
+    real, seen = BD.figure_from_spec, set()
+
+    def interrupting(shard, spec, *args, **kwargs):
+        seen.add(spec.orbit)
+        if len(seen) > 2:  # the first figure of the second chunk
+            raise KeyboardInterrupt
+        return real(shard, spec, *args, **kwargs)
+
+    monkeypatch.setattr(BD, "figure_from_spec", interrupting)
+    os.remove("./FAST_calculated_extrema.json")
+    with pytest.raises(KeyboardInterrupt):
+        _run_driver(output_base="./cut/", progress_json_path="./cut.json", flush_batch_size=1)
+    monkeypatch.setattr(BD, "figure_from_spec", real)
+    last = json.load(open("./cut.json")).get("linear_log_last_orbit") if os.path.exists("./cut.json") else None
+    for name in gold["batch_pngs"]:
+        if last is not None and int(name.split("/")[2]) <= last:
+            assert os.path.exists(os.path.join("./cut", name)), name
+    if os.path.exists("./FAST_calculated_extrema.json"):  # each run computes its own extrema
+        os.remove("./FAST_calculated_extrema.json")
+    res = _run_driver(output_base="./again/", progress_json_path="./again.json")
+    assert sorted((r["orbit"], r["status"]) for r in res) == [tuple(x) for x in gold["batch_status"]]
+    assert _png_tree("./again") == _png_tree("./full") == gold["batch_pngs"]
+    for name in gold["batch_pngs"]:
+        a = png.decode_rgba(open(os.path.join("./again", name), "rb").read())
+        assert np.array_equal(a, png.decode_rgba(open(os.path.join("./full", name), "rb").read())), name
+
+
 def test_directory_driver_timeouts_and_retry(tmp_path, monkeypatch):
     """Soft timeouts after the fact + one retry (reference batch_directory.py:316-324,422-431,455-514)."""
     _write_tree(tmp_path)

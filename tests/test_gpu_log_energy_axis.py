@@ -90,7 +90,7 @@ def _figures(ctx):
     return d_rgba, host_figs, dev_figs
 
 
-def test_device_png_matches_host_compose_on_log_axes(ctx, tmp_path):
+def test_device_png_and_deferred_files_match_host_compose_on_log_axes(ctx, tmp_path):
     from PIL import Image
 
     from configurable_spectrograms_b200 import png
@@ -110,8 +110,7 @@ def test_device_png_matches_host_compose_on_log_axes(ctx, tmp_path):
     # of several groups
     paths = [str(tmp_path / f"f{k}.png") for k in range(len(dev_figs))]
     for budget in (160_000, 700):
-        handle = png.encode_figures_device(ctx, d_rgba.ptr, dev_figs, dpi=100, max_segments=budget, paths=paths, wait=False,
-                                           defer=True)
+        handle = png.encode_figures_device(ctx, d_rgba.ptr, dev_figs, dpi=100, max_segments=budget, paths=paths, defer=True)
         for fut in handle.complete():
             fut.result()
         for path, fig in zip(paths, host_figs):
@@ -119,7 +118,7 @@ def test_device_png_matches_host_compose_on_log_axes(ctx, tmp_path):
             os.remove(path)
 
 
-def test_tile_with_row_map_flag_and_no_map_table_raises(ctx, tmp_path, monkeypatch):
+def test_row_map_tile_without_map_table_raises(ctx, tmp_path, monkeypatch):
     """A TILE_ROW_MAP tile with a NULL ``d_row_maps`` is reported by the kernel; no file is written, and the
     context encodes again afterwards."""
     from configurable_spectrograms_b200 import png
@@ -128,9 +127,9 @@ def test_tile_with_row_map_flag_and_no_map_table_raises(ctx, tmp_path, monkeypat
     tables = png._device_tables
 
     def without_maps(figures, dpi):
-        canvases, tiles, rows, row_maps, per_figure = tables(figures, dpi)
-        assert row_maps is not None
-        return canvases, tiles, rows, None, per_figure
+        full = tables(figures, dpi)
+        assert full.row_maps is not None
+        return full._replace(row_maps=None)
 
     monkeypatch.setattr(png, "_device_tables", without_maps)
     path = str(tmp_path / "f.png")

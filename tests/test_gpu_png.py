@@ -57,7 +57,7 @@ def _twin_figures(rng, flat, specs, grid, lines):
     return figs
 
 
-def test_device_png_matches_host_compose(ctx):
+def test_device_png_and_deferred_files_match_host_compose(ctx):
     from configurable_spectrograms_b200 import png
 
     rng = np.random.default_rng(12)
@@ -119,7 +119,7 @@ def test_device_png_matches_host_compose(ctx):
     with tempfile.TemporaryDirectory() as tmp:
         paths = [f"{tmp}/f{k}.png" for k in range(len(dev_figs))]
         for budget in (160_000, 700):  # everything deferred / only the last of several groups
-            handle = png.encode_figures_device(ctx, d_rgba.ptr, dev_figs, dpi=100, max_segments=budget, paths=paths, wait=False, defer=True)
+            handle = png.encode_figures_device(ctx, d_rgba.ptr, dev_figs, dpi=100, max_segments=budget, paths=paths, defer=True)
             with pytest.raises(RuntimeError, match="deferred encode is still open"):
                 png.encode_figures_device(ctx, d_rgba.ptr, dev_figs[:1], dpi=100)
             for fut in handle.complete():
@@ -128,7 +128,7 @@ def test_device_png_matches_host_compose(ctx):
             for path, fig in zip(paths, host_figs):
                 assert np.array_equal(png.decode_rgba(open(path, "rb").read()), fig.compose(100))
                 os.remove(path)
-        handle = png.encode_figures_device(ctx, d_rgba.ptr, dev_figs, dpi=100, paths=paths, wait=False, defer=True)
+        handle = png.encode_figures_device(ctx, d_rgba.ptr, dev_figs, dpi=100, paths=paths, defer=True)
         handle.abandon()
         assert handle.complete() == [] and not any(os.path.exists(p) for p in paths)
         blobs = png.encode_figures_device(ctx, d_rgba.ptr, dev_figs, dpi=100)  # the context is free again

@@ -10,7 +10,7 @@ import numpy as np
 import pytest
 
 
-def test_png_round_trip(tmp_path):
+def test_png_round_trip_through_written_files(tmp_path):
     from configurable_spectrograms_b200 import png
 
     rng = np.random.default_rng(0)
@@ -18,7 +18,8 @@ def test_png_round_trip(tmp_path):
     data = png.encode_rgba(img)
     assert data[:8] == b"\x89PNG\r\n\x1a\n"
     assert np.array_equal(png.decode_rgba(data), img)
-    png.write_many([(tmp_path / f"{i}.png", img[i:]) for i in range(3)], max_workers=2)
+    for i in (0, 2):
+        png.write_rgba(tmp_path / f"{i}.png", img[i:])
     assert np.array_equal(png.decode_rgba((tmp_path / "2.png").read_bytes()), img[2:])
     from PIL import Image  # an independent decoder agrees
 
@@ -163,7 +164,7 @@ def test_figure_layout_serves_host_and_device_rasters():
     assert rows[0] == 0 and np.all(np.diff(rows) > 0) and rows[-1] < t0.H
 
 
-def test_png_assembly_splices_repeated_lines():
+def test_png_assembly_and_native_writer_splice_repeated_lines():
     """``png.assemble_png``: content scanlines come as byte-aligned DEFLATE pieces (here from zlib, standing in
     for the device's segments), the runs of repeated lines in between are ``png.zero_run`` constants; the file
     decodes (own decoder and Pillow: Adler-32 and CRC verified) to the composed image."""
@@ -217,17 +218,20 @@ def test_png_assembly_splices_repeated_lines():
     sizes = np.array([len(x) for x in segs] * 2)
     offsets2 = np.concatenate([[0], np.cumsum(sizes)])
     rows2 = np.concatenate([rows, rows]).astype(np.int32)
-    group = [[W, H, 0, 0, 0, 0, per_row, 0], [W, H, 0, 0, 0, len(segs), per_row, len(rows)]]
-    jobs = [(W, H, rows), (W, H, rows)]
+    canvases = np.zeros(2, dtype=_lib.PNG_CANVAS)
+    canvases["W"], canvases["H"], canvases["segs_per_row"] = W, H, per_row
+    canvases["seg_first"], canvases["row_first"] = (0, len(segs)), (0, len(rows))
+    n_rows = [len(rows), len(rows)]
     with tempfile.TemporaryDirectory() as tmp:
         paths = [os.path.join(tmp, "a.png"), os.path.join(tmp, "b \u00e9.png")]
-        png.write_files_native(lib, paths, group, jobs, rows2, packed2, offsets2, adler2, n_threads=2)
+        png.write_files_native(lib, paths, canvases, n_rows, rows2, packed2, offsets2, adler2, n_threads=2)
         for path in paths:
             data = open(path, "rb").read()
             assert np.array_equal(png.decode_rgba(data), img)
             assert np.array_equal(np.asarray(Image.open(io.BytesIO(data)).convert("RGBA")), img)
         with pytest.raises(OSError, match="not written"):
-            png.write_files_native(lib, [os.path.join(tmp, "missing_dir", "c.png"), paths[0]], group, jobs, rows2, packed2, offsets2, adler2)
+            png.write_files_native(lib, [os.path.join(tmp, "missing_dir", "c.png"), paths[0]], canvases, n_rows, rows2, packed2,
+                                   offsets2, adler2)
         assert np.array_equal(png.decode_rgba(open(paths[0], "rb").read()), img)  # the good file of a failing group is still written
 
 
