@@ -30,12 +30,17 @@ def run_batch(
     flush_batch_size: int = 10,
     log_flush_batch_size: int | None = None,
     install_signal_handlers: bool = True,
+    *,
+    _comm=None,
 ) -> list[tuple[Any, str]]:
     """Run ``worker_fn`` over ``items`` on the executor with resumable progress (reference ``:33-178``).
 
     Items already listed under ``completed_items`` are skipped; every finished item is filed
     under ``completed_items`` / ``no_data`` / ``errors`` by its status; the JSON is rewritten
     every ``flush_batch_size`` items and once at the end.  Returns ``[(item, status)]``.
+
+    ``_comm`` (internal; a ``comm.TorchComm`` over the ranks of one job whose executors resolve every
+    item on every rank): every rank reads the progress JSON, and once all have, rank 0 alone writes it.
     """
     previous_sigint = None
     if install_signal_handlers:
@@ -57,6 +62,9 @@ def run_batch(
                         state[key] = loaded[key]
         except (OSError, json.JSONDecodeError) as exc:
             log_error(f"[PROGRESS] Failed to read existing progress JSON '{progress_json_path}': {exc}")
+    writer = _comm is None or _comm.rank == 0
+    if _comm is not None and _comm.size > 1:
+        _comm.barrier()  # rank 0's first (truncating) write comes after every rank's read
     item_list = list(items)
     done = set(state.get("completed_items", []))
     pending = [item for item in item_list if repr(item) not in done]
@@ -66,7 +74,7 @@ def run_batch(
 
     def flush(force: bool = False) -> None:
         nonlocal unwritten
-        if progress_json_path is None or (unwritten == 0 and not force) or (unwritten < flush_batch_size and not force):
+        if progress_json_path is None or not writer or (unwritten == 0 and not force) or (unwritten < flush_batch_size and not force):
             return
         try:
             with open(progress_json_path, "w") as handle:

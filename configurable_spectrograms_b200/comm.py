@@ -10,14 +10,48 @@ from __future__ import annotations
 import numpy as np
 
 
+def rank_world():
+    """``(rank, world size, torch.distributed)`` of this process; ``(0, 1, None)`` outside an initialised job."""
+    try:
+        import torch.distributed as dist
+
+        if dist.is_available() and dist.is_initialized():
+            return dist.get_rank(), dist.get_world_size(), dist
+    except ImportError:
+        pass
+    return 0, 1, None
+
+
+def current_device() -> int:
+    """The calling thread's CUDA device (``torchrun`` workers select theirs with ``torch.cuda.set_device``).
+    Read it on the thread that was called: a new host thread starts on device 0."""
+    try:
+        import torch
+
+        if torch.cuda.is_available():
+            return int(torch.cuda.current_device())
+    except ImportError:
+        pass
+    return 0
+
+
+def block_of(n: int, rank: int, world: int) -> tuple[int, int]:
+    """``[lo, hi)``: the rank's contiguous block of ``n`` ordered items, ``ceil(n / world)`` per rank (ranks past
+    the end get an empty block, ``lo >= hi``)."""
+    per = -(-n // world)
+    return rank * per, min(n, (rank + 1) * per)
+
+
 class TorchComm:
-    def __init__(self, dist, device=None):
+    def __init__(self, dist, device=None, group=None):
+        """``group``: the process group the collectives run in (``None``: the default group)."""
         import torch
 
         self.torch = torch
         self.dist = dist
-        self.rank = dist.get_rank()
-        self.size = dist.get_world_size()
+        self.group = group
+        self.rank = dist.get_rank(group)
+        self.size = dist.get_world_size(group)
         self.device = device if device is not None else torch.device("cpu")
 
     def allgather(self, arr: np.ndarray) -> list[np.ndarray]:
@@ -27,16 +61,16 @@ class TorchComm:
         view = arr.view(np.uint8).reshape(-1)
         t = torch.from_numpy(view.copy()).to(self.device)
         outs = [torch.empty_like(t) for _ in range(self.size)]
-        self.dist.all_gather(outs, t)
+        self.dist.all_gather(outs, t, group=self.group)
         return [o.cpu().numpy().view(arr.dtype).reshape(arr.shape) for o in outs]
 
     def allgather_object(self, obj):
         outs = [None] * self.size
-        self.dist.all_gather_object(outs, obj)
+        self.dist.all_gather_object(outs, obj, group=self.group)
         return outs
 
     def barrier(self):
-        self.dist.barrier()
+        self.dist.barrier(group=self.group)
 
     # ---- device-pointer collectives (NCCL): the payload never leaves HBM, nothing blocks the host
     def _tensor(self, ptr: int, nbytes: int):
@@ -70,10 +104,10 @@ class TorchComm:
         """dst[rank][nbytes] <- every rank's src[nbytes], enqueued behind the context stream's work."""
         dst, src = self._tensor(dst_ptr, nbytes * self.size), self._tensor(src_ptr, nbytes)
         if stream_handle is None:
-            self.dist.all_gather_into_tensor(dst, src)
+            self.dist.all_gather_into_tensor(dst, src, group=self.group)
             return
         with self._on(stream_handle):
-            self.dist.all_gather_into_tensor(dst, src)
+            self.dist.all_gather_into_tensor(dst, src, group=self.group)
 
     def allreduce_max_dev(self, ptr: int, count: int, kind: str, stream_handle: int | None = 0):
         key = (ptr, count, kind)
@@ -84,10 +118,10 @@ class TorchComm:
             dt = {"i8": torch.int64, "f8": torch.float64, "i4": torch.int32}[kind]
             t = cache[key] = self._tensor(ptr, count * dt.itemsize).view(dt)
         if stream_handle is None:
-            self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX)
+            self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX, group=self.group)
             return
         with self._on(stream_handle):
-            self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX)
+            self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX, group=self.group)
 
 
 # ----------------------------------------------------------------------------------------

@@ -25,11 +25,10 @@ from concurrent.futures import ThreadPoolExecutor
 from dataclasses import dataclass
 from typing import Any
 
-import numpy as np
-
 from .. import _lib
 from ..cdf_utils import get_cdf_file_type, get_timestamps_for_orbit, load_fast_cdf_dataset, load_filtered_orbits
 from ..colormaps import get_lut
+from ..comm import block_of, current_device, rank_world
 from ..constants import DEFAULT_ZOOM_WINDOW_MINUTES
 from ..figure import close_all_axes_and_clear
 from ..logging_utils import configure_log_batch, flush_log_buffer, log_exception
@@ -43,17 +42,6 @@ from .process_orbit import SAVE_DPI, figure_filename
 _INSTRUMENT_KEYS = DEFAULT_INSTRUMENT_ORDER
 
 __all__ = ["FAST_plot_spectrograms_directory"]
-
-
-def _rank_world():
-    try:
-        import torch.distributed as dist
-
-        if dist.is_available() and dist.is_initialized():
-            return dist.get_rank(), dist.get_world_size(), dist
-    except ImportError:
-        pass
-    return 0, 1, None
 
 
 def FAST_plot_spectrograms_directory(
@@ -196,7 +184,7 @@ def _run_directory(directory_path, output_base, y_scale, z_scale, zoom_duration_
         return _time.perf_counter()
 
     t_phase = _time.perf_counter()
-    rank, world, dist = _rank_world()
+    rank, world, dist = rank_world()
     frame = load_filtered_orbits()
     configure_log_batch(log_flush_batch_size or flush_batch_size)
 
@@ -233,8 +221,7 @@ def _run_directory(directory_path, output_base, y_scale, z_scale, zoom_duration_
     n_threads = max(1, int(max_workers))
 
     # ---- this rank's contiguous block of the ascending orbit sequence
-    per = (total_orbits + world - 1) // world if total_orbits else 0
-    lo, hi = rank * per, min(total_orbits, (rank + 1) * per)
+    lo, hi = block_of(total_orbits, rank, world)
     comm = None
     if world > 1:
         import torch
@@ -251,7 +238,7 @@ def _run_directory(directory_path, output_base, y_scale, z_scale, zoom_duration_
     if need_extrema:
         scan_needs = orbits_the_scan_needs(sequence, instrument_order, y_scale, z_scale, load_extrema_state())
     results: list[dict[str, Any]] = []
-    ctx = _lib.default_context(_current_device())
+    ctx = _lib.default_context(current_device())
     shard = ShardPlan(ctx, y_scale, z_scale, zoom_duration_minutes, instrument_order=instrument_order)
     shard.first_orbit_index = lo
     load_errors: dict[int, list[str]] = {}
@@ -292,18 +279,7 @@ def _run_directory(directory_path, output_base, y_scale, z_scale, zoom_duration_
     t_phase = tick("discover_and_resume", t_phase)
     ingest_orbits(shard, range(len(mine)), load_one, refused, n_threads=n_threads)
     if world > 1:
-        # one pool, one key width: every rank computes in the same dtype.  A rank without orbits of its own
-        # (more GPUs than orbits) adopts its peers'; ranks that read cubes of different float dtypes cannot
-        # share a pool (ShardPlan.add_orbit refuses that within a shard for the same reason)
-        mine_dtype = None if shard._dtype is None else shard._dtype.name
-        seen: list = [None] * world
-        dist.all_gather_object(seen, mine_dtype)
-        kinds = sorted({d for d in seen if d is not None})
-        if len(kinds) > 1:
-            raise TypeError(f"ranks read cubes of different dtypes ({', '.join(kinds)}): one run computes in one dtype")
-        if shard._dtype is None and kinds:
-            shard._dtype = np.dtype(kinds[0])
-            shard._batch = None
+        shard.agree_dtype(dist, world)
     if not mine:  # such a rank still joins the extrema exchange, with empty outputs of K1
         shard.collapse_pending()
     # ranks that loaded only part of the sequence still index it globally
@@ -564,14 +540,3 @@ def _write_json(path, data):
             json.dump(data, f, indent=2)
     except OSError as exc:
         log_exception("[ERROR] Failed to write progress JSON", exc, level="error")
-
-
-def _current_device() -> int:
-    try:
-        import torch
-
-        if torch.cuda.is_available():
-            return int(torch.cuda.current_device())
-    except ImportError:
-        pass
-    return 0

@@ -24,6 +24,7 @@ from typing import Any, NamedTuple
 
 import numpy as np
 
+from ..comm import TorchComm, block_of, current_device, rank_world
 from ..logging_utils import log_exception
 from ..percentile_utils import round_extrema
 from .constants import FAST_EXTREMA_JSON_PATH
@@ -599,6 +600,11 @@ def compute_global_extrema(
     scan needs stream through pinned slots chunk by chunk (``Batch.collapse_pending``), so neither host
     RAM nor HBM holds more than a few chunks of cubes.
 
+    Stand-alone under ``torchrun`` (``torch.distributed`` initialised, several ranks) the ranks share the
+    scan like the directory driver's: each reads the files of its contiguous block of the ascending orbit
+    sequence on its own GPU, and the pooled extrema are exchanged.  Rank 0 reads the cache and hands it to
+    the others, every rank returns the same dict, and rank 0 alone writes the JSON.
+
     ``flush_batch_size`` is accepted for call compatibility: the reference rewrites the JSON every
     ``flush_batch_size`` steps of a pass that takes minutes to hours, so that an interrupted run can resume
     (``:333-344``); here the whole pass is a few kernel launches whose results -- the maxima over EVERY
@@ -609,7 +615,19 @@ def compute_global_extrema(
     from .orbit_discovery import discover_orbit_files
 
     instrument_order = tuple(instrument_order)
-    state = load_extrema_state(extrema_json_path)
+    comm, device = _comm, 0
+    rank, world, dist = rank_world() if _shard is None and _comm is None else (0, 1, None)
+    if world > 1:
+        import torch
+
+        device = current_device()
+        comm = TorchComm(dist, torch.device("cuda", device))
+        # every rank plans the same scan from rank 0's reading, and no rank reads the file rank 0 rewrites
+        box = [load_extrema_state(extrema_json_path) if rank == 0 else None]
+        dist.broadcast_object_list(box, src=0)
+        state = box[0]
+    else:
+        state = load_extrema_state(extrema_json_path)
 
     orbit_files = discover_orbit_files(directory_path, instrument_order)
     orbits = sorted(orbit_files)
@@ -617,7 +635,7 @@ def compute_global_extrema(
     last_key = f"{y_scale}_{z_scale}_last_orbit"
 
     def dump():
-        if _comm is not None and getattr(_comm, "rank", 0) != 0:
+        if comm is not None and getattr(comm, "rank", 0) != 0:
             return  # every rank holds the same state; rank 0 owns the cache file
         payload = state
         if last_key in state:
@@ -636,8 +654,9 @@ def compute_global_extrema(
             from .. import _lib
             from .pipeline import ShardPlan, ingest_orbits
 
-            shard = ShardPlan(_lib.default_context(), y_scale, z_scale, instrument_order=instrument_order)
-            shard.first_orbit_index = 0
+            lo, hi = block_of(len(orbits), rank, world)
+            shard = ShardPlan(_lib.default_context(device), y_scale, z_scale, instrument_order=instrument_order)
+            shard.first_orbit_index = lo
 
             def load_one(oi, alloc):
                 datasets = {}
@@ -654,7 +673,11 @@ def compute_global_extrema(
             def refused(orbit, exc):
                 log_exception(f"[EXTREMA] Ingest failure orbit={orbit}", exc, level="message")
 
-            ingest_orbits(shard, range(len(orbits)), load_one, refused)
+            ingest_orbits(shard, range(lo, hi), load_one, refused)
+            if world > 1:
+                shard.agree_dtype(dist, world)
+                if lo >= hi:  # a rank past the last orbit still joins the exchange, with empty outputs of K1
+                    shard.collapse_pending()
     if shard is None:
         # nothing reaches the scan (everything re-used or complete): only the bookkeeping runs
         totals = {i: sum(1 for _, h in sequence if i in h) for i in instrument_order}
@@ -673,7 +696,7 @@ def compute_global_extrema(
         extrema_from_shard(
             shard, sequence, instrument_order, y_scale, z_scale, state, compute_mins=compute_mins,
             max_percentile=max_percentile, log_floor_cutoff=log_floor_cutoff, log_floor_value=log_floor_value,
-            comm=_comm,
+            comm=comm,
         )
         touched = json.dumps(state, sort_keys=True, default=str) != before
     if touched:

@@ -153,6 +153,23 @@ class ShardPlan:
             entry["files"][inst] = fid
         self.orbits.append(entry)
 
+    def agree_dtype(self, dist, world: int):
+        """Collective (every rank of a multi-rank scan, after its ingest): one pool, one key width, so every
+        rank computes in the same dtype.  A rank that read no cube (more GPUs than orbits, or a block the scan
+        does not need) adopts its peers'; ranks that read cubes of different float dtypes cannot share a pool
+        (:meth:`add_orbit` refuses that within a shard for the same reason)."""
+        mine = self._dtype.name if self.file_meta else None
+        seen: list = [None] * world
+        dist.all_gather_object(seen, mine)
+        kinds = sorted({d for d in seen if d is not None})
+        if len(kinds) > 1:
+            raise TypeError(f"ranks read cubes of different dtypes ({', '.join(kinds)}): one run computes in one dtype")
+        if kinds and self._dtype != np.dtype(kinds[0]):
+            self._dtype = np.dtype(kinds[0])
+            self._batch = None
+            if self.orbits:  # orbits added without files: their (empty) K1 outputs again, in the new batch
+                self.collapse_pending()
+
     def upload(self):
         self.batch.upload_cubes()
 
