@@ -15,8 +15,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 # CSG_LIBRARY: another build of the same ABI (A/B experiments: a kernel variant compiled with a different -D)
 LIB_PATH = os.environ.get("CSG_LIBRARY") or os.path.join(HERE, "libcsgpu.so")
 
-ABI_VERSION = 26
+ABI_VERSION = 27
 F32, F64 = 0, 1
+I8, U8, I16, U16, I32, U32 = 2, 3, 4, 5, 6, 7  # integer cube dtypes: K1 only (float64 sums)
 LAYOUT_TPE, LAYOUT_TEP = 0, 1
 K1_GENERIC, K1_STREAM = 0, 1
 MAX_GROUPS = 7
@@ -288,6 +289,17 @@ def np_dtype_code(dtype) -> int:
     if dt == np.float64:
         return F64
     raise TypeError(f"unsupported cube dtype {dt}: libcsgpu computes in float32 or float64")
+
+
+#: integer cube dtypes K1 reads at their stored width (float64 sums, exact; every later stage computes in float64)
+INT_CUBE_CODES = {np.dtype(np.int8): I8, np.dtype(np.uint8): U8, np.dtype(np.int16): I16, np.dtype(np.uint16): U16,
+                  np.dtype(np.int32): I32, np.dtype(np.uint32): U32}
+
+
+def np_cube_code(dtype) -> int:
+    """``csg_collapse`` dtype code of a cube: float32 / float64, or one of the integer codes."""
+    code = INT_CUBE_CODES.get(np.dtype(dtype))
+    return np_dtype_code(dtype) if code is None else code
 
 
 class DevBuf:

@@ -34,6 +34,9 @@
 //   collapse_tep_rows_kernel (stored (T,E,P) view, no groups, 8 <= P <= 128, P % 8 == 0) two lanes
 //       per (t,e) row own numpy's eight pairwise accumulators; P/8 vector loads in flight.
 //   collapse_tep_kernel      (stored (T,E,P) view, general) rows staged in shared memory.
+//   collapse_int_stream_kernel / collapse_int_tpe_kernel / collapse_int_tep_kernel: the same three
+//       roles for integer cubes (CSG_I8 .. CSG_U32), read at their stored width into integer
+//       accumulators, float64 sums out (see the section "Integer cubes" below).
 #include <string.h>
 
 #include <vector>
@@ -767,6 +770,376 @@ int launch_tep(csg_ctx* ctx, const csg_file_desc* d_files, int n_files, int tota
   return CSG_OK;
 }
 
+// =================================================================================
+// Integer cubes (CSG_I8 .. CSG_U32): numpy sums them in int64 / uint64, and integer addition is
+// associative, so any order gives the same bits -- there is no numpy order to copy.  The kernels
+// read the stored type and accumulate in 32 bits (8- and 16-bit input: |sum| <= 65535 * 32768 < 2^31
+// at the largest P csg_collapse accepts) or 64 bits (32-bit input: |sum| <= 2^32 * 2^15 = 2^47), then
+// write float64 sums -- exact, since every such sum is below 2^53 -- the dtype every later stage
+// reads.  There is no NaN: the row flags of row t are bit 0 and bit 1+k for every group k with a
+// member bin, as the widened float64 path sets them.
+// =================================================================================
+template <typename I>
+struct IntAcc {
+  typedef int32_t A;
+};
+template <>
+struct IntAcc<int32_t> {
+  typedef long long A;
+};
+template <>
+struct IntAcc<uint32_t> {
+  typedef long long A;
+};
+
+// value v of the 16 bytes w of stored integers (v is a constant after unrolling: a shift and a convert)
+template <typename I>
+__device__ __forceinline__ typename IntAcc<I>::A int_elem(const uint4& w, int v) {
+  constexpr int PER = 4 / sizeof(I);
+  const int k = v / PER, j = v % PER;
+  const unsigned word = k == 0 ? w.x : k == 1 ? w.y : k == 2 ? w.z : w.w;
+  return (typename IntAcc<I>::A)(I)(word >> (8 * sizeof(I) * j));
+}
+
+__device__ __forceinline__ uint4 ld_stream_u4(const void* p) {
+  uint4 r;
+  asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];"
+               : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w)
+               : "l"(p));
+  return r;
+}
+
+inline size_t int_itemsize(int dtype) {
+  switch (dtype) {
+    case CSG_I8:
+    case CSG_U8:
+      return 1;
+    case CSG_I16:
+    case CSG_U16:
+      return 2;
+    case CSG_I32:
+    case CSG_U32:
+      return 4;
+  }
+  return 0;
+}
+inline bool is_int_dtype(int dtype) { return int_itemsize(dtype) != 0; }
+inline size_t cube_itemsize(int dtype) { return dtype == CSG_F64 ? 8 : (dtype == CSG_F32 ? 4 : int_itemsize(dtype)); }
+inline size_t sums_itemsize(int dtype) { return dtype == CSG_F32 ? 4 : 8; }
+
+// ---- stream kernel (TPE, 16-byte aligned, E * itemsize a multiple of 16): block = 16 time rows x the
+// EV = E * itemsize / 16 chunks of a row, thread = (row, 16 bytes of consecutive energies).  The pitch
+// axis is walked in the runs of constant group membership of the float stream kernel, eight 128-bit
+// streaming loads in flight per thread.  The transposed tile leaves through shared memory one group at
+// a time (the shared tile is E x 17 doubles whatever the number of groups).
+constexpr int kIntStreamMaxEV = 32;  // blocks of at most 16 x 32 = 512 threads
+
+inline int int_stream_ev(int E, int dtype) {
+  const size_t es = int_itemsize(dtype);
+  if (es == 0 || E <= 0 || (E * es) % 16 != 0) return 0;
+  const int ev = (int)(E * es / 16);
+  return ev <= kIntStreamMaxEV ? ev : 0;
+}
+
+template <typename I, int NG, int MASK>
+__device__ __forceinline__ void int_stream_run(const I* __restrict__ ptr, long long E, int p0, int p1,
+                                               const uint8_t* __restrict__ bits_p, unsigned keep,
+                                               typename IntAcc<I>::A (&acc)[NG + 1][16 / sizeof(I)], unsigned& flag) {
+  using A = typename IntAcc<I>::A;
+  constexpr int V = 16 / sizeof(I);
+  // eight loads in flight; four where the accumulators alone take 64 registers (they would spill)
+  constexpr int U = (NG + 1) * V * sizeof(A) >= 256 ? 4 : 8;
+  auto one = [&](const uint4& w, int p) {
+    const unsigned bits = MASK < 0 ? (__ldg(bits_p + p) & keep) : (unsigned)MASK;
+#pragma unroll
+    for (int v = 0; v < V; ++v) {
+      const A z = int_elem<I>(w, v);
+      acc[0][v] += z;
+#pragma unroll
+      for (int g = 0; g < NG; ++g)
+        if ((bits >> g) & 1u) acc[g + 1][v] += z;
+    }
+    if (MASK < 0) flag |= (bits << 1) | 1u;
+  };
+  int p = p0;
+  for (; p + U <= p1; p += U) {
+    uint4 x[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) x[u] = ld_stream_u4(ptr + (long long)(p + u) * E);
+#pragma unroll
+    for (int u = 0; u < U; ++u) one(x[u], p + u);
+  }
+  for (; p < p1; ++p) one(ld_stream_u4(ptr + (long long)p * E), p);
+  if (MASK >= 0 && p1 > p0) flag |= ((unsigned)MASK << 1) | 1u;
+}
+
+template <typename I, int NG>
+__global__ void __launch_bounds__(kTileRows* kIntStreamMaxEV, 1)
+    collapse_int_stream_kernel(const csg_file_desc* __restrict__ files, int n_files, const int32_t* __restrict__ runs,
+                               const uint8_t* __restrict__ pa_bits, int n_groups, double* __restrict__ sums,
+                               uint8_t* __restrict__ row_flags) {
+  using A = typename IntAcc<I>::A;
+  constexpr int V = 16 / sizeof(I);
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  double* s_out = reinterpret_cast<double*>(smem_raw);  // [E][kOutPitch], one group at a time
+
+  const int fi = find_file(files, n_files, blockIdx.x);
+  const csg_file_desc f = files[fi];
+  const int EV = blockDim.x / kTileRows;  // every file of the launch has E = EV * V
+  const int E = EV * V;
+  const int t0 = (blockIdx.x - f.first_block) * kTileRows;
+  const int rows_here = min(kTileRows, f.T - t0);
+  const int r = threadIdx.x / EV, c = threadIdx.x - r * EV;
+
+  const unsigned alias = (unsigned)f.reserved[2];  // groups holding every pitch bin
+  A acc[NG + 1][V];
+#pragma unroll
+  for (int g = 0; g <= NG; ++g)
+#pragma unroll
+    for (int v = 0; v < V; ++v) acc[g][v] = A(0);
+  unsigned flag = 0;
+  if (r < rows_here) {
+    const I* ptr = static_cast<const I*>(f.d_cube) + ((long long)(t0 + r) * f.P) * E + c * V;
+    const int32_t* run = runs + 3 * (long long)f.reserved[0];
+    const int n_runs = f.reserved[1];
+    const uint8_t* bits_p = pa_bits + f.bits_off;
+    for (int k = 0; k < n_runs; ++k) {
+      const int p0 = __ldg(run + 3 * k), p1 = __ldg(run + 3 * k + 1), mask = __ldg(run + 3 * k + 2);
+      if (NG == 4) {
+        switch (mask & 15) {
+#define CSG_RUN(M)                                                             \
+  case M:                                                                      \
+    int_stream_run<I, NG, M>(ptr, E, p0, p1, bits_p, ~alias, acc, flag); \
+    break;
+          CSG_RUN(0)
+          CSG_RUN(1)
+          CSG_RUN(2)
+          CSG_RUN(3)
+          CSG_RUN(4)
+          CSG_RUN(5)
+          CSG_RUN(6)
+          CSG_RUN(7)
+          CSG_RUN(8)
+          CSG_RUN(9)
+          CSG_RUN(10)
+          CSG_RUN(11)
+          CSG_RUN(12)
+          CSG_RUN(13)
+          CSG_RUN(14)
+          CSG_RUN(15)
+#undef CSG_RUN
+        }
+      } else if (NG == 0) {
+        int_stream_run<I, NG, 0>(ptr, E, p0, p1, bits_p, ~alias, acc, flag);
+      } else {
+        int_stream_run<I, NG, -1>(ptr, E, p0, p1, bits_p, ~alias, acc, flag);
+      }
+    }
+    if (flag & 1u) flag |= alias << 1;
+  }
+  // every thread of a row walked every pitch bin: its flag is the row's
+  if (row_flags != nullptr && r < rows_here && c == 0) row_flags[f.flags_off + t0 + r] = (uint8_t)flag;
+
+  const int Tp = pitch_of(f.T);
+  const long long plane = (long long)E * Tp;
+  double* out = sums + f.sums_off + t0;
+  const int rr = threadIdx.x & (kTileRows - 1);
+  const int step = blockDim.x / kTileRows;
+#pragma unroll
+  for (int g = 0; g <= NG; ++g) {
+    if (g > n_groups) break;
+    if (g > 0) __syncthreads();  // the previous group's tile has left
+    if (r < rows_here) {
+      const bool copy = g > 0 && ((alias >> (g - 1)) & 1u);
+#pragma unroll
+      for (int v = 0; v < V; ++v) s_out[(c * V + v) * kOutPitch + r] = (double)(copy ? acc[0][v] : acc[g][v]);
+    }
+    __syncthreads();
+    if (rr < rows_here)
+      for (int e = threadIdx.x / kTileRows; e < E; e += step) out[g * plane + (long long)e * Tp + rr] = s_out[e * kOutPitch + rr];
+  }
+}
+
+// ---- generic (TPE, any E or alignment): thread = one (t, e) cell column, consecutive threads read
+// consecutive energies of a (t, p) row.
+template <typename I, int NG>
+__global__ void __launch_bounds__(kBlock)
+    collapse_int_tpe_kernel(const csg_file_desc* __restrict__ files, int n_files, const uint8_t* __restrict__ pa_bits,
+                            int n_groups, double* __restrict__ sums, uint8_t* __restrict__ row_flags) {
+  using A = typename IntAcc<I>::A;
+  extern __shared__ unsigned char smem_raw[];
+  uint8_t* s_bits = smem_raw;  // [P]
+  const int fi = find_file(files, n_files, blockIdx.x);
+  const csg_file_desc f = files[fi];
+  const int P = f.P, E = f.E;
+  const long long item = (long long)(blockIdx.x - f.first_block) * kBlock + threadIdx.x;
+  for (int p = threadIdx.x; p < P; p += kBlock) s_bits[p] = NG ? pa_bits[f.bits_off + p] : 0;
+  __syncthreads();
+  if (item >= (long long)f.T * E) return;
+  const int t = (int)(item / E), e = (int)(item - (long long)t * E);
+  const I* ptr = static_cast<const I*>(f.d_cube) + (long long)t * P * E + e;
+  A acc[NG + 1];
+#pragma unroll
+  for (int g = 0; g <= NG; ++g) acc[g] = A(0);
+  unsigned flag = 0;
+  auto one = [&](I x, int p) {
+    const unsigned bits = s_bits[p];
+    const A z = (A)x;
+    acc[0] += z;
+#pragma unroll
+    for (int g = 0; g < NG; ++g)
+      if ((bits >> g) & 1u) acc[g + 1] += z;
+    flag |= (bits << 1) | 1u;
+  };
+  constexpr int U = 8;
+  int p = 0;
+  for (; p + U <= P; p += U) {
+    I x[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) x[u] = __ldg(ptr + (long long)(p + u) * E);
+#pragma unroll
+    for (int u = 0; u < U; ++u) one(x[u], p + u);
+  }
+  for (; p < P; ++p) one(__ldg(ptr + (long long)p * E), p);
+  const int Tp = pitch_of(f.T);
+  const long long plane = (long long)E * Tp;
+  double* out = sums + f.sums_off + (long long)e * Tp + t;
+#pragma unroll
+  for (int g = 0; g <= NG; ++g)
+    if (g <= n_groups) out[g * plane] = (double)acc[g];
+  if (row_flags != nullptr && e == 0) row_flags[f.flags_off + t] = (uint8_t)flag;  // the same for every e
+}
+
+// ---- stored (T,E,P) view: rows of P contiguous pitch samples, L = int_tep_lanes(P) lanes per (t, e)
+// row (about four samples a lane for short rows), consecutive lanes read consecutive samples; the
+// lanes' partial sums meet through shuffles.  Any P, any alignment, any number of groups.
+__host__ __device__ inline int int_tep_lanes(int P) {
+  return P >= 128 ? 32 : P >= 64 ? 16 : P >= 32 ? 8 : P >= 16 ? 4 : P >= 8 ? 2 : 1;
+}
+
+template <typename I, int NG>
+__global__ void __launch_bounds__(kBlock)
+    collapse_int_tep_kernel(const csg_file_desc* __restrict__ files, int n_files, const uint8_t* __restrict__ pa_bits,
+                            int n_groups, double* __restrict__ sums, uint8_t* __restrict__ row_flags) {
+  using A = typename IntAcc<I>::A;
+  extern __shared__ unsigned char smem_raw[];
+  uint8_t* s_bits = smem_raw;  // [P]
+  const int fi = find_file(files, n_files, blockIdx.x);
+  const csg_file_desc f = files[fi];
+  const int P = f.P, E = f.E;
+  const int L = int_tep_lanes(P);
+  const long long row = (long long)(blockIdx.x - f.first_block) * (kBlock / L) + threadIdx.x / L;
+  const int h = threadIdx.x & (L - 1);
+  for (int p = threadIdx.x; p < P; p += kBlock) s_bits[p] = NG ? pa_bits[f.bits_off + p] : 0;
+  __syncthreads();
+  const bool in = row < (long long)f.T * E;
+  A acc[NG + 1];
+#pragma unroll
+  for (int g = 0; g <= NG; ++g) acc[g] = A(0);
+  unsigned flag = 0;
+  if (in) {
+    const I* q = static_cast<const I*>(f.d_cube) + row * P;
+    for (int p = h; p < P; p += L) {
+      const unsigned bits = s_bits[p];
+      const A z = (A)__ldg(q + p);
+      acc[0] += z;
+#pragma unroll
+      for (int g = 0; g < NG; ++g)
+        if ((bits >> g) & 1u) acc[g + 1] += z;
+      flag |= (bits << 1) | 1u;
+    }
+  }
+  for (int o = 1; o < L; o <<= 1) {  // L is uniform in the block: every lane of the warp takes part
+#pragma unroll
+    for (int g = 0; g <= NG; ++g) acc[g] += __shfl_xor_sync(0xffffffffu, acc[g], o);
+    flag |= __shfl_xor_sync(0xffffffffu, flag, o);
+  }
+  if (!in || h != 0) return;
+  const int t = (int)(row / E), e = (int)(row - (long long)t * E);
+  const int Tp = pitch_of(f.T);
+  const long long plane = (long long)E * Tp;
+  double* out = sums + f.sums_off + (long long)e * Tp + t;
+#pragma unroll
+  for (int g = 0; g <= NG; ++g)
+    if (g <= n_groups) out[g * plane] = (double)acc[g];
+  if (row_flags != nullptr && e == 0) row_flags[f.flags_off + t] = (uint8_t)flag;  // the same for every e
+}
+
+// 8-bit input with more than 4 groups would keep 8 x 16 accumulators per thread: the generic kernel
+inline bool int_stream_file_ok(int32_t T, int32_t P, int32_t E, int dtype, const void* d_cube, int n_groups) {
+  if (int_itemsize(dtype) == 1 && n_groups > 4) return false;
+  return T > 0 && P > 0 && int_stream_ev(E, dtype) > 0 && (reinterpret_cast<uintptr_t>(d_cube) & 15) == 0;
+}
+
+template <typename I>
+int launch_int(csg_ctx* ctx, int layout, int kernel, const csg_file_desc* d_files, int n_files, int total_blocks,
+               const uint8_t* d_pa_bits, const int32_t* d_runs, int n_groups, int max_P, int max_E, int dtype,
+               double* d_sums, uint8_t* d_row_flags) {
+  auto go = [&](auto kern, int threads, size_t smem) -> int {
+    if (smem > 48 * 1024) CSG_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<total_blocks, threads, smem, ctx->stream>>>(d_files, n_files, d_pa_bits, n_groups, d_sums, d_row_flags);
+    return CSG_OK;
+  };
+  auto by_groups = [&](auto k0, auto k4, auto k7, int threads, size_t smem) -> int {
+    return n_groups == 0 ? go(k0, threads, smem) : n_groups <= 4 ? go(k4, threads, smem) : go(k7, threads, smem);
+  };
+  int st;
+  if (layout == CSG_LAYOUT_TEP) {
+    st = by_groups(collapse_int_tep_kernel<I, 0>, collapse_int_tep_kernel<I, 4>, collapse_int_tep_kernel<I, CSG_MAX_GROUPS>,
+                   kBlock, (size_t)max_P);
+    if (st != CSG_OK) return st;
+    CSG_LAUNCH_CHECK(ctx, "collapse_int_tep_kernel");
+    return CSG_OK;
+  }
+  if (kernel != CSG_K1_STREAM) {
+    st = by_groups(collapse_int_tpe_kernel<I, 0>, collapse_int_tpe_kernel<I, 4>, collapse_int_tpe_kernel<I, CSG_MAX_GROUPS>,
+                   kBlock, (size_t)max_P);
+    if (st != CSG_OK) return st;
+    CSG_LAUNCH_CHECK(ctx, "collapse_int_tpe_kernel");
+    return CSG_OK;
+  }
+  const int ev = int_stream_ev(max_E, dtype);
+  if (ev == 0)
+    return csg_fail(ctx, CSG_ERR_ARG, "integer stream kernel cannot handle E=%d: use CSG_K1_GENERIC for this table", max_E);
+  if (!d_runs) return csg_fail(ctx, CSG_ERR_ARG, "d_runs is NULL for the stream kernel");
+  const int threads = kTileRows * ev;
+  const size_t smem = (size_t)max_E * kOutPitch * sizeof(double);
+  auto stream = [&](auto kern) -> int {
+    if (smem > 48 * 1024) CSG_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<total_blocks, threads, smem, ctx->stream>>>(d_files, n_files, d_runs, d_pa_bits, n_groups, d_sums, d_row_flags);
+    return CSG_OK;
+  };
+  if constexpr (sizeof(I) == 1) {
+    if (n_groups > 4) return csg_fail(ctx, CSG_ERR_ARG, "8-bit cubes with more than 4 groups take CSG_K1_GENERIC");
+    st = n_groups == 0 ? stream(collapse_int_stream_kernel<I, 0>) : stream(collapse_int_stream_kernel<I, 4>);
+  } else {
+    st = n_groups == 0   ? stream(collapse_int_stream_kernel<I, 0>)
+         : n_groups <= 4 ? stream(collapse_int_stream_kernel<I, 4>)
+                         : stream(collapse_int_stream_kernel<I, CSG_MAX_GROUPS>);
+  }
+  if (st != CSG_OK) return st;
+  CSG_LAUNCH_CHECK(ctx, "collapse_int_stream_kernel");
+  return CSG_OK;
+}
+
+int launch_int_dtype(csg_ctx* ctx, int dtype, int layout, int kernel, const csg_file_desc* d_files, int n_files,
+                     int total_blocks, const uint8_t* d_pa_bits, const int32_t* d_runs, int n_groups, int max_P, int max_E,
+                     double* d_sums, uint8_t* d_row_flags) {
+#define CSG_INT(CODE, TYPE) \
+  case CODE:                \
+    return launch_int<TYPE>(ctx, layout, kernel, d_files, n_files, total_blocks, d_pa_bits, d_runs, n_groups, max_P, max_E, dtype, d_sums, d_row_flags);
+  switch (dtype) {
+    CSG_INT(CSG_I8, int8_t)
+    CSG_INT(CSG_U8, uint8_t)
+    CSG_INT(CSG_I16, int16_t)
+    CSG_INT(CSG_U16, uint16_t)
+    CSG_INT(CSG_I32, int32_t)
+    CSG_INT(CSG_U32, uint32_t)
+  }
+#undef CSG_INT
+  return csg_fail(ctx, CSG_ERR_ARG, "bad dtype %d", dtype);
+}
+
 }  // namespace
 
 extern "C" {
@@ -776,6 +1149,8 @@ int csg_collapse_kernel(int32_t T, int32_t P, int32_t E, int dtype, int layout, 
 }
 
 int csg_collapse_kernel_for(int32_t T, int32_t P, int32_t E, int dtype, int layout, const void* d_cube, int n_groups) {
+  if (is_int_dtype(dtype))  // stored (T,E,P) integer views always take the row kernel
+    return layout == CSG_LAYOUT_TEP || int_stream_file_ok(T, P, E, dtype, d_cube, n_groups) ? CSG_K1_STREAM : CSG_K1_GENERIC;
   if (layout == CSG_LAYOUT_TEP) return tep_rows_ok(T, P, E, d_cube, n_groups) ? CSG_K1_STREAM : CSG_K1_GENERIC;
   return stream_file_ok(T, P, E, dtype, d_cube) ? CSG_K1_STREAM : CSG_K1_GENERIC;
 }
@@ -798,6 +1173,14 @@ int csg_pitch_runs(const uint8_t* h_pa_bits, int P, int n_groups, int32_t* h_run
 
 int32_t csg_collapse_blocks(int32_t T, int32_t P, int32_t E, int dtype, int layout, int kernel) {
   if (T <= 0 || E <= 0) return 0;
+  if (is_int_dtype(dtype)) {
+    if (layout == CSG_LAYOUT_TEP) {
+      const int rows = kBlock / int_tep_lanes(P);
+      return (int32_t)(((long long)T * E + rows - 1) / rows);
+    }
+    if (kernel == CSG_K1_STREAM) return (T + kTileRows - 1) / kTileRows;
+    return (int32_t)(((long long)T * E + kBlock - 1) / kBlock);
+  }
   if (layout == CSG_LAYOUT_TEP) {
     if (kernel == CSG_K1_STREAM) return (T + kTepTile - 1) / kTepTile;
     const int rows = tep_rows_per_block(P, dtype);
@@ -820,11 +1203,14 @@ int csg_collapse(csg_ctx* ctx, const csg_file_desc* d_files, int n_files, int to
   if (!ctx) return CSG_ERR_ARG;
   if (n_groups < 0 || n_groups > CSG_MAX_GROUPS) return csg_fail(ctx, CSG_ERR_ARG, "n_groups %d out of range", n_groups);
   if (n_groups > 0 && !d_pa_bits) return csg_fail(ctx, CSG_ERR_ARG, "d_pa_bits is NULL with n_groups > 0");
-  if (dtype != CSG_F32 && dtype != CSG_F64) return csg_fail(ctx, CSG_ERR_ARG, "bad dtype %d", dtype);
+  if (dtype != CSG_F32 && dtype != CSG_F64 && !is_int_dtype(dtype)) return csg_fail(ctx, CSG_ERR_ARG, "bad dtype %d", dtype);
   if (layout != CSG_LAYOUT_TPE && layout != CSG_LAYOUT_TEP) return csg_fail(ctx, CSG_ERR_ARG, "bad layout %d", layout);
   if (n_files <= 0 || total_blocks <= 0) return CSG_OK;
   if (!d_files || !d_sums) return csg_fail(ctx, CSG_ERR_ARG, "NULL table or output");
   if (max_P <= 0 || max_P > 32768) return csg_fail(ctx, CSG_ERR_ARG, "max_P %d out of range (1..32768)", max_P);
+  if (is_int_dtype(dtype))
+    return launch_int_dtype(ctx, dtype, layout, kernel, d_files, n_files, total_blocks, d_pa_bits, d_runs, n_groups, max_P,
+                            max_E, (double*)d_sums, d_row_flags);
   if (layout == CSG_LAYOUT_TPE) {
     if (kernel == CSG_K1_STREAM) {
       if (!d_runs) return csg_fail(ctx, CSG_ERR_ARG, "d_runs is NULL for the stream kernel");
@@ -872,10 +1258,10 @@ int csg_collapse_host(csg_ctx* ctx, const void* h_cube, int32_t T, int32_t P, in
                       const uint8_t* h_pa_bits, int n_groups, void* h_sums, uint8_t* h_row_flags) {
   if (!ctx) return CSG_ERR_ARG;
   if (T < 0 || P <= 0 || E <= 0) return csg_fail(ctx, CSG_ERR_ARG, "bad cube shape (%d,%d,%d)", T, P, E);
-  if (dtype != CSG_F32 && dtype != CSG_F64) return csg_fail(ctx, CSG_ERR_ARG, "bad dtype %d", dtype);
+  if (dtype != CSG_F32 && dtype != CSG_F64 && !is_int_dtype(dtype)) return csg_fail(ctx, CSG_ERR_ARG, "bad dtype %d", dtype);
   if (T == 0) return CSG_OK;
-  const size_t es = dtype == CSG_F64 ? 8 : 4;
-  const size_t cube_bytes = (size_t)T * P * E * es;
+  const size_t es = sums_itemsize(dtype);  // an integer cube's sums are float64
+  const size_t cube_bytes = (size_t)T * P * E * cube_itemsize(dtype);
   const int Tp = (T + 3) & ~3;
   const size_t sums_bytes = (size_t)csg_sums_elems(T, E, n_groups) * es;
   const size_t flag_bytes = ((size_t)T + 3) & ~size_t(3);
@@ -906,7 +1292,7 @@ int csg_collapse_host(csg_ctx* ctx, const void* h_cube, int32_t T, int32_t P, in
   desc.reserved[1] = csg_pitch_runs(h_pa_bits, P, n_groups, h_runs.data(), &alias);
   desc.reserved[2] = alias;
   CSG_TRY(csg_h2d(ctx, d_runs, h_runs.data(), h_runs.size() * sizeof(int32_t)));
-  const int kernel = csg_collapse_kernel(T, P, E, dtype, layout, d_cube);
+  const int kernel = csg_collapse_kernel_for(T, P, E, dtype, layout, d_cube, is_int_dtype(dtype) ? n_groups : 1);
   const int blocks = csg_collapse_blocks(T, P, E, dtype, layout, kernel);
   CSG_TRY(csg_h2d(ctx, d_cube, h_cube, cube_bytes));
   CSG_TRY(csg_h2d(ctx, d_desc, &desc, sizeof(desc)));

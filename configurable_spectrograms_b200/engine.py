@@ -6,7 +6,8 @@ reference-shaped host functions (``plotting.make_spectrogram`` ...) build batche
 one file; the FAST batch driver builds one batch per GPU shard.
 
 Data layout in HBM (DESIGN.md section 3):
-  cubes   one allocation, each file 256-byte aligned, dtype D
+  cubes   one allocation, each file 256-byte aligned, in its stored dtype (D, or an 8/16/32-bit
+          integer type when D is float64)
   sums    per file [(G+1)][E][Tp] dtype D, energy-major (group 0 = every pitch bin; Tp = T
           rounded up to a multiple of 4) -- the orientation imshow draws (matrix_plot = collapsed.T)
   flags   per file [T] uint8 (bit g: a non-NaN cell exists in row t of group g)
@@ -32,6 +33,7 @@ from ._lib import (
     Context,
     CsgError,
     DevBuf,
+    np_cube_code,
     np_dtype_code,
 )
 
@@ -50,6 +52,13 @@ _WANT_RANK = {WANT_GEOMETRY: 0, WANT_REDUCTIONS: 1, WANT_PERCENTILES: 2}
 
 def _align(n: int, a: int = 256) -> int:
     return (n + a - 1) // a * a
+
+
+def compute_dtype(cube_dtype) -> np.dtype:
+    """The dtype numpy computes a cube of ``cube_dtype`` in: float32 / float64 stay; integer counts go through
+    float64 (``np.nansum`` sums them exactly in int64 / uint64; ``np.nanpercentile`` and matplotlib work in float64)."""
+    dt = np.dtype(cube_dtype)
+    return dt if dt in (np.float32, np.float64) else np.dtype(np.float64)
 
 
 def classify_cube(cube: np.ndarray):
@@ -97,7 +106,10 @@ class ZSlot(float):
 
 
 class Batch:
-    """Cubes of one dtype on one GPU plus the tables of everything to compute from them."""
+    """Cubes of one compute dtype D on one GPU plus the tables of everything to compute from them.
+
+    A float64 batch also takes 8/16/32-bit integer cubes (``_lib.INT_CUBE_CODES``): K1 reads them at their
+    stored width and writes float64 sums, the same bits as the cube widened to float64."""
 
     def __init__(self, ctx: Context, dtype, n_groups: int = 0):
         if not 0 <= n_groups <= _lib.MAX_GROUPS:
@@ -150,16 +162,22 @@ class Batch:
         self._flags_valid_bytes = 0
 
     # ------------------------------------------------------------------ files
-    def add_file(self, cube: np.ndarray | None, pa_bits: np.ndarray | None = None, *, shape=None, layout=None, device_ptr=None) -> int:
-        """Register one cube (host array, or a device pointer with ``shape``/``layout``)."""
+    def add_file(self, cube: np.ndarray | None, pa_bits: np.ndarray | None = None, *, shape=None, layout=None, device_ptr=None,
+                 cube_dtype=None) -> int:
+        """Register one cube (host array, or a device pointer with ``shape``/``layout`` and ``cube_dtype``, by
+        default the batch dtype)."""
         if cube is not None:
-            if cube.dtype != self.dtype:
+            if cube.dtype != self.dtype and not (self.dtype == np.float64 and cube.dtype in _lib.INT_CUBE_CODES):
                 raise TypeError(f"cube dtype {cube.dtype} != batch dtype {self.dtype}")
             host, layout, (T, P, E) = classify_cube(cube)
+            cube_dtype = cube.dtype
         else:
             host = None
             T, P, E = shape
             layout = _lib.LAYOUT_TPE if layout is None else layout
+            cube_dtype = self.dtype if cube_dtype is None else np.dtype(cube_dtype)
+            if cube_dtype != self.dtype and not (self.dtype == np.float64 and cube_dtype in _lib.INT_CUBE_CODES):
+                raise TypeError(f"cube dtype {cube_dtype} != batch dtype {self.dtype}")
         if self.G > 0:
             if pa_bits is None or len(pa_bits) != P:
                 raise ValueError("pa_bits (uint8[P]) is required when the batch has pitch-angle groups")
@@ -171,6 +189,8 @@ class Batch:
             "P": P,
             "E": E,
             "layout": layout,
+            "dtype": np.dtype(cube_dtype),
+            "code": np_cube_code(cube_dtype),
             "host": host,
             "device_ptr": device_ptr,
             "cube_off": self._cube_bytes,
@@ -179,7 +199,7 @@ class Batch:
             "bits_off": self._bits_len,
         }
         f["Tp"] = (T + 3) // 4 * 4
-        self._cube_bytes += _align(T * P * E * self.dtype.itemsize)
+        self._cube_bytes += _align(T * P * E * f["dtype"].itemsize)
         self._sums_elems += _align((self.G + 1) * E * f["Tp"] * self.dtype.itemsize) // self.dtype.itemsize
         self._flags_bytes += _align(T, 4)
         self._bits.append(bits)
@@ -190,7 +210,7 @@ class Batch:
 
     @property
     def cube_bytes(self) -> int:
-        return sum(f["T"] * f["P"] * f["E"] for f in self.files) * self.dtype.itemsize
+        return sum(f["T"] * f["P"] * f["E"] * f["dtype"].itemsize for f in self.files)
 
     def upload_cubes(self):
         """H2D of every host cube into one device allocation (async on the ctx stream)."""
@@ -215,25 +235,27 @@ class Batch:
         return buf
 
     def _file_tables(self, indices, ptr_of, tag="all"):
-        """Descriptor tables for the files ``indices``: one per (storage layout, K1 kernel, E) -- a launch
-        handles files of one kind.  ``ptr_of(i)``: device address of file i's cube.  Returns
-        ``({key: (table, n, blocks, max_P, max_E)}, d_runs, d_bits)``; the pitch-angle membership bytes
+        """Descriptor tables for the files ``indices``: one per (storage layout, K1 kernel, E) and cube dtype -- a
+        launch handles files of one kind; the key of an integer file's table ends with its cube dtype code.
+        ``ptr_of(i)``: device address of file i's cube.  Returns ``({key: (table, n, blocks, max_P, max_E)}, d_runs,
+        d_bits)``; the pitch-angle membership bytes
         are packed for these files only (``bits_off`` is local to the returned ``d_bits``)."""
         lib = self.ctx.lib
         indices = list(indices)
-        groups: dict[tuple[int, int, int], list[int]] = {}
+        groups: dict[tuple, list[int]] = {}
         for i in indices:
             f = self.files[i]
             if f["T"] <= 0:
                 continue
-            kern = lib.csg_collapse_kernel_for(f["T"], f["P"], f["E"], self.code, f["layout"], ptr_of(i), self.G)
+            kern = lib.csg_collapse_kernel_for(f["T"], f["P"], f["E"], f["code"], f["layout"], ptr_of(i), self.G)
             # every file of a stream-kernel table shares one energy count (it fixes the block shape)
-            groups.setdefault((f["layout"], kern, f["E"] if kern == _lib.K1_STREAM else 0), []).append(i)
+            key = (f["layout"], kern, f["E"] if kern == _lib.K1_STREAM else 0)
+            groups.setdefault(key if f["code"] == self.code else key + (f["code"],), []).append(i)
         # runs of constant pitch-angle group membership (stream kernel), one entry per distinct table
         runs_tab: list[np.ndarray] = []
         runs_len = 0
         runs_of: dict[bytes, tuple[int, int, int]] = {}
-        for (layout, kern, _e), idx in groups.items():
+        for (layout, kern, *_), idx in groups.items():
             if kern != _lib.K1_STREAM:
                 continue
             for i in idx:
@@ -255,7 +277,8 @@ class Batch:
             bits_off[i] = off
             off += len(self._bits[i])
         tables = {}
-        for (layout, kern, _e), idx in groups.items():
+        for key, idx in groups.items():
+            layout, kern, code = key[0], key[1], self._key_code(key)
             tab = np.zeros(len(idx), dtype=FILE_DESC)
             blocks, max_p, max_e = 0, 1, 1
             for j, i in enumerate(idx):
@@ -268,9 +291,9 @@ class Batch:
                 tab[j]["first_block"] = blocks
                 if kern == _lib.K1_STREAM:
                     tab[j]["reserved"] = runs_of[self._bits[i].tobytes()]
-                blocks += lib.csg_collapse_blocks(f["T"], f["P"], f["E"], self.code, layout, kern)
+                blocks += lib.csg_collapse_blocks(f["T"], f["P"], f["E"], code, layout, kern)
                 max_p, max_e = max(max_p, f["P"]), max(max_e, f["E"])
-            tables[(layout, kern, _e)] = (self._table(f"{tag}_files_{layout}_{kern}_{_e}", tab), len(idx), blocks, max_p, max_e)
+            tables[key] = (self._table(f"{tag}_files_" + "_".join(map(str, key)), tab), len(idx), blocks, max_p, max_e)
         packed = [self._bits[i] for i in indices]
         d_bits = self._table(f"{tag}_bits", np.concatenate(packed) if packed else np.zeros(1, np.uint8))
         return tables, d_runs, d_bits
@@ -302,12 +325,16 @@ class Batch:
         self._ensure_outputs_of_k1()
         self._tables_dirty = False
 
+    def _key_code(self, key) -> int:
+        """Cube dtype code of a K1 table key (see :meth:`_file_tables`)."""
+        return key[3] if len(key) > 3 else self.code
+
     def _launch_k1(self, tables, d_runs, d_bits):
-        for (layout, kern, _e), (tab, n, blocks, max_p, max_e) in tables.items():
+        for key, (tab, n, blocks, max_p, max_e) in tables.items():
             self.ctx._check(
                 self.ctx.lib.csg_collapse(
                     self.ctx.handle, tab.ptr, n, blocks, d_bits.ptr, d_runs.ptr if d_runs is not None else None, self.G,
-                    max_p, max_e, self.code, layout, kern, self.d_sums.ptr, self.d_flags.ptr,
+                    max_p, max_e, self._key_code(key), key[0], key[1], self.d_sums.ptr, self.d_flags.ptr,
                 )
             )
 
@@ -701,13 +728,13 @@ class Batch:
 def collapse_host(cube: np.ndarray, pa_bits: np.ndarray | None = None, n_groups: int = 0, ctx: Context | None = None):
     """``csg_collapse_host``: the drop-in for ``COLLAPSE_FUNCTION(cube, axis=1)``.
 
-    Returns ``(sums[(G+1), T, E], row_flags[T])``.
+    Returns ``(sums[(G+1), T, E], row_flags[T])``; the sums of an 8/16/32-bit integer cube are float64 (exact).
     """
     ctx = ctx or _lib.default_context()
     host, layout, (T, P, E) = classify_cube(np.asarray(cube))
     host = np.ascontiguousarray(host)
-    code = np_dtype_code(host.dtype)
-    sums = np.zeros((n_groups + 1, T, E), dtype=host.dtype)
+    code = np_cube_code(host.dtype)
+    sums = np.zeros((n_groups + 1, T, E), dtype=compute_dtype(host.dtype))
     flags = np.zeros(T, dtype=np.uint8)
     bits = np.ascontiguousarray(pa_bits, dtype=np.uint8) if n_groups else None
     ctx._check(
@@ -721,13 +748,16 @@ def collapse_host(cube: np.ndarray, pa_bits: np.ndarray | None = None, n_groups:
 
 def nansum(cube, axis: int = 1):
     """GPU ``np.nansum(cube, axis=1)`` with numpy's exact summation order (the
-    reference's pluggable ``COLLAPSE_FUNCTION``, ``constants.py:12``)."""
+    reference's pluggable ``COLLAPSE_FUNCTION``, ``constants.py:12``).  An 8/16/32-bit integer cube gives
+    numpy's int64 (signed) or uint64 (unsigned) sums, converted exactly from the float64 sums of K1."""
     cube = np.asarray(cube)
     if cube.ndim != 3:
         raise ValueError("nansum: expected a 3-D cube")
     if axis != 1:
         cube = np.moveaxis(cube, axis, 1)
     sums, _ = collapse_host(cube)
+    if cube.dtype in _lib.INT_CUBE_CODES:
+        return sums[0].astype(np.uint64 if cube.dtype.kind == "u" else np.int64)
     return sums[0]
 
 

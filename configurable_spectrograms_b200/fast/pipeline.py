@@ -20,7 +20,7 @@ from dataclasses import dataclass, field
 import numpy as np
 
 from .. import _lib
-from ..engine import WANT_GEOMETRY, WANT_PERCENTILES, WANT_REDUCTIONS, Batch
+from ..engine import WANT_GEOMETRY, WANT_PERCENTILES, WANT_REDUCTIONS, Batch, compute_dtype
 from .constants import DEFAULT_INSTRUMENT_ORDER, DEFAULT_PITCH_ANGLE_CATEGORIES, PITCH_ANGLE_ROW_KEYS
 
 
@@ -116,8 +116,7 @@ class ShardPlan:
     def compute_dtype(data_dtype) -> np.dtype:
         """The dtype numpy computes a cube of ``data_dtype`` in: float32 / float64 stay; everything else
         (integer counts) goes through float64, the dtype ``np.nanpercentile`` and matplotlib use for it."""
-        dt = np.dtype(data_dtype)
-        return dt if dt in (np.float32, np.float64) else np.dtype(np.float64)
+        return compute_dtype(data_dtype)
 
     # ------------------------------------------------------------- phase 1: files
     def add_orbit(self, orbit: int, datasets: dict, lines: dict | None = None):
@@ -146,7 +145,9 @@ class ShardPlan:
                 fid = self.batch.add_file(None, bits, shape=ds["shape"], layout=ds.get("layout"), device_ptr=ds["device_ptr"])
             else:
                 data = np.asarray(ds["data"])
-                if data.dtype != self.batch.dtype:  # integer counts only (see compute_dtype): exact in float64
+                # integer counts only (see compute_dtype); 8/16/32-bit ones stay as stored (in their pinned
+                # staging slot) -- K1 reads them and writes the exact float64 sums
+                if data.dtype != self.batch.dtype and data.dtype not in _lib.INT_CUBE_CODES:
                     data = data.astype(self.batch.dtype)
                 fid = self.batch.add_file(data, bits)
             self.file_meta.append({"times": np.asarray(ds["times"]), "energy": energy, "keys": keys, "inst": inst, "orbit": orbit})

@@ -24,7 +24,7 @@ from . import _lib
 from .colormaps import get_lut
 from .constants import AXIS_LABEL_FONT_SIZE, PLOT_FIGURE_HEIGHT_INCHES, PLOT_FIGURE_WIDTH_INCHES, TICK_LABEL_FONT_SIZE
 from .cusp_marking import draw_cusp_both_markers, draw_cusp_bracket_marker, draw_cusp_line_markers
-from .engine import Batch
+from .engine import Batch, compute_dtype
 from .fast.pipeline import check_norm_status, zoom_window
 from .figure import FigureCanvas, SpectrogramFigure, close_all_axes_and_clear
 from .logging_utils import log_message
@@ -95,9 +95,9 @@ def _as_cube(data_array_3d, collapse_axis):
         raise ValueError(f"make_spectrogram expects a 3-D array, got shape {cube.shape}")
     if collapse_axis != 1:
         cube = np.moveaxis(cube, collapse_axis, 1)
-    if cube.dtype not in (np.float32, np.float64):
+    if cube.dtype not in (np.float32, np.float64) and cube.dtype not in _lib.INT_CUBE_CODES:
         cube = cube.astype(np.float64)  # numpy sums and ranks integer input exactly; float64 keeps that
-    return cube
+    return cube  # 8/16/32-bit integers stay as stored: K1 reads them and writes the exact float64 sums
 
 
 def make_spectrogram(
@@ -204,7 +204,7 @@ def make_spectrogram(
         _group.plan(cube, keep, rows, log_scale, z_axis_min, z_axis_max, axis_object, x_axis_plot, y_kept, annotate)
         return axis_object, x_axis_plot
     ctx = _context or _lib.default_context()
-    batch = Batch(ctx, cube.dtype, n_groups=0)
+    batch = Batch(ctx, compute_dtype(cube.dtype), n_groups=0)
     f = batch.add_file(cube)
     batch.upload_cubes()
     batch.collapse()
@@ -242,7 +242,7 @@ class SpectrogramGroup:
     ``Batch.collapse_pending``; the host array is not kept) -- then :meth:`run` selects every panel's
     percentiles in ONE K2a launch, rasterises them in ONE K3 launch and finishes the axes from device
     rasters, so the figures go to ``png.write_figures_device`` without a pixel crossing PCIe uncompressed.
-    One batch per cube dtype (numpy computes each cube in its own dtype)."""
+    One batch per compute dtype (numpy computes each cube in its own dtype; integer cubes in float64)."""
 
     def __init__(self, colormap="viridis", context=None):
         self.ctx = context or _lib.default_context()
@@ -251,9 +251,10 @@ class SpectrogramGroup:
         self.pending: list = []
 
     def plan(self, cube, keep, rows, log_scale, z_min, z_max, axis_object, x_axis_plot, y_kept, annotate):
-        batch = self.batches.get(cube.dtype)
+        dtype = compute_dtype(cube.dtype)
+        batch = self.batches.get(dtype)
         if batch is None:
-            batch = self.batches[cube.dtype] = Batch(self.ctx, cube.dtype, n_groups=0)
+            batch = self.batches[dtype] = Batch(self.ctx, dtype, n_groups=0)
         f = batch.add_file(cube)
         batch.collapse_pending()
         region = batch.add_region(f, 0, keep, rows=rows, want_pct=z_min is None or z_max is None)
@@ -289,7 +290,7 @@ class SpectrogramGroup:
         return outcome
 
     def rgba_ptr(self, figure) -> int:
-        """Device address of the RGBA buffer a figure's panels live in (one dtype per figure)."""
+        """Device address of the RGBA buffer a figure's panels live in (one compute dtype per figure)."""
         owners = {id(ax.images[-1].batch): ax.images[-1].batch for ax in figure.axes if ax.images and hasattr(ax.images[-1], "batch")}
         if len(owners) != 1:
             raise ValueError("a figure drawn from a group must hold panels of one cube dtype")

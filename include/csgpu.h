@@ -15,7 +15,10 @@
  *     stream (own stream, or an external cudaStream_t handed to csg_create()).
  *   - dtype: CSG_F32 / CSG_F64 is the dtype D of the counts cube; sums,
  *     percentiles and normalisation are computed in D exactly like numpy /
- *     matplotlib do (SURVEY.md Appendix B).
+ *     matplotlib do (SURVEY.md Appendix B).  The K1 entry points also take
+ *     integer cubes (CSG_I8 .. CSG_U32): their sums are float64 (exact), and
+ *     every later stage sees a CSG_F64 batch; every other entry point refuses
+ *     the integer codes.
  *   - there is NO CPU fallback: without a CUDA device every compute call fails.
  */
 #ifndef CSGPU_H
@@ -28,7 +31,7 @@
 extern "C" {
 #endif
 
-#define CSG_ABI_VERSION 26
+#define CSG_ABI_VERSION 27
 
 #if defined(__GNUC__)
 #define CSG_API __attribute__((visibility("default")))
@@ -46,6 +49,11 @@ typedef enum {
 } csg_status;
 
 enum { CSG_F32 = 0, CSG_F64 = 1 };
+/* cube dtypes of csg_collapse, csg_collapse_host, csg_collapse_kernel(_for) and csg_collapse_blocks only:
+ * numpy sums them in int64 / uint64; integer addition is associative, so the sum does not depend on the
+ * order, and every such sum (|x| < 2^32, P <= 32768) is below 2^47, so its float64 is exact -- the same
+ * bits as the cube widened to float64 on the host. */
+enum { CSG_I8 = 2, CSG_U8 = 3, CSG_I16 = 4, CSG_U16 = 5, CSG_I32 = 6, CSG_U32 = 7 };
 /* memory order of a counts cube */
 enum {
   CSG_LAYOUT_TPE = 0, /* C-contiguous (time, pitch, energy): np.nansum(axis=1) is an ascending-p chain  */
@@ -128,7 +136,7 @@ CSG_API int csg_event_sync(csg_ctx* ctx, int slot);
  * data[:, mask, :] (CS/fast/plotting.py:121-127) and the zoom test
  * np.any(~np.isnan(cube[window])) (CS/plotting.py:597-603). */
 typedef struct {
-  const void* d_cube; /* device cube, dtype D, layout as given to csg_collapse()         */
+  const void* d_cube; /* device cube of the call's cube dtype, layout as given to csg_collapse() */
   int64_t sums_off;   /* element offset in d_sums of this file's [(G+1)][E][Tp] block (multiple of 4) */
   int64_t flags_off;  /* byte offset in d_row_flags of this file's [T] flag bytes       */
   int32_t T, P, E;
@@ -140,8 +148,9 @@ typedef struct {
 
 /* Which kernel collapses a file: the stream kernel (16-row tiles, loop bodies specialised per
  * run of constant group membership, coalesced transposed output) needs a 16-byte aligned
- * C-contiguous (T,P,E) cube with E / (16 bytes / sizeof D) in {16,24,32,48,64}; everything else
- * takes the generic kernel.  A csg_collapse() call handles files of ONE kernel, and every file of
+ * C-contiguous (T,P,E) cube with E / (16 bytes / sizeof D) in {16,24,32,48,64} (integer cubes:
+ * E * itemsize a multiple of 16 bytes, at most 512 bytes); everything else takes the generic
+ * kernel.  A stored (T,E,P) integer view always takes the row kernel (CSG_K1_STREAM).  A csg_collapse() call handles files of ONE kernel, and every file of
  * a STREAM table has the same E (= max_E). */
 enum { CSG_K1_GENERIC = 0, CSG_K1_STREAM = 1 };
 CSG_API int csg_collapse_kernel(int32_t T, int32_t P, int32_t E, int dtype, int layout, const void* d_cube);
@@ -162,7 +171,8 @@ CSG_API int64_t csg_sums_elems(int32_t T, int32_t E, int n_groups);
  * sums[file][g][e][t] at sums_off + (g*E + e)*Tp + t; g = 0 is the sum over every pitch bin,
  * g = 1+k the sum over bins p with (d_pa_bits[bits_off+p] >> k) & 1 (cells t >= T of a row
  * are padding and never read).  NaN counts as +0, fill values and +-inf are summed as-is,
- * result dtype = D, summation order bit-identical to numpy's (SURVEY.md Appendix B).
+ * result dtype = D, summation order bit-identical to numpy's (SURVEY.md Appendix B); for an
+ * integer cube dtype the result is float64 (d_sums holds doubles) and the order is free.
  * d_row_flags[flags_off+t] bit 0 / bit 1+k: some non-NaN cell exists in time row t among
  * all / group-k pitch bins (any energy); zero it before the call.
  * All files of one call share dtype, layout, kernel and n_groups. */
@@ -181,7 +191,8 @@ CSG_API int csg_window_any(csg_ctx* ctx, const uint8_t* d_row_flags, const csg_f
                    const int32_t* d_index_pool, uint8_t* d_out);
 
 /* Host-buffer convenience for one cube: the drop-in for COLLAPSE_FUNCTION(array, axis=1).
- * h_pa_bits may be NULL when n_groups == 0.  h_sums receives [(G+1)][T][E] of dtype D,
+ * h_pa_bits may be NULL when n_groups == 0.  h_sums receives [(G+1)][T][E] of dtype D (float64
+ * for an integer cube),
  * h_row_flags (may be NULL) [T]. */
 CSG_API int csg_collapse_host(csg_ctx* ctx, const void* h_cube, int32_t T, int32_t P, int32_t E, int dtype,
                       int layout, const uint8_t* h_pa_bits, int n_groups, void* h_sums,
